@@ -3,7 +3,7 @@
 queries/sec & HBM GB/s vs roofline").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                  [--dtype f32|bf16] [--dist grid|random] [--batch B]
+                  [--dtype f32|bf16] [--dist grid|random] [--batch B] [--dump-outputs DIR]
 
 One "step" = one forward + one backward of the drop-in op
 ``MSDeformAttnFunction`` (C ABI msda_forward + msda_backward) over one batch of B=8 frames of
@@ -17,6 +17,12 @@ no data-path collective) -> weak scaling; time = max over ranks.
 restatement of ms_deform_attn_core_pytorch (oracle/msda_oracle.py; the original cannot be
 imported on the GPU box, /root/reference does not travel) -- fwd + autograd bwd, all host
 threads, on a bounded sample (1 frame per step).
+
+``--dump-outputs DIR`` writes what the timed op returned in its last timed step (rank 0) as
+DIR/<name>.npy in float32: output, grad_value, grad_sampling_loc, grad_attn_weight.  An array of
+more than DUMP_SAMPLE elements is stored as the elements at DUMP_SAMPLE fixed positions drawn from
+a seeded generator (the same positions in every run), so two builds run with the same arguments
+can be compared output for output.
 """
 import argparse
 import json
@@ -29,11 +35,14 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
 
 COCO_SHAPES = [(100, 167), (50, 84), (25, 42), (13, 21)]
 M, D, P = 8, 32, 4
 METRIC = "msda_fwd_bwd_queries_per_sec"
 UNIT = "queries/s"
+DUMP_NAMES = ("output", "grad_value", "grad_sampling_loc", "grad_attn_weight")
+DUMP_SAMPLE = 3 << 20                   # elements kept per array: 4 arrays x 12 MiB of float32 <= 64 MiB
 
 
 def level_start(shapes):
@@ -75,6 +84,24 @@ def make_inputs(torch, n, seed, dist):
         loc = ref[None, :, None, None, None, :] + off / norm[None, None, None, :, None, :]
     grad_out = torch.randn(n, lq, M * D, generator=g)
     return value.contiguous(), loc.contiguous(), attn.contiguous(), grad_out.contiguous()
+
+
+def dump_positions(torch, numel, seed):
+    """The flat positions --dump-outputs keeps of an array of more than DUMP_SAMPLE elements: sorted, drawn from a
+    generator seeded by the array's place in DUMP_NAMES, so they depend on the array's size alone."""
+    return torch.randint(numel, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(seed)).sort().values
+
+
+def dump_outputs(torch, path, arrays):
+    """Write the op's results (in DUMP_NAMES order) as <path>/<name>.npy in float32; an array of more than
+    DUMP_SAMPLE elements is written flat, as its elements at dump_positions()."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for seed, (name, t) in enumerate(zip(DUMP_NAMES, arrays)):
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            t = t.reshape(-1)[dump_positions(torch, t.numel(), seed).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
 
 
 def algorithmic_bytes(n, e_v):
@@ -230,7 +257,7 @@ def time_cpu_reference(torch, steps, warmup, dist, seed=0):
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        msda_oracle.core_pytorch_fwd_bwd(value, COCO_SHAPES, loc, attn, gout)
+        outputs = msda_oracle.core_pytorch_fwd_bwd(value, COCO_SHAPES, loc, attn, gout)
         times.append(time.perf_counter() - t0)
     timed = times[warmup:]
     total = sum(timed)
@@ -239,7 +266,7 @@ def time_cpu_reference(torch, steps, warmup, dist, seed=0):
             "sample": f"{len(timed)} x (1 frame, {value.shape[1]} queries) fwd+bwd, fp32, "
                       f"oracle.core_pytorch (= reference ms_deform_attn_core_pytorch) + autograd, "
                       f"os.cpu_count()={os.cpu_count()}",
-            "ms_per_step": 1e3 * total / len(timed)}
+            "ms_per_step": 1e3 * total / len(timed), "outputs": outputs}
 
 
 def run_reference(args):
@@ -259,6 +286,8 @@ def run_reference(args):
             "cpu_baseline": {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")},
             "e2e": {"value": cb["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
+    if args.dump_outputs:
+        dump_outputs(torch, args.dump_outputs, cb["outputs"])
     print(json.dumps(line), flush=True)
 
 
@@ -660,9 +689,12 @@ def run_b200(args):
         t_start = torch.cuda.Event(enable_timing=True)
         t_end = torch.cuda.Event(enable_timing=True)
         t_start.record()
-        ev, _ = run_steps(args.steps)
+        ev, last = run_steps(args.steps)
         t_end.record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, (last[0], *last[1]))
+    del last
     elapsed_ms = t_start.elapsed_time(t_end)
     fwd_all = sorted(e[0].elapsed_time(e[1]) for e in ev)
     bwd_all = sorted(e[1].elapsed_time(e[2]) for e in ev)
@@ -873,7 +905,11 @@ def main():
     ap.add_argument("--batch", type=int, default=8)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the encoder / training-step side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the op's results of the last timed step as DIR/<name>.npy (float32, <= 64 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,13 +6,16 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import torch
+
 from tests.util import ROOT
 
 
-def test_reference_arm_prints_the_contract_line():
+def test_reference_arm_prints_the_contract_line(tmp_path):
     proc = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                           "--warmup", "1"], cwd=ROOT, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True,
-                          timeout=600)
+                           "--warmup", "1", "--dump-outputs", str(tmp_path)], cwd=ROOT, stdout=subprocess.PIPE,
+                          stderr=subprocess.PIPE, text=True, timeout=600)
     assert proc.returncode == 0, proc.stderr[-2000:]
     lines = [ln for ln in proc.stdout.splitlines() if ln.startswith("{")]
     assert len(lines) == 1
@@ -27,6 +30,19 @@ def test_reference_arm_prints_the_contract_line():
     assert line["e2e"] == {"value": line["value"], "unit": "queries/s", "h2d_bytes_per_step": 0,
                            "d2h_bytes_per_step": 0}
     assert line["gpu_launches"] == 0
+    # --dump-outputs: the last step's results in float32, 64 MiB at most; a large array is kept at dump_positions()
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle import msda_oracle
+    dumped = {name: np.load(tmp_path / (name + ".npy")) for name in bench.DUMP_NAMES}
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(n + ".npy" for n in bench.DUMP_NAMES)
+    assert all(a.dtype == np.float32 for a in dumped.values())
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+    value, loc, attn, _ = bench.make_inputs(torch, 1, 0, "grid")
+    out = msda_oracle.core_pytorch(value, bench.COCO_SHAPES, loc, attn).reshape(-1)
+    np.testing.assert_allclose(dumped["output"], out[bench.dump_positions(torch, out.numel(), 0)].numpy(),
+                               rtol=1e-6, atol=1e-7)
+    assert dumped["grad_attn_weight"].shape == tuple(attn.shape)        # small enough to be stored whole
 
 
 def test_algorithmic_bytes_match_the_stated_per_query_figures():
