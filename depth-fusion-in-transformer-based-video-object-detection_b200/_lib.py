@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # MSDA_B200_LIB selects another build of the same ABI (A/B kernel experiments); default: in-tree
 LIB_PATH = os.environ.get("MSDA_B200_LIB") or os.path.join(_HERE, "libmsda_b200.so")
 
-ABI_VERSION = 20
+ABI_VERSION = 21
 DTYPE_F32, DTYPE_F64, DTYPE_BF16, DTYPE_F16 = 0, 1, 2, 3
 FLAG_FORCE_GENERIC = 1
 FLAG_TC = 4
@@ -89,6 +89,12 @@ def load():
     lib.msda_layer_linear_bf16_supported.argtypes = [c_int, c_int]
     lib.msda_layer_linear_bf16.restype = c_int
     lib.msda_layer_linear_bf16.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp, c_vp]
+    lib.msda_layer_linear_bf16_wgrad_supported.restype = c_int
+    lib.msda_layer_linear_bf16_wgrad_supported.argtypes = [c_int, c_int]
+    lib.msda_layer_linear_bf16_wgrad_scratch_floats.restype = c_i64
+    lib.msda_layer_linear_bf16_wgrad_scratch_floats.argtypes = [c_i64, c_int, c_int]
+    lib.msda_layer_linear_bf16_wgrad.restype = c_int
+    lib.msda_layer_linear_bf16_wgrad.argtypes = [c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_vp]
     lib.msda_layer_linear_tf32x3_supported.restype = c_int
     lib.msda_layer_linear_tf32x3_supported.argtypes = [c_int, c_int]
     lib.msda_layer_linear_tf32x3.restype = c_int

@@ -13,8 +13,11 @@
 // 9 TMA producer.
 #include <cuda.h>
 
+#include <atomic>
+
 #include "msda_common.cuh"
 #include "msda_launch.h"
+#include "msda_tc.cuh"
 #include "umma.cuh"
 
 namespace msda {
@@ -284,6 +287,249 @@ cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const un
     const int grid = (int)(units < clusters ? units : clusters) * kLbCluster;
     linear_bf16_kernel<<<grid, kLbThreads, kLbSmem, stream>>>(tm_x, tm_w, tm_y, (const __nv_bfloat16*)bias, row_mask, rows, n, k,
                                                                relu, bn);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
+// weight / bias gradient of the same layer (training):
+//
+//     dW [N, K] = g^T x,   db [N] = sum over rows of g,   g [rows, N], x [rows, K], bf16, fp32 accumulation.
+//
+// The reduction runs over `rows`, so both operands are MN-major: a TMA box {64 columns, 64 rows} with SWIZZLE_128B lands
+// as 64 rows of 128 bytes = the MN-major SWIZZLE_128B image of 64 output features (or inputs) x 64 reduction steps.  An
+// output tile is 128 features (two g boxes, M) x up to 256 inputs (four x boxes, N).  There are only 2-8 such tiles at
+// the model's shapes, so `rows` is split into contiguous slices (split-K), about one CTA per SM: each CTA accumulates its
+// slice in TMEM and writes the fp32 partial tile to `scratch`; a second kernel sums the partials in split order (the
+// result does not depend on scheduling) and rounds to bf16.  The bias gradient comes from the same g tiles: CTAs of
+// column tile 0 issue one more M = 128, N = 16 MMA per K step against a constant all-ones K-major B tile, which puts
+// sum_rows g of their 128 features into 16 extra TMEM columns (all equal; column 0 is kept) -- g is read once.
+// Warp roles (6 warps): 0-3 epilogue (warp = TMEM lane quadrant), 4 MMA issuer, 5 TMA producer.
+// ------------------------------------------------------------------------------------------
+constexpr int kWgBM = 128;                  // output features per tile (TMEM lanes)
+constexpr int kWgBN = 256;                  // inputs per tile (TMEM columns)
+constexpr int kWgBK = 64;                   // rows per K block
+constexpr int kWgBox = 64 * kWgBK * 2;      // one {64 columns, 64 rows} bf16 box: 8 KB
+constexpr int kWgStageBytes = (kWgBM / 64 + kWgBN / 64) * kWgBox;   // 2 g boxes + 4 x boxes: 48 KB
+constexpr int kWgStages = 4;
+constexpr int kWgOnesBytes = 16 * 128;      // all-ones B tile of the bias MMA: 16 rows x 64 bf16
+constexpr int kWgDbCol = kWgBN;             // TMEM column of the bias accumulator
+constexpr int kWgEpiThreads = 128;
+constexpr int kWgThreads = kWgEpiThreads + 64;
+constexpr int kWgSmem = kWgStages * kWgStageBytes + kWgOnesBytes + 256 + 1024;   // + barriers + alignment slack
+static_assert(kWgSmem <= 232448, "exceeds the 227 KB of shared memory a CTA can opt in to");
+constexpr int kWgTargetCtas = 148;          // B200 SMs: split count aimed at one CTA per SM, fixed so that the split (and
+                                            // so the rounding of the result) does not depend on the device
+constexpr int kWgMinKBlocks = 4;            // a split reads at least 256 rows: its partial tile is small against its loads
+
+struct WgBars {
+    unsigned long long full[kWgStages], empty[kWgStages], acc_full;
+    unsigned tmem_base;
+};
+
+__global__ void __launch_bounds__(kWgThreads, 1)
+linear_bf16_wgrad_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_constant__ CUtensorMap tm_x,
+                         float* __restrict__ partial, long long rows, int N, int K, int bn, int tiles_n, int tiles,
+                         int splits, int kb_per_split, long long blk_floats, int want_db)
+{
+    extern __shared__ unsigned char smem_raw[];
+    unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+    unsigned char* s_ones = smem + kWgStages * kWgStageBytes;          // 1024-byte aligned
+    WgBars* bars = reinterpret_cast<WgBars*>(s_ones + kWgOnesBytes);
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // CTAs of one split (same rows) are adjacent: the tiles that share a slice of g or x read it from L2
+    const int split = blockIdx.x / tiles, t = blockIdx.x % tiles;
+    const int m0 = (t / tiles_n) * kWgBM, n0 = (t % tiles_n) * bn;
+    const int n_cur = min(bn, K - n0);
+    const int kblocks = (int)((rows + kWgBK - 1) / kWgBK);
+    const int kb0 = split * kb_per_split, kb1 = min(kb0 + kb_per_split, kblocks);
+    const bool with_db = want_db && n0 == 0;
+
+    if (warp == 0) tmem_alloc(&bars->tmem_base, 512);
+    for (int i = tid; i < kWgOnesBytes / 16; i += kWgThreads)            // bf16 1.0 = 0x3f80
+        reinterpret_cast<uint4*>(s_ones)[i] = make_uint4(0x3f803f80u, 0x3f803f80u, 0x3f803f80u, 0x3f803f80u);
+    fence_proxy_async();                                                // generic writes -> tensor-core reads
+    if (tid == kWgEpiThreads) {
+        for (int i = 0; i < kWgStages; ++i) { mbar_init(&bars->full[i], 1); mbar_init(&bars->empty[i], 1); }
+        mbar_init(&bars->acc_full, 1);
+        fence_mbar_init();
+        tma_prefetch_desc(&tm_g); tma_prefetch_desc(&tm_x);
+    }
+    tcgen05_fence_before();
+    __syncthreads();
+    tcgen05_fence_after();
+    const unsigned tmem = bars->tmem_base;
+
+    if (warp == 5) {
+        // ======================================= TMA producer =======================================
+        if (elect_one()) {
+            // boxes wholly past the last feature / input are not loaded: they only feed accumulator lanes / columns
+            // that are never read.  Rows past the end arrive as zeros (TMA out-of-bounds fill).
+            const int g_boxes = min(kWgBM, N - m0) / 64, x_boxes = n_cur / 64;
+            const unsigned bytes = (unsigned)(g_boxes + x_boxes) * kWgBox;
+            for (int kb = kb0; kb < kb1; ++kb) {
+                const int i = kb - kb0, s = i % kWgStages;
+                if (i >= kWgStages) mbar_wait(&bars->empty[s], ((i / kWgStages) - 1) & 1);
+                unsigned char* st = smem + s * kWgStageBytes;
+                mbar_expect_tx(&bars->full[s], bytes);
+                for (int c = 0; c < g_boxes; ++c) tma_load_2d(st + c * kWgBox, &tm_g, m0 + 64 * c, kb * kWgBK, &bars->full[s]);
+                for (int c = 0; c < x_boxes; ++c)
+                    tma_load_2d(st + (kWgBM / 64 + c) * kWgBox, &tm_x, n0 + 64 * c, kb * kWgBK, &bars->full[s]);
+            }
+        }
+        __syncwarp();
+    } else if (warp == 4) {
+        // ======================================= MMA issuer =======================================
+        // A = g^T (M = 128 features, MN-major), B = x (N = inputs, MN-major): leading byte offset = distance between the
+        // 64-element boxes along M / N, stride byte offset = 8 rows of 128 bytes; one K = 16 step = 16 rows = 2048 bytes
+        const unsigned idesc = tc::make_idesc(kWgBM, n_cur, 1, 1);
+        const unsigned idesc_db = tc::make_idesc(kWgBM, 16, 1, 0);
+        const unsigned long long d_ones = make_desc_sw128(s_ones);
+        for (int kb = kb0; kb < kb1; ++kb) {
+            const int i = kb - kb0, s = i % kWgStages;
+            mbar_wait(&bars->full[s], (i / kWgStages) & 1);
+            tcgen05_fence_after();
+            if (elect_one()) {
+                unsigned char* st = smem + s * kWgStageBytes;
+                const unsigned long long d_g = tc::make_desc(st, kWgBox, 1024, 2);
+                const unsigned long long d_x = tc::make_desc(st + (kWgBM / 64) * kWgBox, kWgBox, 1024, 2);
+#pragma unroll
+                for (int j = 0; j < kWgBK / 16; ++j) {
+                    mma_bf16(tmem, desc_advance(d_g, j * 2048), desc_advance(d_x, j * 2048), idesc, (i | j) != 0);
+                    if (with_db) mma_bf16(tmem + kWgDbCol, desc_advance(d_g, j * 2048), desc_advance(d_ones, j * 32), idesc_db,
+                                          (i | j) != 0);
+                }
+                mma_commit(&bars->empty[s]);                                 // stage free once these MMAs are done
+                if (kb == kb1 - 1) mma_commit(&bars->acc_full);
+            }
+            __syncwarp();
+        }
+    } else {
+        // ======================================= epilogue warps =======================================
+        // TMEM lane = feature row of the tile -> this CTA's fp32 partial block [128][bn] (+ [128] bias partial)
+        const unsigned lane_base = (unsigned)(warp * 32) << 16;
+        const int r = warp * 32 + lane;
+        float* blk = partial + ((long long)t * splits + split) * blk_floats;
+        mbar_wait(&bars->acc_full, 0);
+        tcgen05_fence_after();
+        for (int c = 0; c < n_cur; c += 32) {
+            float v[32];
+            tmem_ld32(tmem + c + lane_base, v);
+            float4* dst = reinterpret_cast<float4*>(blk + (long long)r * bn + c);
+#pragma unroll
+            for (int q = 0; q < 8; ++q) dst[q] = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+        }
+        if (with_db) {
+            float v[16];
+            tmem_ld16(tmem + kWgDbCol + lane_base, v);
+            blk[(long long)kWgBM * bn + r] = v[0];
+        }
+    }
+    tcgen05_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_free(tmem, 512);
+}
+
+// dW / db = sum over the splits of the partial blocks, in split order, rounded to bf16.  Block (32, 8): x = 4 consecutive
+// outputs, y = every 8th split; the 8 sums are added in y order.
+__global__ void __launch_bounds__(256)
+linear_bf16_wgrad_reduce_kernel(const float* __restrict__ partial, __nv_bfloat16* __restrict__ dw, __nv_bfloat16* __restrict__ db,
+                                int N, int K, int bn, int tiles_n, int splits, long long blk_floats)
+{
+    __shared__ float4 s_sum[8][32];
+    const long long q = (long long)blockIdx.x * 32 + threadIdx.x;        // quad of outputs
+    const long long qw = (long long)N * K / 4, qb = db != nullptr ? N / 4 : 0;
+    long long base = -1, dst = 0;
+    if (q < qw) {
+        const long long e = q * 4;
+        const int o = (int)(e / K), i = (int)(e % K);
+        base = ((long long)((o / kWgBM) * tiles_n + i / bn) * splits) * blk_floats + (long long)(o % kWgBM) * bn + i % bn;
+        dst = e;
+    } else if (q < qw + qb) {
+        const int o = (int)(q - qw) * 4;
+        base = ((long long)((o / kWgBM) * tiles_n) * splits) * blk_floats + (long long)kWgBM * bn + o % kWgBM;
+        dst = o;
+    }
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (base >= 0)
+        for (int s = threadIdx.y; s < splits; s += 8) {
+            const float4 v = __ldg(reinterpret_cast<const float4*>(partial + base + (long long)s * blk_floats));
+            acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+        }
+    s_sum[threadIdx.y][threadIdx.x] = acc;
+    __syncthreads();
+    if (threadIdx.y != 0 || base < 0) return;
+#pragma unroll
+    for (int y = 1; y < 8; ++y) {
+        const float4 v = s_sum[y][threadIdx.x];
+        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    }
+    __nv_bfloat162 lo = __floats2bfloat162_rn(acc.x, acc.y), hi = __floats2bfloat162_rn(acc.z, acc.w);
+    uint2 packed;
+    packed.x = *reinterpret_cast<unsigned*>(&lo);
+    packed.y = *reinterpret_cast<unsigned*>(&hi);
+    *reinterpret_cast<uint2*>((q < qw ? dw : db) + dst) = packed;
+}
+
+bool linear_bf16_wgrad_supported(int n, int k)
+{
+    return n >= 64 && n % 64 == 0 && k >= 64 && k % 64 == 0;
+}
+
+struct WgPlan {
+    int bn, tiles_n, tiles, splits, kb_per_split;
+    long long blk_floats;
+};
+
+static bool wgrad_plan(long long rows, int n, int k, WgPlan* p)
+{
+    if (!linear_bf16_wgrad_supported(n, k) || rows < 1 || rows >= (1ll << 31) - 1024) return false;
+    p->tiles_n = (k + kWgBN - 1) / kWgBN;
+    p->bn = ((k + p->tiles_n - 1) / p->tiles_n + 63) / 64 * 64;         // equal column tiles, multiples of 64
+    p->tiles = ((n + kWgBM - 1) / kWgBM) * p->tiles_n;
+    const int kblocks = (int)((rows + kWgBK - 1) / kWgBK);
+    const int want = max(1, kWgTargetCtas / p->tiles);
+    p->kb_per_split = max(kWgMinKBlocks, (kblocks + want - 1) / want);
+    p->splits = (kblocks + p->kb_per_split - 1) / p->kb_per_split;     // every split has at least one K block
+    p->blk_floats = (long long)kWgBM * p->bn + kWgBM;
+    return true;
+}
+
+long long linear_bf16_wgrad_scratch_floats(long long rows, int n, int k)
+{
+    WgPlan p;
+    return wgrad_plan(rows, n, k, &p) ? (long long)p.tiles * p.splits * p.blk_floats : 0;
+}
+
+cudaError_t linear_bf16_wgrad(const void* g, const void* x, long long rows, int n, int k, void* dw, void* db,
+                              float* scratch, long long scratch_floats, cudaStream_t stream)
+{
+    WgPlan p;
+    if (!wgrad_plan(rows, n, k, &p) || scratch_floats < (long long)p.tiles * p.splits * p.blk_floats || dw == nullptr)
+        return cudaErrorInvalidValue;
+    if ((reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dw) |
+         reinterpret_cast<uintptr_t>(db) | reinterpret_cast<uintptr_t>(scratch)) % 16 != 0)
+        return cudaErrorInvalidValue;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    // the attribute is per device; concurrent first calls may both set it (harmless), none reads a torn flag
+    static std::atomic<bool> configured[64];
+    if (dev < 0 || dev >= 64 || !configured[dev].load(std::memory_order_acquire)) {
+        cudaError_t e = cudaFuncSetAttribute(linear_bf16_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
+        if (e != cudaSuccess) return e;
+        if (dev >= 0 && dev < 64) configured[dev].store(true, std::memory_order_release);
+    }
+    alignas(64) CUtensorMap tm_g, tm_x;
+    if (!lb_make_map(&tm_g, g, (unsigned long long)rows, (unsigned long long)n, kWgBK) ||
+        !lb_make_map(&tm_x, x, (unsigned long long)rows, (unsigned long long)k, kWgBK))
+        return cudaErrorNotSupported;
+    linear_bf16_wgrad_kernel<<<p.tiles * p.splits, kWgThreads, kWgSmem, stream>>>(
+        tm_g, tm_x, scratch, rows, n, k, p.bn, p.tiles_n, p.tiles, p.splits, p.kb_per_split, p.blk_floats, db != nullptr);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const long long quads = (long long)n * k / 4 + (db != nullptr ? n / 4 : 0);
+    linear_bf16_wgrad_reduce_kernel<<<(unsigned)((quads + 31) / 32), dim3(32, 8), 0, stream>>>(
+        scratch, (__nv_bfloat16*)dw, (__nv_bfloat16*)db, n, k, p.bn, p.tiles_n, p.splits, p.blk_floats);
     return cudaGetLastError();
 }
 

@@ -7,7 +7,7 @@ static bool bad_dims(int N, int S, int M, int D, int L, int Lq, int P)
     return N < 0 || S < 0 || M < 0 || D < 0 || L < 0 || Lq < 0 || P < 0;
 }
 
-extern "C" int msda_abi_version(void) { return 20; }
+extern "C" int msda_abi_version(void) { return 21; }
 
 extern "C" const char* msda_error_string(int code)
 {
@@ -391,6 +391,24 @@ extern "C" int msda_layer_linear_bf16(const void* x, const void* weight, const v
     if (rows < 0) return (int)cudaErrorInvalidValue;
     return (int)msda::linear_bf16(x, weight, bias, zero_rows, (long long)rows, out_features, in_features, relu, y,
                                   (cudaStream_t)stream);
+}
+
+extern "C" int msda_layer_linear_bf16_wgrad_supported(int out_features, int in_features)
+{
+    return msda::linear_bf16_wgrad_supported(out_features, in_features) ? 1 : 0;
+}
+
+extern "C" int64_t msda_layer_linear_bf16_wgrad_scratch_floats(int64_t rows, int out_features, int in_features)
+{
+    return (int64_t)msda::linear_bf16_wgrad_scratch_floats((long long)rows, out_features, in_features);
+}
+
+extern "C" int msda_layer_linear_bf16_wgrad(const void* grad_y, const void* x, int64_t rows, int out_features,
+                                            int in_features, void* grad_weight, void* grad_bias, float* scratch,
+                                            int64_t scratch_floats, void* stream)
+{
+    return (int)msda::linear_bf16_wgrad(grad_y, x, (long long)rows, out_features, in_features, grad_weight, grad_bias,
+                                        scratch, (long long)scratch_floats, (cudaStream_t)stream);
 }
 
 extern "C" int msda_layer_linear_tf32x3_supported(int out_features, int in_features)

@@ -174,6 +174,12 @@ cudaError_t tf32_split(const float* x, float* out, long long rows, int cols, cud
 bool linear_bf16_supported(int n, int k);
 cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const unsigned char* row_mask, long long rows, int n,
                         int k, int relu, void* y, cudaStream_t stream);
+// weight / bias gradient of that layer: dW [n, k] = g^T x, db [n] = sum over rows of g (bf16, fp32 split-K partials in
+// `scratch`, summed in a fixed order by a second kernel: deterministic)
+bool linear_bf16_wgrad_supported(int n, int k);
+long long linear_bf16_wgrad_scratch_floats(long long rows, int n, int k);   // 0 = unsupported
+cudaError_t linear_bf16_wgrad(const void* g, const void* x, long long rows, int n, int k, void* dw, void* db,
+                              float* scratch, long long scratch_floats, cudaStream_t stream);
 bool linear_tf32x3_supported(int n, int k);
 cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, const float* bias, long long rows, int n,
                           int k, int relu, float* y, cudaStream_t stream);

@@ -213,7 +213,8 @@ def column_sum(g2):
 
 class LinearFunction(Function):
     """x @ W^T + b as the library GEMM, with a backward that takes the bias gradient from the
-    column-sum kernel instead of PyTorch's generic reduction."""
+    column-sum kernel instead of PyTorch's generic reduction.  bf16 training from BF16_TRAIN_KERNEL_MIN_ROWS rows up:
+    the package's own kernels in both directions (_bf16_train_kernels_apply)."""
 
     @staticmethod
     def forward(ctx, x2, weight, bias):              # x2 [rows, in] -> fresh [rows, out] (never a view)
@@ -226,6 +227,9 @@ class LinearFunction(Function):
             weight_c, bias_c = weight, bias
         ctx.save_for_backward(x2, weight_c)
         ctx.param_dtypes = (weight.dtype, bias.dtype)
+        ctx.kernels = any(ctx.needs_input_grad) and _bf16_train_kernels_apply(x2, weight_c, bias_c)
+        if ctx.kernels:
+            return linear_bf16(x2, weight_c, bias_c)
         return torch.addmm(bias_c, x2, weight_c.t())
 
     @staticmethod
@@ -236,6 +240,8 @@ class LinearFunction(Function):
             g2 = g2.contiguous()
         if g2.dtype != weight.dtype:
             g2 = g2.to(weight.dtype)
+        if ctx.kernels:
+            return _bf16_linear_backward(ctx.needs_input_grad, g2, x2, weight, ctx.param_dtypes)
         dx = g2 @ weight if ctx.needs_input_grad[0] else None
         dw = (g2.t() @ x2).to(ctx.param_dtypes[0]) if ctx.needs_input_grad[1] else None
         db = column_sum(g2).to(ctx.param_dtypes[1]) if ctx.needs_input_grad[2] else None
@@ -392,7 +398,77 @@ def linear_bf16(x, weight, bias, relu=False, zero_rows=None):
                                                   None if m is None else m.data_ptr(), x2.shape[0], weight.shape[0], k,
                                                   1 if relu else 0, y.data_ptr(), torch.cuda.current_stream().cuda_stream)
     _lib.check(code, "msda_layer_linear_bf16")
-    return y.view(*x.shape[:-1], weight.shape[0])
+    # (a 2-d input gets y itself, not a view of it: LinearFunction hands it to autograd, where it may be modified in place)
+    return y if x.dim() == 2 else y.view(*x.shape[:-1], weight.shape[0])
+
+
+# bf16 training: from BF16_TRAIN_KERNEL_MIN_ROWS rows up, LinearFunction and LinearReLUFunction run their forward on
+# csrc/linear_bf16.cu and their backward as dx = g W (the same kernel with W^T as its weight) and one weight-gradient kernel
+# that also gives the bias gradient (linear_bf16_wgrad: g is read once for both).  Set to None to keep the library GEMMs.
+# The kernels spread 128-row tiles (forward, dx) and row slices (dW) over all SMs; the threshold keeps the decoder-sized
+# GEMMs (1200 rows) on the library.  Graphed Encoder-Cross-Fusion training step on one B200 (DESIGN.md section 3.13):
+# 22.05 ms with the library GEMMs, 21.53 ms on the kernels (1000 W power limit).
+BF16_TRAIN_KERNEL_MIN_ROWS = 16384
+
+
+def _bf16_train_kernels_win(n, k):
+    """Measured on B200 at 88 892 rows (tools/bench_train_linears.py, DESIGN.md section 3.13): dx + dW + db on the kernels
+    beat the library's three calls where the layer's input is one column tile wide (256 <- 256, 384 <- 256,
+    1024 <- 256: 5-14 % faster) and lose at 256 <- 1024 (linear2 of the feed-forward block: 6 % slower), which keeps
+    the library."""
+    return k <= 256
+
+
+def _bf16_train_kernels_apply(x2, weight, bias):
+    """Gradients flow (checked by the caller), the operands as multiplied are CUDA bf16, enough rows, a shape where the
+    kernels are faster, and the forward, input-gradient and weight-gradient kernels all take it."""
+    if BF16_TRAIN_KERNEL_MIN_ROWS is None or not x2.is_cuda or x2.shape[0] < BF16_TRAIN_KERNEL_MIN_ROWS:
+        return False
+    if x2.dtype != torch.bfloat16 or weight.dtype != torch.bfloat16 or (bias is not None and bias.dtype != torch.bfloat16):
+        return False
+    n, k = weight.shape
+    lib = _lib.load()
+    return (x2.shape[1] == k and _bf16_train_kernels_win(n, k) and bool(lib.msda_layer_linear_bf16_supported(n, k))
+            and bool(lib.msda_layer_linear_bf16_supported(k, n)) and bool(lib.msda_layer_linear_bf16_wgrad_supported(n, k)))
+
+
+def linear_bf16_wgrad(g2, x2, with_bias=True):
+    """(g2^T x2, g2.sum(0) or None) for bf16 g2 [rows, out], x2 [rows, in] through csrc/linear_bf16.cu: one pass over g2
+    gives both; fp32 split-K partials summed in a fixed order (deterministic)."""
+    rows, n = g2.shape
+    k = x2.shape[1]
+    if x2.shape[0] != rows or g2.dtype != torch.bfloat16 or x2.dtype != torch.bfloat16:
+        raise ValueError("linear_bf16_wgrad: bf16 g [rows, out] and x [rows, in] expected")
+    lib = _lib.load()
+    floats = lib.msda_layer_linear_bf16_wgrad_scratch_floats(rows, n, k)
+    if floats == 0:
+        raise ValueError(f"linear_bf16_wgrad: shape rows={rows}, out={n}, in={k} not supported")
+    if not g2.is_contiguous() or g2.data_ptr() % 16 != 0:
+        g2 = g2.contiguous()
+    if not x2.is_contiguous() or x2.data_ptr() % 16 != 0:
+        x2 = x2.contiguous()
+    dw = torch.empty((n, k), dtype=torch.bfloat16, device=g2.device)
+    db = torch.empty(n, dtype=torch.bfloat16, device=g2.device) if with_bias else None
+    scratch = torch.empty(floats, dtype=torch.float32, device=g2.device)
+    with torch.cuda.device(g2.device):
+        code = lib.msda_layer_linear_bf16_wgrad(g2.data_ptr(), x2.data_ptr(), rows, n, k, dw.data_ptr(),
+                                                None if db is None else db.data_ptr(), scratch.data_ptr(), floats,
+                                                torch.cuda.current_stream().cuda_stream)
+    _lib.check(code, "msda_layer_linear_bf16_wgrad")
+    return dw, db
+
+
+def _bf16_linear_backward(needs_input_grad, g2, x2, weight, param_dtypes):
+    """(dx, dW, db) of a bf16 linear layer on the package's kernels; g2 [rows, out] contiguous bf16 (after the ReLU mask),
+    dW / db cast to the parameters' dtypes (autocast)."""
+    # W^T is made from the live weight on every backward (at most 0.5 MB): a cached copy goes stale under .data writes
+    dx = linear_bf16(g2, weight.t().contiguous(), None) if needs_input_grad[0] else None
+    dw = db = None
+    if needs_input_grad[1]:
+        dw, db = linear_bf16_wgrad(g2, x2, with_bias=needs_input_grad[2])
+    elif needs_input_grad[2]:
+        db = column_sum(g2)
+    return dx, (None if dw is None else dw.to(param_dtypes[0])), (None if db is None else db.to(param_dtypes[1]))
 
 
 def linear_wb(x, weight, bias):
@@ -428,12 +504,17 @@ def linear_zero_rows(module, x, zero_rows):
 
 class LinearReLUFunction(Function):
     """relu(x @ W^T + b) with bias and ReLU in the GEMM epilogue (cuBLASLt through
-    torch._addmm_activation): the pre-activation never reaches HBM."""
+    torch._addmm_activation): the pre-activation never reaches HBM.  bf16 training from BF16_TRAIN_KERNEL_MIN_ROWS rows up:
+    the package's own kernels in both directions (_bf16_train_kernels_apply)."""
 
     @staticmethod
     def forward(ctx, x, weight, bias):
         x2 = x.reshape(-1, x.shape[-1])
-        out = torch._addmm_activation(bias, x2, weight.t(), use_gelu=False)
+        ctx.kernels = any(ctx.needs_input_grad) and _bf16_train_kernels_apply(x2, weight, bias)
+        if ctx.kernels:
+            out = linear_bf16(x2, weight, bias, relu=True)
+        else:
+            out = torch._addmm_activation(bias, x2, weight.t(), use_gelu=False)
         ctx.save_for_backward(x2, weight, out)
         ctx.x_shape = x.shape
         return out.view(*x.shape[:-1], weight.shape[0])
@@ -443,9 +524,13 @@ class LinearReLUFunction(Function):
     def backward(ctx, grad):
         x2, weight, out = ctx.saved_tensors
         g = torch.ops.aten.threshold_backward(grad.reshape(out.shape), out, 0)
-        dx = g @ weight if ctx.needs_input_grad[0] else None
-        dw = g.t() @ x2 if ctx.needs_input_grad[1] else None
-        db = column_sum(g) if ctx.needs_input_grad[2] else None
+        if ctx.kernels:
+            dx, dw, db = _bf16_linear_backward(ctx.needs_input_grad, g.contiguous(), x2, weight,
+                                               (weight.dtype, weight.dtype))
+        else:
+            dx = g @ weight if ctx.needs_input_grad[0] else None
+            dw = g.t() @ x2 if ctx.needs_input_grad[1] else None
+            db = column_sum(g) if ctx.needs_input_grad[2] else None
         return (None if dx is None else dx.view(ctx.x_shape)), dw, db
 
 
