@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # MSDA_B200_LIB selects another build of the same ABI (A/B kernel experiments); default: in-tree
 LIB_PATH = os.environ.get("MSDA_B200_LIB") or os.path.join(_HERE, "libmsda_b200.so")
 
-ABI_VERSION = 21
+ABI_VERSION = 22
 DTYPE_F32, DTYPE_F64, DTYPE_BF16, DTYPE_F16 = 0, 1, 2, 3
 FLAG_FORCE_GENERIC = 1
 FLAG_TC = 4
@@ -99,6 +99,12 @@ def load():
     lib.msda_layer_linear_tf32x3_supported.argtypes = [c_int, c_int]
     lib.msda_layer_linear_tf32x3.restype = c_int
     lib.msda_layer_linear_tf32x3.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_int, c_vp, c_vp]
+    lib.msda_layer_linear_tf32x3_wgrad_supported.restype = c_int
+    lib.msda_layer_linear_tf32x3_wgrad_supported.argtypes = [c_int, c_int]
+    lib.msda_layer_linear_tf32x3_wgrad_scratch_floats.restype = c_i64
+    lib.msda_layer_linear_tf32x3_wgrad_scratch_floats.argtypes = [c_i64, c_int, c_int]
+    lib.msda_layer_linear_tf32x3_wgrad.restype = c_int
+    lib.msda_layer_linear_tf32x3_wgrad.argtypes = [c_vp, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_vp]
     lib.msda_layer_sine_coordinates.restype = c_int
     lib.msda_layer_sine_coordinates.argtypes = [c_vp, c_int, c_int, c_int, c_int, c_f, c_vp, c_vp, c_vp]
     lib.msda_layer_sine_position_tokens.restype = c_int

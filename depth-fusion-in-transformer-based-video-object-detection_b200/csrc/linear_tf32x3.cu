@@ -26,6 +26,8 @@
 //                      stages of 48 KB
 #include <cuda.h>
 
+#include <atomic>
+
 #include "msda_common.cuh"
 #include "msda_launch.h"
 #include "umma.cuh"
@@ -359,6 +361,322 @@ cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, 
     const long long clusters = sms / kLtCluster;
     const int grid = (int)(units < clusters ? units : clusters) * kLtCluster;
     linear_tf32x3_kernel<<<grid, kLtThreads, kLtSmem, stream>>>(tm_x, tm_wh, tm_wl, tm_y, bias, rows, n, k, relu, bn);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
+// weight / bias gradient of the same layer (fp32 training):
+//
+//     dW [N, K] = g^T x,   db [N] = sum over rows of g,   g [rows, N], x [rows, K], fp32.
+//
+// The same three-term split, now with BOTH operands activations:  g^T x ~= g_hi^T x_hi + (g_lo^T x_hi + g_hi^T x_lo).
+// The reduction runs over `rows`, so as loaded both operands are MN-major: a TMA box {32 columns, 32 rows} with
+// SWIZZLE_128B is 32 rows of 128 bytes, 32 features (or inputs) x 32 reduction steps.  kind::tf32 does not take MN-major
+// operands: with the transpose bits set it wrote zeros for every descriptor encoding tried, while the same data loaded
+// K-major gave the exact product (tools/umma/tf32_mn_probe.cu, profiles/r4_tf32_mn_probe.txt).  So the converter warps
+// TRANSPOSE: thread f reads column f of the loaded g tile (feature f, 32 rows; conflict-free, a warp reads one 128-byte
+// row per step) and writes row f of the K-major SWIZZLE_128B tiles g_hi^T (the words as loaded; the tensor core truncates
+// them to TF32) and g_lo^T, and the same for x.  An output tile is 128 features (four g boxes, M) x up to 128 inputs (four
+// x boxes, N); every MMA waits for the converter.
+//
+// Accumulator truncation: the tensor core truncates towards zero, about half an ulp of the running sum per instruction
+// (DESIGN.md section 3.5: 32 instructions into one accumulator 6.9e-7 of the output range, 96 gave 2.3e-6).  A slice of
+// ~2 400 rows would be 300 instructions, so (1) the two correction terms go to an accumulator of their own, and (2) the
+// main accumulator is drained every kTwChunk K blocks (kTwChunk * 4 instructions): the epilogue warps add (main +
+// correction) into fp32 registers with round-to-nearest adds while the MMA issuer fills the other accumulator pair.
+// TMEM: pair p = main [256 p, 256 p + 128) | correction [256 p + 128, 256 p + 256) = 512 columns.  Measured on B200
+// (DESIGN.md section 3.14): without the drain dW was up to 4.8e-5 of its range off fp64 at 177 784 rows; with a drain
+// every 8 K blocks 6-9.5e-7 (the IEEE SGEMM: 4.6e-7-2.1e-6), every 2 K blocks 2.8-5.1e-7.
+//
+// The bias gradient comes from the converter warps, which read every g element anyway: thread f owns feature f of the
+// tile and adds the 32 rows of a K block it transposes (a partial sum per K block, then into the slice sum: fixed order).
+// Split-K, scratch layout, the reduce kernel and the determinism argument are those of linear_bf16_wgrad (linear_bf16.cu).
+// Warp roles (14 warps): 0-7 epilogue (warp % 4 = TMEM lane quadrant, warp / 4 = which 64 columns), 8-11 converter,
+// 12 MMA issuer, 13 TMA producer.
+// ------------------------------------------------------------------------------------------
+#ifndef MSDA_TF32_WG_CHUNK
+#define MSDA_TF32_WG_CHUNK 8
+#endif
+constexpr int kTwChunk = MSDA_TF32_WG_CHUNK;   // K blocks (of 32 rows) per drain of the main accumulator: 32 instructions
+constexpr int kTwBM = 128;                  // output features per tile (TMEM lanes)
+constexpr int kTwBN = 128;                  // inputs per tile (TMEM columns of one accumulator)
+constexpr int kTwBK = 32;                   // rows per K block
+constexpr int kTwBox = 32 * kTwBK * 4;      // one {32 columns, 32 rows} fp32 box: 4 KB
+constexpr int kTwOpBytes = 128 * kTwBK * 4;   // one K-major operand tile, 128 rows x 128 bytes: 16 KB
+// stage: g as loaded | x as loaded | g_hi^T | g_lo^T | x_hi^T | x_lo^T (converter) = 96 KB
+constexpr int kTwStageBytes = 6 * kTwOpBytes;
+constexpr int kTwStages = 2;
+static_assert(kTwBM == 128 && kTwBN == 128 && kTwBox * 4 == kTwOpBytes, "four 32-wide boxes per operand tile");
+constexpr int kTwEpiThreads = 256, kTwConvThreads = 128;
+constexpr int kTwThreads = kTwEpiThreads + kTwConvThreads + 64;
+constexpr int kTwSmem = kTwStages * kTwStageBytes + 256;       // + barriers
+static_assert(kTwSmem <= 232448, "exceeds the 227 KB of shared memory a CTA can opt in to");
+static_assert(kTwChunk >= 1, "at least one K block per accumulator drain");
+constexpr int kTwTargetCtas = 148;          // B200 SMs: split count aimed at one CTA per SM, fixed so that the split (and
+                                            // so the rounding of the result) does not depend on the device
+constexpr int kTwMinKBlocks = 8;            // a split reads at least 256 rows: its partial tile is small against its loads
+constexpr long long kTwBlkFloats = (long long)kTwBM * kTwBN + kTwBM;   // partial dW tile + partial db
+
+struct TwBars {
+    unsigned long long full[kTwStages], conv[kTwStages], empty[kTwStages], acc_full[2], acc_free[2];
+    unsigned tmem_base;
+};
+
+// Converter step for one operand: column c (< 128) of the loaded tile (four {32 columns, 32 rows} SWIZZLE_128B boxes) ->
+// row c of the K-major SWIZZLE_128B tiles hi (the words as loaded) and lo (x - x_hi on TF32's 10 mantissa bits, rounded
+// to nearest, so that the tensor core's own truncation of it is a no-op, as in the forward's converter).  Returns the sum
+// of the column (the bias gradient's share of this K block when the operand is g).
+__device__ __forceinline__ float tw_transpose_column(const unsigned char* loaded, unsigned char* hi, unsigned char* lo, int c)
+{
+    const float* box = reinterpret_cast<const float*>(loaded + (c >> 5) * kTwBox);
+    const int chunk = (c & 31) >> 2, word = c & 3;
+    float v[kTwBK];
+#pragma unroll
+    for (int r = 0; r < kTwBK; ++r) v[r] = box[r * 32 + ((chunk ^ (r & 7)) << 2) + word];
+    float sum = 0.f;
+#pragma unroll
+    for (int r = 0; r < kTwBK; ++r) sum += v[r];
+    auto lo_of = [](float x) -> unsigned {
+        const float l = x - __uint_as_float(__float_as_uint(x) & 0xffffe000u);
+        return (__float_as_uint(l) + 0x1000u) & 0xffffe000u;
+    };
+    const unsigned row = (unsigned)((c >> 3) * 1024 + (c & 7) * 128);
+#pragma unroll
+    for (int q = 0; q < kTwBK / 4; ++q) {
+        const unsigned off = row + ((q ^ (c & 7)) << 4);
+        *reinterpret_cast<uint4*>(hi + off) = make_uint4(__float_as_uint(v[4 * q]), __float_as_uint(v[4 * q + 1]),
+                                                         __float_as_uint(v[4 * q + 2]), __float_as_uint(v[4 * q + 3]));
+        *reinterpret_cast<uint4*>(lo + off) = make_uint4(lo_of(v[4 * q]), lo_of(v[4 * q + 1]), lo_of(v[4 * q + 2]),
+                                                         lo_of(v[4 * q + 3]));
+    }
+    return sum;
+}
+
+__global__ void __launch_bounds__(kTwThreads, 1)
+linear_tf32x3_wgrad_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_constant__ CUtensorMap tm_x,
+                           float* __restrict__ partial, long long rows, int N, int K, int tiles_n, int tiles, int splits,
+                           int kb_per_split, int want_db)
+{
+    extern __shared__ __align__(1024) unsigned char smem[];
+    TwBars* bars = reinterpret_cast<TwBars*>(smem + kTwStages * kTwStageBytes);
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // CTAs of one split (same rows) are adjacent: the tiles that share a slice of g or x read it from L2
+    const int split = blockIdx.x / tiles, t = blockIdx.x % tiles;
+    const int m0 = (t / tiles_n) * kTwBM, n0 = (t % tiles_n) * kTwBN;
+    const int m_cur = min(kTwBM, N - m0), n_cur = min(kTwBN, K - n0);
+    const int g_boxes = m_cur / 32, x_boxes = n_cur / 32;
+    const int kblocks = (int)((rows + kTwBK - 1) / kTwBK);
+    const int kb0 = split * kb_per_split, kb1 = min(kb0 + kb_per_split, kblocks);
+    const int chunks = (kb1 - kb0 + kTwChunk - 1) / kTwChunk;
+    const bool with_db = want_db && n0 == 0;
+    float* blk = partial + ((long long)t * splits + split) * kTwBlkFloats;
+
+    if (warp == 0) tmem_alloc(&bars->tmem_base, 512);
+    if (tid == kTwEpiThreads) {
+        for (int i = 0; i < kTwStages; ++i) {
+            mbar_init(&bars->full[i], 1);
+            mbar_init(&bars->conv[i], kTwConvThreads);
+            mbar_init(&bars->empty[i], 1);
+        }
+        for (int i = 0; i < 2; ++i) { mbar_init(&bars->acc_full[i], 1); mbar_init(&bars->acc_free[i], kTwEpiThreads); }
+        fence_mbar_init();
+        tma_prefetch_desc(&tm_g); tma_prefetch_desc(&tm_x);
+    }
+    tcgen05_fence_before();
+    __syncthreads();
+    tcgen05_fence_after();
+    const unsigned tmem = bars->tmem_base;
+
+    if (warp == 13) {
+        // ======================================= TMA producer =======================================
+        if (elect_one()) {
+            // boxes wholly past the last feature / input are not loaded: they only feed accumulator lanes / columns
+            // that are never read.  Rows past the end arrive as zeros (TMA out-of-bounds fill).
+            const unsigned bytes = (unsigned)(g_boxes + x_boxes) * kTwBox;
+            for (int kb = kb0; kb < kb1; ++kb) {
+                const int i = kb - kb0, s = i % kTwStages;
+                if (i >= kTwStages) mbar_wait(&bars->empty[s], ((i / kTwStages) - 1) & 1);
+                unsigned char* st = smem + s * kTwStageBytes;
+                mbar_expect_tx(&bars->full[s], bytes);
+                for (int c = 0; c < g_boxes; ++c) tma_load_2d(st + c * kTwBox, &tm_g, m0 + 32 * c, kb * kTwBK, &bars->full[s]);
+                for (int c = 0; c < x_boxes; ++c)
+                    tma_load_2d(st + kTwOpBytes + c * kTwBox, &tm_x, n0 + 32 * c, kb * kTwBK, &bars->full[s]);
+            }
+        }
+        __syncwarp();
+    } else if (warp == 12) {
+        // ======================================= MMA issuer =======================================
+        const unsigned idesc = make_idesc_tf32(kTwBM, n_cur);
+        for (int kb = kb0; kb < kb1; ++kb) {
+            const int i = kb - kb0, s = i % kTwStages, chunk = i / kTwChunk, p = chunk & 1;
+            const bool chunk_first = i % kTwChunk == 0, chunk_last = i % kTwChunk == kTwChunk - 1 || kb == kb1 - 1;
+            const unsigned acc_main = tmem + p * 256, acc_corr = acc_main + kTwBN;
+            // the epilogue has drained this pair (chunk - 2)
+            if (chunk_first && chunk >= 2) mbar_wait(&bars->acc_free[p], ((chunk >> 1) - 1) & 1);
+            unsigned char* st = smem + s * kTwStageBytes;
+            const unsigned long long d_gh = make_desc_sw128(st + 2 * kTwOpBytes), d_gl = make_desc_sw128(st + 3 * kTwOpBytes);
+            const unsigned long long d_xh = make_desc_sw128(st + 4 * kTwOpBytes), d_xl = make_desc_sw128(st + 5 * kTwOpBytes);
+            mbar_wait(&bars->conv[s], (i / kTwStages) & 1);                  // K-major hi / lo tiles written
+            tcgen05_fence_after();
+            if (elect_one()) {
+#pragma unroll
+                for (int j = 0; j < kTwBK / 8; ++j) {                        // K = 8 per instruction: 32 bytes of the row
+                    const bool acc = !chunk_first || j != 0;
+                    mma_tf32(acc_main, desc_advance(d_gh, j * 32), desc_advance(d_xh, j * 32), idesc, acc);
+                    mma_tf32(acc_corr, desc_advance(d_gl, j * 32), desc_advance(d_xh, j * 32), idesc, acc);
+                    mma_tf32(acc_corr, desc_advance(d_gh, j * 32), desc_advance(d_xl, j * 32), idesc, true);
+                }
+                mma_commit(&bars->empty[s]);                                 // stage free once these MMAs are done
+                if (chunk_last) mma_commit(&bars->acc_full[p]);
+            }
+            __syncwarp();
+        }
+    } else if (warp >= 8) {
+        // ======================================= converter warps =======================================
+        // thread ct transposes feature ct of the g tile and input ct of the x tile (columns past the loaded boxes are
+        // left alone: they only feed accumulator lanes / columns that are never read)
+        const int ct = tid - kTwEpiThreads;
+        float db = 0.f;
+        for (int kb = kb0; kb < kb1; ++kb) {
+            const int i = kb - kb0, s = i % kTwStages;
+            mbar_wait(&bars->full[s], (i / kTwStages) & 1);
+            unsigned char* st = smem + s * kTwStageBytes;
+            if (ct < m_cur) db += tw_transpose_column(st, st + 2 * kTwOpBytes, st + 3 * kTwOpBytes, ct);
+            if (ct < n_cur) tw_transpose_column(st + kTwOpBytes, st + 4 * kTwOpBytes, st + 5 * kTwOpBytes, ct);
+            fence_proxy_async();                     // generic-proxy writes -> tensor-core (async proxy) reads
+            mbar_arrive(&bars->conv[s]);
+        }
+        if (with_db && ct < m_cur) blk[(long long)kTwBM * kTwBN + ct] = db;
+    } else {
+        // ======================================= epilogue warps =======================================
+        // TMEM lane = feature row of the tile; this warp's 64 columns of it summed over the chunks in registers
+        const int quad = warp & 3, half = warp >> 2, r = quad * 32 + lane;
+        const unsigned lane_base = (unsigned)(quad * 32) << 16;
+        float sum[64];
+#pragma unroll
+        for (int c = 0; c < 64; ++c) sum[c] = 0.f;
+        for (int chunk = 0; chunk < chunks; ++chunk) {
+            const int p = chunk & 1;
+            mbar_wait(&bars->acc_full[p], (chunk >> 1) & 1);
+            tcgen05_fence_after();
+#pragma unroll
+            for (int c = 0; c < 64; c += 16) {
+                if (half * 64 + c < n_cur) {
+                    float v[16], w[16];
+                    tmem_ld16(tmem + p * 256 + half * 64 + c + lane_base, v);
+                    tmem_ld16(tmem + p * 256 + kTwBN + half * 64 + c + lane_base, w);
+#pragma unroll
+                    for (int e = 0; e < 16; ++e) sum[c + e] += v[e] + w[e];
+                }
+            }
+            tcgen05_fence_before();
+            mbar_arrive(&bars->acc_free[p]);
+        }
+        float4* dst = reinterpret_cast<float4*>(blk + (long long)r * kTwBN + half * 64);
+#pragma unroll
+        for (int q = 0; q < 16; ++q)
+            if (half * 64 + 4 * q < n_cur) dst[q] = make_float4(sum[4 * q], sum[4 * q + 1], sum[4 * q + 2], sum[4 * q + 3]);
+    }
+    tcgen05_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_free(tmem, 512);
+}
+
+// dW / db = sum over the splits of the partial blocks, in split order.  Block (32, 8): x = 4 consecutive outputs, y = every
+// 8th split; the 8 sums are added in y order.
+__global__ void __launch_bounds__(256)
+linear_tf32x3_wgrad_reduce_kernel(const float* __restrict__ partial, float* __restrict__ dw, float* __restrict__ db, int N,
+                                  int K, int tiles_n, int splits)
+{
+    __shared__ float4 s_sum[8][32];
+    const long long q = (long long)blockIdx.x * 32 + threadIdx.x;        // quad of outputs
+    const long long qw = (long long)N * K / 4, qb = db != nullptr ? N / 4 : 0;
+    long long base = -1;
+    float* dst = nullptr;
+    if (q < qw) {
+        const long long e = q * 4;
+        const int o = (int)(e / K), i = (int)(e % K);
+        base = ((long long)((o / kTwBM) * tiles_n + i / kTwBN) * splits) * kTwBlkFloats + (long long)(o % kTwBM) * kTwBN + i % kTwBN;
+        dst = dw + e;
+    } else if (q < qw + qb) {
+        const int o = (int)(q - qw) * 4;
+        base = ((long long)((o / kTwBM) * tiles_n) * splits) * kTwBlkFloats + (long long)kTwBM * kTwBN + o % kTwBM;
+        dst = db + o;
+    }
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (base >= 0)
+        for (int s = threadIdx.y; s < splits; s += 8) {
+            const float4 v = __ldg(reinterpret_cast<const float4*>(partial + base + (long long)s * kTwBlkFloats));
+            acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+        }
+    s_sum[threadIdx.y][threadIdx.x] = acc;
+    __syncthreads();
+    if (threadIdx.y != 0 || base < 0) return;
+#pragma unroll
+    for (int y = 1; y < 8; ++y) {
+        const float4 v = s_sum[y][threadIdx.x];
+        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    }
+    *reinterpret_cast<float4*>(dst) = acc;
+}
+
+bool linear_tf32x3_wgrad_supported(int n, int k)
+{
+    return n >= 32 && n % 32 == 0 && k >= 32 && k % 32 == 0;
+}
+
+struct TwPlan {
+    int tiles_n, tiles, splits, kb_per_split;
+};
+
+static bool tf32x3_wgrad_plan(long long rows, int n, int k, TwPlan* p)
+{
+    if (!linear_tf32x3_wgrad_supported(n, k) || rows < 1 || rows >= (1ll << 31) - 1024) return false;
+    p->tiles_n = (k + kTwBN - 1) / kTwBN;
+    p->tiles = ((n + kTwBM - 1) / kTwBM) * p->tiles_n;
+    const int kblocks = (int)((rows + kTwBK - 1) / kTwBK);
+    const int want = max(1, kTwTargetCtas / p->tiles);
+    p->kb_per_split = max(kTwMinKBlocks, (kblocks + want - 1) / want);
+    p->splits = (kblocks + p->kb_per_split - 1) / p->kb_per_split;     // every split has at least one K block
+    return true;
+}
+
+long long linear_tf32x3_wgrad_scratch_floats(long long rows, int n, int k)
+{
+    TwPlan p;
+    return tf32x3_wgrad_plan(rows, n, k, &p) ? (long long)p.tiles * p.splits * kTwBlkFloats : 0;
+}
+
+cudaError_t linear_tf32x3_wgrad(const float* g, const float* x, long long rows, int n, int k, float* dw, float* db,
+                                float* scratch, long long scratch_floats, cudaStream_t stream)
+{
+    TwPlan p;
+    if (!tf32x3_wgrad_plan(rows, n, k, &p) || scratch_floats < (long long)p.tiles * p.splits * kTwBlkFloats || dw == nullptr)
+        return cudaErrorInvalidValue;
+    if ((reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dw) |
+         reinterpret_cast<uintptr_t>(db) | reinterpret_cast<uintptr_t>(scratch)) % 16 != 0)
+        return cudaErrorInvalidValue;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    // the attribute is per device; concurrent first calls may both set it (harmless), none reads a torn flag
+    static std::atomic<bool> configured[64];
+    if (dev < 0 || dev >= 64 || !configured[dev].load(std::memory_order_acquire)) {
+        cudaError_t e = cudaFuncSetAttribute(linear_tf32x3_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTwSmem);
+        if (e != cudaSuccess) return e;
+        if (dev >= 0 && dev < 64) configured[dev].store(true, std::memory_order_release);
+    }
+    alignas(64) CUtensorMap tm_g, tm_x;
+    if (!lt_make_map(&tm_g, g, (unsigned long long)rows, (unsigned long long)n, kTwBK, 32) ||
+        !lt_make_map(&tm_x, x, (unsigned long long)rows, (unsigned long long)k, kTwBK, 32))
+        return cudaErrorNotSupported;
+    linear_tf32x3_wgrad_kernel<<<p.tiles * p.splits, kTwThreads, kTwSmem, stream>>>(
+        tm_g, tm_x, scratch, rows, n, k, p.tiles_n, p.tiles, p.splits, p.kb_per_split, db != nullptr);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const long long quads = (long long)n * k / 4 + (db != nullptr ? n / 4 : 0);
+    linear_tf32x3_wgrad_reduce_kernel<<<(unsigned)((quads + 31) / 32), dim3(32, 8), 0, stream>>>(scratch, dw, db, n, k,
+                                                                                                p.tiles_n, p.splits);
     return cudaGetLastError();
 }
 

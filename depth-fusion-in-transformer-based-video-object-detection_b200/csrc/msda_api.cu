@@ -7,7 +7,7 @@ static bool bad_dims(int N, int S, int M, int D, int L, int Lq, int P)
     return N < 0 || S < 0 || M < 0 || D < 0 || L < 0 || Lq < 0 || P < 0;
 }
 
-extern "C" int msda_abi_version(void) { return 21; }
+extern "C" int msda_abi_version(void) { return 22; }
 
 extern "C" const char* msda_error_string(int code)
 {
@@ -422,4 +422,22 @@ extern "C" int msda_layer_linear_tf32x3(const float* x, const float* weight_hi, 
     if (rows < 0) return (int)cudaErrorInvalidValue;
     return (int)msda::linear_tf32x3(x, weight_hi, weight_lo, bias, (long long)rows, out_features, in_features, relu, y,
                                     (cudaStream_t)stream);
+}
+
+extern "C" int msda_layer_linear_tf32x3_wgrad_supported(int out_features, int in_features)
+{
+    return msda::linear_tf32x3_wgrad_supported(out_features, in_features) ? 1 : 0;
+}
+
+extern "C" int64_t msda_layer_linear_tf32x3_wgrad_scratch_floats(int64_t rows, int out_features, int in_features)
+{
+    return (int64_t)msda::linear_tf32x3_wgrad_scratch_floats((long long)rows, out_features, in_features);
+}
+
+extern "C" int msda_layer_linear_tf32x3_wgrad(const float* grad_y, const float* x, int64_t rows, int out_features,
+                                              int in_features, float* grad_weight, float* grad_bias, float* scratch,
+                                              int64_t scratch_floats, void* stream)
+{
+    return (int)msda::linear_tf32x3_wgrad(grad_y, x, (long long)rows, out_features, in_features, grad_weight, grad_bias,
+                                          scratch, (long long)scratch_floats, (cudaStream_t)stream);
 }

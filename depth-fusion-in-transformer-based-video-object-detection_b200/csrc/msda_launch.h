@@ -183,6 +183,12 @@ cudaError_t linear_bf16_wgrad(const void* g, const void* x, long long rows, int 
 bool linear_tf32x3_supported(int n, int k);
 cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, const float* bias, long long rows, int n,
                           int k, int relu, float* y, cudaStream_t stream);
+// weight / bias gradient of that layer: dW [n, k] = g^T x, db [n] = sum over rows of g (fp32, the three-term split with
+// both operands split in shared memory; fp32 split-K partials in `scratch`, summed in a fixed order: deterministic)
+bool linear_tf32x3_wgrad_supported(int n, int k);
+long long linear_tf32x3_wgrad_scratch_floats(long long rows, int n, int k);   // 0 = unsupported
+cudaError_t linear_tf32x3_wgrad(const float* g, const float* x, long long rows, int n, int k, float* dw, float* db,
+                                float* scratch, long long scratch_floats, cudaStream_t stream);
 cudaError_t sine_coordinates(const unsigned char* mask, float* y_embed, float* x_embed, int N, int H, int W,
                              int normalize, float scale, cudaStream_t stream);
 cudaError_t sine_position_tokens(int dtype, const float* y_embed, const float* x_embed, const float* dim_t,

@@ -214,7 +214,8 @@ def column_sum(g2):
 class LinearFunction(Function):
     """x @ W^T + b as the library GEMM, with a backward that takes the bias gradient from the
     column-sum kernel instead of PyTorch's generic reduction.  bf16 training from BF16_TRAIN_KERNEL_MIN_ROWS rows up:
-    the package's own kernels in both directions (_bf16_train_kernels_apply)."""
+    the package's own kernels in both directions (_bf16_train_kernels_apply); fp32 training in fp32 train-GEMM mode
+    "tf32x3": the three-term TF32 kernels in both directions (_fp32_train_kernels_apply)."""
 
     @staticmethod
     def forward(ctx, x2, weight, bias):              # x2 [rows, in] -> fresh [rows, out] (never a view)
@@ -228,8 +229,11 @@ class LinearFunction(Function):
         ctx.save_for_backward(x2, weight_c)
         ctx.param_dtypes = (weight.dtype, bias.dtype)
         ctx.kernels = any(ctx.needs_input_grad) and _bf16_train_kernels_apply(x2, weight_c, bias_c)
+        ctx.tf32x3 = not ctx.kernels and any(ctx.needs_input_grad) and _fp32_train_kernels_apply(x2, weight_c, bias_c)
         if ctx.kernels:
             return linear_bf16(x2, weight_c, bias_c)
+        if ctx.tf32x3:
+            return _linear_tf32x3_kernel(x2, *_tf32_weight_split(weight_c, live=True), bias_c)
         return torch.addmm(bias_c, x2, weight_c.t())
 
     @staticmethod
@@ -242,6 +246,8 @@ class LinearFunction(Function):
             g2 = g2.to(weight.dtype)
         if ctx.kernels:
             return _bf16_linear_backward(ctx.needs_input_grad, g2, x2, weight, ctx.param_dtypes)
+        if ctx.tf32x3:
+            return _tf32x3_linear_backward(ctx.needs_input_grad, g2, x2, weight)
         dx = g2 @ weight if ctx.needs_input_grad[0] else None
         dw = (g2.t() @ x2).to(ctx.param_dtypes[0]) if ctx.needs_input_grad[1] else None
         db = column_sum(g2).to(ctx.param_dtypes[1]) if ctx.needs_input_grad[2] else None
@@ -295,17 +301,20 @@ def _tf32x3_wanted(x, weight):
             and not (torch.is_grad_enabled() and (x.requires_grad or weight.requires_grad)))
 
 
-def _tf32_weight_split(weight):
+def _tf32_weight_split(weight, live=False):
     """weight -> (hi, lo): hi = weight rounded to TF32's 10 mantissa bits (nearest, ties away), lo = weight - hi (exact).
     Cached ON the weight tensor (weights are static in inference) together with the version counter it was made from:
-    the cache dies with the tensor, and an in-place update (optimizer step, load_state_dict) invalidates it."""
+    the cache dies with the tensor, and an in-place update (optimizer step, load_state_dict) invalidates it.
+    live=True (training): under CUDA-graph capture the split is always made inside the graph, never taken from the cache,
+    so that every replay splits the weights as the optimizer left them (its in-place updates happen outside the graph)."""
     hit = getattr(weight, "_dfvod_tf32_split", None)
-    if hit is None or hit[0] != weight._version or hit[1].device != weight.device:
+    capturing = weight.is_cuda and torch.cuda.is_current_stream_capturing()
+    if hit is None or hit[0] != weight._version or hit[1].device != weight.device or (live and capturing):
         w = weight.detach().contiguous()
         hi = ((w.view(torch.int32) + 0x1000) & -0x2000).view(torch.float32)
         hit = (weight._version, hi, w - hi)
         # (tensors made during a CUDA-graph capture live in the graph's private pool: never cache those)
-        if not (weight.is_cuda and torch.cuda.is_current_stream_capturing()):
+        if not capturing:
             try:
                 weight._dfvod_tf32_split = hit
             except (AttributeError, RuntimeError):      # a tensor that takes no attributes: split every call
@@ -326,24 +335,29 @@ def _tf32x3_kernel_wins(n, k):
     return True
 
 
+def _linear_tf32x3_kernel(x2, w_hi, w_lo, bias, relu=False):
+    """x2 [rows, k] @ (w_hi + w_lo)^T + bias -> a fresh [rows, n] (ReLU) on csrc/linear_tf32x3.cu; (w_hi, w_lo) [n, k]
+    contiguous, the TF32 split of a weight (_tf32_weight_split) or of its transpose."""
+    n, k = w_hi.shape
+    if not x2.is_contiguous() or x2.data_ptr() % 16 != 0:
+        x2 = x2.contiguous()
+    b = None if bias is None else bias.detach().contiguous()
+    y = torch.empty((x2.shape[0], n), dtype=torch.float32, device=x2.device)
+    with torch.cuda.device(x2.device):
+        code = _lib.load().msda_layer_linear_tf32x3(x2.data_ptr(), w_hi.data_ptr(), w_lo.data_ptr(),
+                                                    None if b is None else b.data_ptr(), x2.shape[0], n, k,
+                                                    1 if relu else 0, y.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(code, "msda_layer_linear_tf32x3")
+    return y
+
+
 def linear_tf32x3(x, weight, bias, relu=False, route=None):
     """route: None = the faster of the two for the shape, "kernel" / "library" to force one (tests, measurements)."""
     k = x.shape[-1]
     use_kernel = linear_tf32x3_kernel_supported(x, weight) and route != "library" and (
         route == "kernel" or _tf32x3_kernel_wins(weight.shape[0], k))
     if use_kernel:
-        x2 = x.reshape(-1, k)
-        if not x2.is_contiguous() or x2.data_ptr() % 16 != 0:
-            x2 = x2.contiguous()
-        w_hi, w_lo = _tf32_weight_split(weight)
-        b = None if bias is None else bias.detach().contiguous()
-        y = torch.empty((x2.shape[0], weight.shape[0]), dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            code = _lib.load().msda_layer_linear_tf32x3(x2.data_ptr(), w_hi.data_ptr(), w_lo.data_ptr(),
-                                                        None if b is None else b.data_ptr(), x2.shape[0],
-                                                        weight.shape[0], k, 1 if relu else 0, y.data_ptr(),
-                                                        torch.cuda.current_stream().cuda_stream)
-        _lib.check(code, "msda_layer_linear_tf32x3")
+        y = _linear_tf32x3_kernel(x.reshape(-1, k), *_tf32_weight_split(weight), bias, relu)
         return y.view(*x.shape[:-1], weight.shape[0])
     # shapes the kernel does not take: the same split as ONE library TF32 GEMM over the concatenated reduction
     a = _tf32_split(x.reshape(-1, k).contiguous())                       # [rows, 3k] = [lo | hi | hi]
@@ -471,6 +485,97 @@ def _bf16_linear_backward(needs_input_grad, g2, x2, weight, param_dtypes):
     return dx, (None if dw is None else dw.to(param_dtypes[0])), (None if db is None else db.to(param_dtypes[1]))
 
 
+# fp32 training (the backward, and the forward of a layer whose gradients flow):
+#   "library"  (default) torch's GEMMs, IEEE SGEMM unless the caller allowed TF32: the reference's own arithmetic, bit for
+#              bit.  fp32 training is compared against it, so it stays the default until an fp32 convergence comparison
+#              says otherwise.
+#   "tf32x3"   the three-term TF32 kernels of csrc/linear_tf32x3.cu in both directions, from FP32_TRAIN_KERNEL_MIN_ROWS rows
+#              up at the shapes where they were measured faster (_fp32_train_kernels_win): forward y = x W^T + b and
+#              dx = g W are linear_tf32x3 (with the split of W^T as the weight pair for dx), dW = g^T x and db = sum g
+#              one linear_tf32x3_wgrad (both operands split in shared memory, g read once).  fp32-grade, not bit for
+#              bit the SGEMM: within 1e-5 of fp64 like the library (tests/test_gpu_linear_tf32x3_train.py).
+# A different numerical contract, not a faster route to the same bits: like FP32_GEMM_MODE, the caller chooses.
+# FP32_TRAIN_KERNEL_MIN_ROWS: the smallest row count measured (tools/bench_train_fp32.py, DESIGN.md section 3.14); every
+# shape of the model was already faster on the kernels there (backward 1.17-1.71x, forward 1.48-2.84x on one B200).
+# Graphed fp32 Encoder-Cross-Fusion training step, 4 frames: 106.2 ms in mode "library", 44.1 ms in mode "tf32x3".
+FP32_TRAIN_GEMM_MODE = "library"
+FP32_TRAIN_KERNEL_MIN_ROWS = 2400
+
+
+def set_fp32_train_gemm_mode(mode):
+    """Selects how fp32 training evaluates the linear layers ("library" or "tf32x3"); returns the previous mode."""
+    global FP32_TRAIN_GEMM_MODE
+    if mode not in ("library", "tf32x3"):
+        raise ValueError(f"unknown fp32 training GEMM mode {mode!r}")
+    previous, FP32_TRAIN_GEMM_MODE = FP32_TRAIN_GEMM_MODE, mode
+    return previous
+
+
+def _fp32_train_kernels_win(n, k):
+    """Shapes where forward + dx + dW + db on the kernels beat the SGEMM path.  Measured on B200 (tools/bench_train_fp32.py,
+    DESIGN.md section 3.14) at 2 400, 88 892 and 177 784 rows: every shape of the model wins (256 <- 256, 384 <- 256,
+    1024 <- 256 and 256 <- 1024; backward 1.17-3.60x, forward 1.48-6.19x), so none is excluded."""
+    return True
+
+
+def _fp32_train_kernels_apply(x2, weight, bias):
+    """Mode "tf32x3", gradients flow (checked by the caller), the operands as multiplied are CUDA fp32 (not under
+    autocast), enough rows, a shape where the kernels are faster, and the forward, input-gradient and weight-gradient
+    kernels all take it."""
+    if (FP32_TRAIN_GEMM_MODE != "tf32x3" or FP32_TRAIN_KERNEL_MIN_ROWS is None or not x2.is_cuda
+            or x2.shape[0] < FP32_TRAIN_KERNEL_MIN_ROWS or torch.is_autocast_enabled()):
+        return False
+    if x2.dtype != torch.float32 or weight.dtype != torch.float32 or (bias is not None and bias.dtype != torch.float32):
+        return False
+    n, k = weight.shape
+    lib = _lib.load()
+    return (x2.shape[1] == k and _fp32_train_kernels_win(n, k) and bool(lib.msda_layer_linear_tf32x3_supported(n, k))
+            and bool(lib.msda_layer_linear_tf32x3_supported(k, n))
+            and bool(lib.msda_layer_linear_tf32x3_wgrad_supported(n, k)))
+
+
+def linear_tf32x3_wgrad(g2, x2, with_bias=True):
+    """(g2^T x2, g2.sum(0) or None) for fp32 g2 [rows, out], x2 [rows, in] through csrc/linear_tf32x3.cu: the three-term
+    TF32 split of both operands, fp32-grade; one pass over g2 gives both; split-K partials summed in a fixed order
+    (deterministic)."""
+    rows, n = g2.shape
+    k = x2.shape[1]
+    if x2.shape[0] != rows or g2.dtype != torch.float32 or x2.dtype != torch.float32:
+        raise ValueError("linear_tf32x3_wgrad: fp32 g [rows, out] and x [rows, in] expected")
+    lib = _lib.load()
+    floats = lib.msda_layer_linear_tf32x3_wgrad_scratch_floats(rows, n, k)
+    if floats == 0:
+        raise ValueError(f"linear_tf32x3_wgrad: shape rows={rows}, out={n}, in={k} not supported")
+    if not g2.is_contiguous() or g2.data_ptr() % 16 != 0:
+        g2 = g2.contiguous()
+    if not x2.is_contiguous() or x2.data_ptr() % 16 != 0:
+        x2 = x2.contiguous()
+    dw = torch.empty((n, k), dtype=torch.float32, device=g2.device)
+    db = torch.empty(n, dtype=torch.float32, device=g2.device) if with_bias else None
+    scratch = torch.empty(floats, dtype=torch.float32, device=g2.device)
+    with torch.cuda.device(g2.device):
+        code = lib.msda_layer_linear_tf32x3_wgrad(g2.data_ptr(), x2.data_ptr(), rows, n, k, dw.data_ptr(),
+                                                  None if db is None else db.data_ptr(), scratch.data_ptr(), floats,
+                                                  torch.cuda.current_stream().cuda_stream)
+    _lib.check(code, "msda_layer_linear_tf32x3_wgrad")
+    return dw, db
+
+
+def _tf32x3_linear_backward(needs_input_grad, g2, x2, weight):
+    """(dx, dW, db) of an fp32 linear layer on the three-term TF32 kernels; g2 [rows, out] contiguous fp32 (after the ReLU
+    mask)."""
+    dx = dw = db = None
+    if needs_input_grad[0]:
+        # the transpose of the split is the split of the transpose: (W_hi^T, W_lo^T) is the weight pair of dx = g W
+        w_hi, w_lo = _tf32_weight_split(weight, live=True)
+        dx = _linear_tf32x3_kernel(g2, w_hi.t().contiguous(), w_lo.t().contiguous(), None)
+    if needs_input_grad[1]:
+        dw, db = linear_tf32x3_wgrad(g2, x2, with_bias=needs_input_grad[2])
+    elif needs_input_grad[2]:
+        db = column_sum(g2)
+    return dx, dw, db
+
+
 def linear_wb(x, weight, bias):
     """``F.linear(x, weight, bias)``: same GEMM; the custom backward only when gradients flow."""
     if _tf32x3_wanted(x, weight):
@@ -505,14 +610,18 @@ def linear_zero_rows(module, x, zero_rows):
 class LinearReLUFunction(Function):
     """relu(x @ W^T + b) with bias and ReLU in the GEMM epilogue (cuBLASLt through
     torch._addmm_activation): the pre-activation never reaches HBM.  bf16 training from BF16_TRAIN_KERNEL_MIN_ROWS rows up:
-    the package's own kernels in both directions (_bf16_train_kernels_apply)."""
+    the package's own kernels in both directions (_bf16_train_kernels_apply); fp32 training in fp32 train-GEMM mode
+    "tf32x3": the three-term TF32 kernels in both directions (_fp32_train_kernels_apply)."""
 
     @staticmethod
     def forward(ctx, x, weight, bias):
         x2 = x.reshape(-1, x.shape[-1])
         ctx.kernels = any(ctx.needs_input_grad) and _bf16_train_kernels_apply(x2, weight, bias)
+        ctx.tf32x3 = not ctx.kernels and any(ctx.needs_input_grad) and _fp32_train_kernels_apply(x2, weight, bias)
         if ctx.kernels:
             out = linear_bf16(x2, weight, bias, relu=True)
+        elif ctx.tf32x3:
+            out = _linear_tf32x3_kernel(x2, *_tf32_weight_split(weight, live=True), bias, relu=True)
         else:
             out = torch._addmm_activation(bias, x2, weight.t(), use_gelu=False)
         ctx.save_for_backward(x2, weight, out)
@@ -527,6 +636,8 @@ class LinearReLUFunction(Function):
         if ctx.kernels:
             dx, dw, db = _bf16_linear_backward(ctx.needs_input_grad, g.contiguous(), x2, weight,
                                                (weight.dtype, weight.dtype))
+        elif ctx.tf32x3:
+            dx, dw, db = _tf32x3_linear_backward(ctx.needs_input_grad, g.contiguous(), x2, weight)
         else:
             dx = g @ weight if ctx.needs_input_grad[0] else None
             dw = g.t() @ x2 if ctx.needs_input_grad[1] else None

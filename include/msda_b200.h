@@ -280,6 +280,24 @@ int msda_layer_linear_bf16(const void* x, const void* weight, const void* bias, 
 int msda_layer_linear_tf32x3(const float* x, const float* weight_hi, const float* weight_lo, const float* bias,
                              int64_t rows, int out_features, int in_features, int relu, float* y, void* stream);
 
+/* Weight and bias gradient of that FP32 nn.Linear (training), at the same fp32 grade: grad_weight [out_features,
+ * in_features] = grad_y^T x and grad_bias [out_features] = grad_y summed over the rows, from grad_y [rows, out_features]
+ * and x [rows, in_features], all FP32 row-major.  Both operands are split into TF32 hi / lo parts in shared memory and
+ * the product is g_hi^T x_hi + g_lo^T x_hi + g_hi^T x_lo on the tcgen05 tensor cores; the main accumulator is drained
+ * into fp32 registers every 256 rows, so the tensor core's truncating accumulation does not build up over long
+ * reductions.  One pass over grad_y gives both outputs.  The rows are split into slices whose fp32 partial sums go to
+ * `scratch` (scratch_floats >= msda_layer_linear_tf32x3_wgrad_scratch_floats(rows, ...), 0 = shape not supported), then
+ * a second kernel adds them in a fixed order: two calls on the same inputs give the same bits.  grad_bias may be NULL.
+ * out_features % 32 == 0, in_features % 32 == 0 (both >= 32), rows >= 1, 16-byte aligned buffers;
+ * cudaErrorInvalidValue otherwise.  Stream-ordered on `stream`, no allocation, no synchronisation (can be captured in a
+ * CUDA graph).  The input gradient grad_x = grad_y weight is msda_layer_linear_tf32x3 with the split of weight^T
+ * [in_features, out_features] as its weight pair. */
+int msda_layer_linear_tf32x3_wgrad_supported(int out_features, int in_features);
+int64_t msda_layer_linear_tf32x3_wgrad_scratch_floats(int64_t rows, int out_features, int in_features);
+int msda_layer_linear_tf32x3_wgrad(const float* grad_y, const float* x, int64_t rows, int out_features, int in_features,
+                                   float* grad_weight, float* grad_bias, float* scratch, int64_t scratch_floats,
+                                   void* stream);
+
 /* Weight and bias gradient of that BF16 nn.Linear (training): grad_weight [out_features, in_features] = grad_y^T x and
  * grad_bias [out_features] = grad_y summed over the rows, from grad_y [rows, out_features] and x [rows, in_features], all
  * BF16 row-major, fp32 accumulation on the tcgen05 tensor cores.  One pass over grad_y gives both: the bias gradient is
