@@ -15,7 +15,9 @@ Deviations from the reference, all deliberate (DESIGN.md "Boundary"):
     reference silently mis-indexes on a level-count mismatch (SURVEY.md section 9.1);
   * kernel launch failures raise instead of being printf'ed (cuh:948-952);
   * the batch is processed in one launch; ``im2col_step`` only keeps its divisibility check
-    (cu:50-52).
+    (cu:50-52);
+  * under ``torch.use_deterministic_algorithms(True)`` the backward runs ``msda_backward_deterministic``
+    (fixed-point accumulation of grad_value, bitwise reproducible; DESIGN.md section 3.15).
 """
 import torch
 
@@ -112,15 +114,19 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
         grad_value = torch.empty_like(value)
         grad_loc = torch.empty_like(sampling_loc)
         grad_attn = torch.empty_like(attn_weight)
-        accum = None
-        if value.dtype in (torch.bfloat16, torch.float16):
-            accum = torch.empty(value.shape, dtype=torch.float32, device=value.device)
-        code = lib.msda_backward(
-            _DTYPES[value.dtype], grad_output.data_ptr(), value.data_ptr(), spatial_shapes.data_ptr(),
-            level_start_index.data_ptr(), sampling_loc.data_ptr(), attn_weight.data_ptr(),
-            n, s, m, d, nl, lq, p, grad_value.data_ptr(), grad_loc.data_ptr(), grad_attn.data_ptr(),
-            accum.data_ptr() if accum is not None else None,
-            _lib.FLAG_FORCE_GENERIC if _FORCE_GENERIC else 0, torch.cuda.current_stream().cuda_stream)
+        args = (_DTYPES[value.dtype], grad_output.data_ptr(), value.data_ptr(), spatial_shapes.data_ptr(),
+                level_start_index.data_ptr(), sampling_loc.data_ptr(), attn_weight.data_ptr(),
+                n, s, m, d, nl, lq, p, grad_value.data_ptr(), grad_loc.data_ptr(), grad_attn.data_ptr())
+        flags = _lib.FLAG_FORCE_GENERIC if _FORCE_GENERIC else 0
+        stream = torch.cuda.current_stream().cuda_stream
+        if torch.are_deterministic_algorithms_enabled():
+            scratch = _lib.deterministic_scratch(value.device, value.numel())
+            code = lib.msda_backward_deterministic(*args, None, flags, scratch.data_ptr(), scratch.numel(), stream)
+        else:
+            accum = None
+            if value.dtype in (torch.bfloat16, torch.float16):
+                accum = torch.empty(value.shape, dtype=torch.float32, device=value.device)
+            code = lib.msda_backward(*args, accum.data_ptr() if accum is not None else None, flags, stream)
     _lib.check(code, "ms_deform_attn_backward")
     if grad_loc.dtype != loc_dtype:
         grad_loc = grad_loc.to(loc_dtype)

@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # MSDA_B200_LIB selects another build of the same ABI (A/B kernel experiments); default: in-tree
 LIB_PATH = os.environ.get("MSDA_B200_LIB") or os.path.join(_HERE, "libmsda_b200.so")
 
-ABI_VERSION = 22
+ABI_VERSION = 23
 DTYPE_F32, DTYPE_F64, DTYPE_BF16, DTYPE_F16 = 0, 1, 2, 3
 FLAG_FORCE_GENERIC = 1
 FLAG_TC = 4
@@ -54,6 +54,12 @@ def load():
     lib.msda_fused_forward_strided.argtypes = [c_int, c_int, c_vp, c_i64] + fused_common[1:] + [c_vp, c_vp]
     lib.msda_fused_backward.restype = c_int
     lib.msda_fused_backward.argtypes = [c_int, c_int, c_vp] + fused_common + [c_vp, c_vp, c_vp, c_fp, c_vp, c_vp]
+    lib.msda_deterministic_scratch_bytes.restype = c_i64
+    lib.msda_deterministic_scratch_bytes.argtypes = [c_i64, c_i64, c_int]
+    lib.msda_backward_deterministic.restype = c_int
+    lib.msda_backward_deterministic.argtypes = lib.msda_backward.argtypes[:-1] + [c_vp, c_i64, c_vp]
+    lib.msda_fused_backward_deterministic.restype = c_int
+    lib.msda_fused_backward_deterministic.argtypes = lib.msda_fused_backward.argtypes[:-1] + [c_vp, c_i64, c_vp]
     lib.msda_fused_forward_head_major.restype = c_int
     lib.msda_fused_forward_head_major.argtypes = [c_int, c_int] + fused_common + [c_vp, c_vp]
     lib.msda_layer_value_proj_head_major_supported.restype = c_int
@@ -79,6 +85,8 @@ def load():
     for fn in (lib.msda_roi_align_forward, lib.msda_roi_align_backward):
         fn.restype = c_int
         fn.argtypes = [c_int, c_vp, c_vp] + [c_int] * 7 + [ctypes.c_double, c_int, c_int, c_vp, c_vp]
+    lib.msda_roi_align_backward_deterministic.restype = c_int
+    lib.msda_roi_align_backward_deterministic.argtypes = lib.msda_roi_align_backward.argtypes[:-1] + [c_vp, c_i64, c_vp]
     lib.msda_layer_proj_layernorm_supported.restype = c_int
     lib.msda_layer_proj_layernorm_supported.argtypes = [c_int, c_int, c_int]
     lib.msda_layer_proj_layernorm_forward.restype = c_int
@@ -129,6 +137,15 @@ def load():
         raise MSDAError(f"libmsda_b200.so ABI {lib.msda_abi_version()} != binding ABI {ABI_VERSION}; rebuild")
     _lib = lib
     return lib
+
+
+def deterministic_scratch(device, grad_elements, grad_reference_elements=0, num_heads=0):
+    """Scratch of the *_deterministic calls, from torch's caching allocator."""
+    import torch
+    nbytes = load().msda_deterministic_scratch_bytes(int(grad_elements), int(grad_reference_elements), int(num_heads))
+    if nbytes < 0:
+        raise MSDAError(f"msda_deterministic_scratch_bytes({grad_elements}, {grad_reference_elements}) failed")
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)
 
 
 def check(code, what):

@@ -7,7 +7,7 @@ static bool bad_dims(int N, int S, int M, int D, int L, int Lq, int P)
     return N < 0 || S < 0 || M < 0 || D < 0 || L < 0 || Lq < 0 || P < 0;
 }
 
-extern "C" int msda_abi_version(void) { return 22; }
+extern "C" int msda_abi_version(void) { return 23; }
 
 extern "C" const char* msda_error_string(int code)
 {
@@ -60,6 +60,38 @@ extern "C" int msda_backward(int dtype, const void* grad_output, const void* val
     a.force_generic = (flags & MSDA_FLAG_FORCE_GENERIC) ? 1 : 0;
     a.no_tc = (flags & MSDA_FLAG_TC) ? 0 : 1;
     return (int)msda::backward(a, (cudaStream_t)stream);
+}
+
+extern "C" int64_t msda_deterministic_scratch_bytes(int64_t grad_elements, int64_t grad_reference_elements,
+                                                   int num_heads)
+{
+    if (grad_elements < 0 || grad_reference_elements < 0 || num_heads < 0) return -1;
+    return (int64_t)msda::det_scratch_bytes((long long)grad_elements, (long long)grad_reference_elements * num_heads);
+}
+
+extern "C" int msda_backward_deterministic(int dtype, const void* grad_output, const void* value,
+                                           const int64_t* spatial_shapes, const int64_t* level_start_index,
+                                           const void* sampling_loc, const void* attn_weight, int batch,
+                                           int spatial_size, int num_heads, int channels, int num_levels,
+                                           int num_query, int num_point, void* grad_value, void* grad_sampling_loc,
+                                           void* grad_attn_weight, void* grad_value_accum_f32, int flags,
+                                           void* scratch, int64_t scratch_bytes, void* stream)
+{
+    (void)grad_value_accum_f32;
+    if (dtype < 0 || dtype > 3 || bad_dims(batch, spatial_size, num_heads, channels, num_levels, num_query, num_point) ||
+        (flags & MSDA_FLAG_TC))
+        return (int)cudaErrorInvalidValue;
+    msda::BwdArgs a;
+    a.dtype = dtype;
+    a.grad_out = grad_output; a.value = value; a.shapes = spatial_shapes; a.lsi = level_start_index;
+    a.loc = sampling_loc; a.attn = attn_weight;
+    a.grad_value = grad_value; a.grad_loc = grad_sampling_loc; a.grad_attn = grad_attn_weight;
+    a.grad_value_accum = nullptr;
+    a.N = batch; a.S = spatial_size; a.M = num_heads; a.D = channels;
+    a.L = num_levels; a.Lq = num_query; a.P = num_point;
+    a.force_generic = (flags & MSDA_FLAG_FORCE_GENERIC) ? 1 : 0;
+    a.no_tc = 1;
+    return (int)msda::backward_deterministic(a, scratch, (long long)scratch_bytes, (cudaStream_t)stream);
 }
 
 static msda::FusedArgs make_fused(int dtype, int raw_dtype, const void* value, const int64_t* shapes,
@@ -138,6 +170,30 @@ extern "C" int msda_fused_backward(int dtype, int raw_dtype, const void* grad_ou
     a.grad_value = grad_value; a.grad_offsets = grad_offsets_raw; a.grad_logits = grad_logits_raw;
     a.grad_ref = grad_reference_points; a.grad_value_accum = (float*)grad_value_accum_f32;
     return (int)msda::fused_backward(a, (cudaStream_t)stream);
+}
+
+extern "C" int msda_fused_backward_deterministic(int dtype, int raw_dtype, const void* grad_output, const void* value,
+                                                 const int64_t* spatial_shapes, const int64_t* level_start_index,
+                                                 const float* reference_points, int ref_dim,
+                                                 const void* sampling_offsets_raw, int64_t offsets_query_stride,
+                                                 const void* attention_logits_raw, int64_t logits_query_stride,
+                                                 int batch, int spatial_size, int num_heads, int channels,
+                                                 int num_levels, int num_query, int num_point, void* grad_value,
+                                                 void* grad_offsets_raw, void* grad_logits_raw,
+                                                 float* grad_reference_points, void* grad_value_accum_f32,
+                                                 void* scratch, int64_t scratch_bytes, void* stream)
+{
+    (void)grad_value_accum_f32;
+    if (bad_dims(batch, spatial_size, num_heads, channels, num_levels, num_query, num_point))
+        return (int)cudaErrorInvalidValue;
+    msda::FusedArgs a = make_fused(dtype, raw_dtype, value, spatial_shapes, level_start_index, reference_points,
+                                   ref_dim, sampling_offsets_raw, offsets_query_stride, attention_logits_raw,
+                                   logits_query_stride, batch, spatial_size, num_heads, channels, num_levels,
+                                   num_query, num_point);
+    a.grad_out = grad_output;
+    a.grad_value = grad_value; a.grad_offsets = grad_offsets_raw; a.grad_logits = grad_logits_raw;
+    a.grad_ref = grad_reference_points;
+    return (int)msda::fused_backward_deterministic(a, scratch, (long long)scratch_bytes, (cudaStream_t)stream);
 }
 
 // ---- layer epilogues --------------------------------------------------------------------------
@@ -272,6 +328,21 @@ extern "C" int msda_roi_align_backward(int dtype, const void* grad_pooled, const
     a.N = batch; a.H = height; a.W = width; a.C = channels; a.K = num_rois; a.PH = pooled_height; a.PW = pooled_width;
     a.scale = spatial_scale; a.sampling_ratio = sampling_ratio; a.aligned = aligned;
     return (int)msda::roi_align_backward(a, (cudaStream_t)stream);
+}
+
+extern "C" int msda_roi_align_backward_deterministic(int dtype, const void* grad_pooled, const void* rois, int batch,
+                                                     int height, int width, int channels, int num_rois,
+                                                     int pooled_height, int pooled_width, double spatial_scale,
+                                                     int sampling_ratio, int aligned, void* grad_feature,
+                                                     void* scratch, int64_t scratch_bytes, void* stream)
+{
+    if (bad_roi_dims(batch, height, width, channels, num_rois, pooled_height, pooled_width) || sampling_ratio < 0)
+        return (int)cudaErrorInvalidValue;
+    msda::RoiAlignArgs a{};
+    a.dtype = dtype; a.grad_out = grad_pooled; a.rois = rois; a.grad_accum = grad_feature;
+    a.N = batch; a.H = height; a.W = width; a.C = channels; a.K = num_rois; a.PH = pooled_height; a.PW = pooled_width;
+    a.scale = spatial_scale; a.sampling_ratio = sampling_ratio; a.aligned = aligned;
+    return (int)msda::roi_align_backward_deterministic(a, scratch, (long long)scratch_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int msda_layer_norm_act_supported(int dtype, int channels)

@@ -125,13 +125,19 @@ __device__ __forceinline__ void reg_put(float (&a)[K], int idx, float v)
     for (int k = 0; k < K; ++k) a[k] = idx == k ? v : a[k];
 }
 
-template <typename VT, int D, bool FUSED, typename RT>
+// DET (deterministic backward, DESIGN.md section 3.15): gv_accum is the int64 accumulator of the caller's scratch and
+// every grad_value contribution is added as a fixed-point integer at the scale of det->scale_f (4 scalar 64-bit
+// reductions per lane and corner instead of one red.v4.f32); the fused op's grad_ref goes, without atomics, to
+// per-(query, level, head) partials in ref_part, which det_fold_ref sums over the heads.  DET = false compiles to the
+// kernel it was before the parameter existed (the two trailing parameters are unused).
+template <typename VT, int D, bool FUSED, typename RT, bool DET = false>
 __global__ void __launch_bounds__(BwdWarps<32 / (D / 4)>::value * 32, MSDA_BWD_MINBLOCKS)
 msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ value,
                      const int64_t* __restrict__ shapes, const int64_t* __restrict__ lsi,
                      const SampleSrc src, float* __restrict__ gv_accum, const GradDst dst,
                      int S, int M, int L, int Lq, int P, int p_magic, long long total_pairs,
-                     const unsigned char* __restrict__ red_levels)
+                     const unsigned char* __restrict__ red_levels,
+                     const DetHeader* __restrict__ det, float* __restrict__ ref_part)
 {
     // red_levels (optional): per pair, bit l set = this kernel issues the grad_value reductions of level l; clear =
     // another kernel accumulates that level (msda_tc_backward.cu).  nullptr = every level.
@@ -146,6 +152,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     constexpr int FCH = (kChunk + CH - 1) / CH;  // passes of the fused op (host guarantees L*P <= kChunk)
     static_assert(G >= 1 && G <= 32 && (G & (G - 1)) == 0, "fast backward needs 1..32 lanes per head");
     static_assert(CH % G == 0, "pass size must split evenly over the lanes");
+    static_assert(!(FUSED && DET) || CH * (MSDA_BWD_COEF_RECORDS ? 5 : 3) + 1 >= kChunk,
+                  "the deterministic grad_ref staging reuses a group's records");
 
     // per-sample records of a pass (+1 record: the groups of a warp start in distinct banks)
     __shared__ int s_meta[3 * kMaxLevelsFast];
@@ -192,8 +200,15 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     // this lane's slice of pixel 0 of its (frame, head), as opaque addresses: a corner address is then one 64-bit add
     // (two instructions) of the 32-bit BYTE offset parked in shared memory -- scaled by 4 / sizeof(VT) for grad_value
     const unsigned long long vaddr = opaque_addr(value + head_off);
-    const unsigned long long gaddr = opaque_addr(gv_accum + head_off);
-    constexpr int kGradShift = sizeof(VT) == 4 ? 0 : 1;
+    // DET: lane `sub` adds channels sub, sub + G, sub + 2G, sub + 3G of a row, so that each of the four 64-bit reductions
+    // of a group covers G consecutive int64 (64 bytes for a 32-channel head): the lane's own 4 consecutive channels
+    // would spread every instruction over the whole 256-byte row (measured 12.6 ms for the COCO fp32 backward)
+    const unsigned long long gaddr =
+        DET ? opaque_addr(reinterpret_cast<long long*>(gv_accum) + (head_off - sub * EPL + sub))
+            : opaque_addr(gv_accum + head_off);
+    constexpr int kGradShift = DET ? (sizeof(VT) == 4 ? 1 : 2) : (sizeof(VT) == 4 ? 0 : 1);
+    float det_scale = 0.f;
+    if constexpr (DET) det_scale = det->scale_f;
     const float* lp = nullptr;
     const float* ap = nullptr;
     const RT* op = nullptr;
@@ -215,6 +230,11 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     }
     F2 G01, G23;
     G01.x = g[0]; G01.y = g[1]; G23.x = g[2]; G23.y = g[3];
+    float gt[DET ? EPL : 1];                         // DET: grad_output at channels sub + k*G
+    if constexpr (DET) {
+#pragma unroll
+        for (int k = 0; k < EPL; ++k) gt[k] = active ? to_f32<VT>(grad_out[pair * D + k * G + sub]) : 0.f;
+    }
 
     // fused: softmax over the pair's L*P logits; this lane keeps the numerators of its own samples
     float prob[FCH * SPL];
@@ -422,8 +442,17 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
                 const float4 cf = reinterpret_cast<const float4*>(rec)[1];   // 0 = row outside the map / issued by another sample
                 const float ck[4] = {cf.x, cf.y, cf.z, cf.w};
 #pragma unroll
-                for (int k = 0; k < 4; ++k)
-                    red_scaled_f32x4_if(reinterpret_cast<float*>(gaddr + ((unsigned long long)ok[k] << kGradShift)), ck[k], G01, G23);
+                for (int k = 0; k < 4; ++k) {
+                    if constexpr (DET) {
+                        if (ck[k] != 0.f) {
+                            long long* gp64 = reinterpret_cast<long long*>(gaddr + ((unsigned long long)ok[k] << kGradShift));
+#pragma unroll
+                            for (int c = 0; c < EPL; ++c) red_fixed(gp64 + c * G, ck[k] * gt[c], det_scale);
+                        }
+                    } else {
+                        red_scaled_f32x4_if(reinterpret_cast<float*>(gaddr + ((unsigned long long)ok[k] << kGradShift)), ck[k], G01, G23);
+                    }
+                }
             }
             if constexpr (BATCHED) {
                 if ((j0 & 3) == 3 && j0 - 3 < cnt) {
@@ -519,7 +548,7 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
             int run_l = -1;                       // lane-local run of samples on one level -> one grad_ref update
             float rx = 0.f, ry = 0.f, rw = 0.f, rh = 0.f;
             auto flush_ref = [&]() {
-                if (dst.ref != nullptr && run_l >= 0) {
+                if (!DET && dst.ref != nullptr && run_l >= 0) {
                     float* gr = dst.ref + (nq * L + run_l) * src.ref_dim;
                     atomicAdd(gr, rx);
                     atomicAdd(gr + 1, ry);
@@ -552,12 +581,36 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
                     store_raw2<RT>(gop + 2 * s, gox, goy);
                     ggp[s] = from_f32<RT>(glogit);
                     if (dst.ref != nullptr) {
-                        if (l != run_l) { flush_ref(); run_l = l; rx = ry = rw = rh = 0.f; }
-                        rx += glx; ry += gly; rw += gwx; rh += gwy;
+                        if constexpr (DET) {
+                            reinterpret_cast<float4*>(&s_rec[warp][grp][0])[s] = make_float4(glx, gly, gwx, gwy);
+                        } else {
+                            if (l != run_l) { flush_ref(); run_l = l; rx = ry = rw = rh = 0.f; }
+                            rx += glx; ry += gly; rw += gwx; rh += gwy;
+                        }
                     }
                 }
             }
             flush_ref();
+        }
+        if constexpr (DET) {
+            // the group's per-sample reference-point gradients are staged in its records (free after the last pass):
+            // one lane per level sums the level's points in order into the (query, level, head) partial
+            if (dst.ref != nullptr) {
+                __syncwarp();
+                if (active) {
+                    const float4* staged = reinterpret_cast<const float4*>(&s_rec[warp][grp][0]);
+                    for (int l = sub; l < L; l += G) {
+                        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+                        for (int p = 0; p < P; ++p) {
+                            const float4 v = staged[l * P + p];
+                            acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+                        }
+                        float* out = ref_part + ((nq * L + l) * M + m) * src.ref_dim;
+                        out[0] = acc.x; out[1] = acc.y;
+                        if (src.ref_dim == 4) { out[2] = acc.z; out[3] = acc.w; }
+                    }
+                }
+            }
         }
     }
 }
@@ -574,7 +627,8 @@ template <> struct ScalarLoad<double> {
     static __device__ __forceinline__ double load(const double* p) { return *p; }
 };
 
-template <typename VT>
+// DET: gv_accum is the int64 accumulator of the deterministic backward (see msda_bwd_fast_kernel)
+template <typename VT, bool DET = false>
 __global__ void __launch_bounds__(256)
 msda_bwd_generic_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ value,
                         const int64_t* __restrict__ shapes, const int64_t* __restrict__ lsi,
@@ -583,10 +637,18 @@ msda_bwd_generic_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ 
                         typename Traits<VT>::acc_t* __restrict__ gv_accum,
                         typename Traits<VT>::loc_t* __restrict__ grad_loc,
                         typename Traits<VT>::loc_t* __restrict__ grad_attn,
-                        int S, int M, int D, int L, int Lq, int P, long long total_pairs)
+                        int S, int M, int D, int L, int Lq, int P, long long total_pairs,
+                        const DetHeader* __restrict__ det)
 {
     using acc_t = typename Traits<VT>::acc_t;
     using loc_t = typename Traits<VT>::loc_t;
+    acc_t det_scale = 0;
+    if constexpr (DET) det_scale = std::is_same<acc_t, double>::value ? (acc_t)det->scale : (acc_t)det->scale_f;
+    long long* const gv64 = reinterpret_cast<long long*>(gv_accum);
+    auto add = [&](long long i, acc_t v) {
+        if constexpr (DET) red_fixed(gv64 + i, v, det_scale);
+        else atomicAdd(gv_accum + i, v);
+    };
     const int lane = threadIdx.x & 31;
     const long long warps_total = ((long long)gridDim.x * blockDim.x) >> 5;
     const long long MD = (long long)M * D;
@@ -617,10 +679,10 @@ msda_bwd_generic_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ 
                         const acc_t gc = ScalarLoad<VT>::load(go + c);
                         const acc_t tg = a * gc;
                         acc_t v1 = 0, v2 = 0, v3 = 0, v4 = 0;
-                        if (f.ok & 1u) { v1 = ScalarLoad<VT>::load(value + o00 + c);            atomicAdd(gv_accum + o00 + c, w1 * tg); }
-                        if (f.ok & 2u) { v2 = ScalarLoad<VT>::load(value + o00 + MD + c);       atomicAdd(gv_accum + o00 + MD + c, w2 * tg); }
-                        if (f.ok & 4u) { v3 = ScalarLoad<VT>::load(value + o00 + row + c);      atomicAdd(gv_accum + o00 + row + c, w3 * tg); }
-                        if (f.ok & 8u) { v4 = ScalarLoad<VT>::load(value + o00 + row + MD + c); atomicAdd(gv_accum + o00 + row + MD + c, w4 * tg); }
+                        if (f.ok & 1u) { v1 = ScalarLoad<VT>::load(value + o00 + c);            add(o00 + c, w1 * tg); }
+                        if (f.ok & 2u) { v2 = ScalarLoad<VT>::load(value + o00 + MD + c);       add(o00 + MD + c, w2 * tg); }
+                        if (f.ok & 4u) { v3 = ScalarLoad<VT>::load(value + o00 + row + c);      add(o00 + row + c, w3 * tg); }
+                        if (f.ok & 8u) { v4 = ScalarLoad<VT>::load(value + o00 + row + MD + c); add(o00 + row + MD + c, w4 * tg); }
                         pa += gc * (w1 * v1 + w2 * v2 + w3 * v3 + w4 * v4);
                         px += tg * (hh * (v2 - v1) + lh * (v4 - v3));
                         py += tg * (hw * (v3 - v1) + lw * (v4 - v2));
@@ -663,9 +725,9 @@ msda_cast_accum_kernel(const float* __restrict__ src, VT* __restrict__ dst, long
 // ------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------
-template <typename VT, int D>
+template <typename VT, int D, bool DET = false>
 static cudaError_t launch_bwd_fast(const BwdArgs& a, float* accum, cudaStream_t stream,
-                                   const unsigned char* red_levels = nullptr)
+                                   const unsigned char* red_levels = nullptr, const DetHeader* det = nullptr)
 {
     constexpr int G = D / 4;
     constexpr int PAIRS = 32 / G;
@@ -683,14 +745,15 @@ static cudaError_t launch_bwd_fast(const BwdArgs& a, float* accum, cudaStream_t 
     src.loc = a.loc; src.attn = a.attn; src.ref = nullptr; src.loc_stride = 0; src.attn_stride = 0; src.ref_dim = 0;
     GradDst dst;
     dst.loc = a.grad_loc; dst.attn = a.grad_attn; dst.ref = nullptr;
-    msda_bwd_fast_kernel<VT, D, false, float><<<(unsigned)blocks, WARPS * 32, 0, stream>>>(
+    msda_bwd_fast_kernel<VT, D, false, float, DET><<<(unsigned)blocks, WARPS * 32, 0, stream>>>(
         (const VT*)a.grad_out, (const VT*)a.value, a.shapes, a.lsi, src, accum, dst,
-        a.S, a.M, a.L, a.Lq, a.P, p_magic, total_pairs, red_levels);
+        a.S, a.M, a.L, a.Lq, a.P, p_magic, total_pairs, red_levels, det, nullptr);
     return cudaGetLastError();
 }
 
-template <typename VT, int D, typename RT>
-static cudaError_t launch_bwd_fused(const FusedArgs& a, float* accum, cudaStream_t stream)
+template <typename VT, int D, typename RT, bool DET = false>
+static cudaError_t launch_bwd_fused(const FusedArgs& a, float* accum, cudaStream_t stream,
+                                    const DetHeader* det = nullptr, float* ref_part = nullptr)
 {
     constexpr int G = D / 4;
     constexpr int PAIRS = 32 / G;
@@ -709,22 +772,23 @@ static cudaError_t launch_bwd_fused(const FusedArgs& a, float* accum, cudaStream
     src.loc_stride = a.off_stride; src.attn_stride = a.logit_stride; src.ref_dim = a.ref_dim;
     GradDst dst;
     dst.loc = a.grad_offsets; dst.attn = a.grad_logits; dst.ref = a.grad_ref;
-    msda_bwd_fast_kernel<VT, D, true, RT><<<(unsigned)blocks, WARPS * 32, 0, stream>>>(
+    msda_bwd_fast_kernel<VT, D, true, RT, DET><<<(unsigned)blocks, WARPS * 32, 0, stream>>>(
         (const VT*)a.grad_out, (const VT*)a.value, a.shapes, a.lsi, src, accum, dst,
-        a.S, a.M, a.L, a.Lq, a.P, p_magic, total_pairs, nullptr);
+        a.S, a.M, a.L, a.Lq, a.P, p_magic, total_pairs, nullptr, det, ref_part);
     return cudaGetLastError();
 }
 
-template <typename VT>
-static cudaError_t launch_bwd_generic(const BwdArgs& a, typename Traits<VT>::acc_t* accum, cudaStream_t stream)
+template <typename VT, bool DET = false>
+static cudaError_t launch_bwd_generic(const BwdArgs& a, typename Traits<VT>::acc_t* accum, cudaStream_t stream,
+                                      const DetHeader* det = nullptr)
 {
     using loc_t = typename Traits<VT>::loc_t;
     const long long total_pairs = (long long)a.N * a.Lq * a.M;
     long long blocks = (total_pairs + 7) / 8;
     if (blocks > (1ll << 30)) blocks = 1ll << 30;
-    msda_bwd_generic_kernel<VT><<<(unsigned)blocks, 256, 0, stream>>>(
+    msda_bwd_generic_kernel<VT, DET><<<(unsigned)blocks, 256, 0, stream>>>(
         (const VT*)a.grad_out, (const VT*)a.value, a.shapes, a.lsi, (const loc_t*)a.loc, (const loc_t*)a.attn,
-        accum, (loc_t*)a.grad_loc, (loc_t*)a.grad_attn, a.S, a.M, a.D, a.L, a.Lq, a.P, total_pairs);
+        accum, (loc_t*)a.grad_loc, (loc_t*)a.grad_attn, a.S, a.M, a.D, a.L, a.Lq, a.P, total_pairs, det);
     return cudaGetLastError();
 }
 
@@ -848,6 +912,97 @@ cudaError_t backward(const BwdArgs& a, cudaStream_t stream)
         }
     }
     return cudaErrorInvalidValue;
+}
+
+// ------------------------------------------------------------------------------------------
+// deterministic backward (DESIGN.md section 3.15): zero the accumulators, bound the gradient, accumulate in fixed
+// point, convert.  Same kernels as above with DET = true; stream-ordered, no allocation, no host read-back.
+// ------------------------------------------------------------------------------------------
+template <typename VT>
+static cudaError_t run_bwd_det(const BwdArgs& a, long long* acc, const DetHeader* det, cudaStream_t stream)
+{
+    float* acc_f = reinterpret_cast<float*>(acc);
+    if (fast_shape_ok(a)) {
+        switch (a.D) {
+            case 4:   return launch_bwd_fast<VT, 4, true>(a, acc_f, stream, nullptr, det);
+            case 8:   return launch_bwd_fast<VT, 8, true>(a, acc_f, stream, nullptr, det);
+            case 16:  return launch_bwd_fast<VT, 16, true>(a, acc_f, stream, nullptr, det);
+            case 32:  return launch_bwd_fast<VT, 32, true>(a, acc_f, stream, nullptr, det);
+            case 64:  return launch_bwd_fast<VT, 64, true>(a, acc_f, stream, nullptr, det);
+            case 128: return launch_bwd_fast<VT, 128, true>(a, acc_f, stream, nullptr, det);
+            default: break;
+        }
+    }
+    return launch_bwd_generic<VT, true>(a, reinterpret_cast<typename Traits<VT>::acc_t*>(acc), stream, det);
+}
+
+cudaError_t backward_deterministic(const BwdArgs& a, void* scratch, long long scratch_bytes, cudaStream_t stream)
+{
+    if (a.dtype < kF32 || a.dtype > kF16 || !a.no_tc) return cudaErrorInvalidValue;   // no tensor-core variant
+    const long long count = (long long)a.N * a.S * a.M * a.D;
+    if (scratch == nullptr || scratch_bytes < det_scratch_bytes(count, 0)) return cudaErrorInvalidValue;
+    if (a.L == 0 || a.P == 0) return backward(a, stream);         // grad_value = 0, nothing is accumulated
+    DetHeader* h = static_cast<DetHeader*>(scratch);
+    long long* acc = reinterpret_cast<long long*>(static_cast<char*>(scratch) + kDetHeaderBytes);
+    cudaError_t err = det_begin(scratch, count, stream);
+    const long long pairs = (long long)a.N * a.Lq * a.M;
+    if (err == cudaSuccess) err = det_absmax(a.dtype, a.grad_out, pairs, a.D, a.D, &h->gmax, stream);
+    if (err == cudaSuccess) err = det_attn_sum_max(a.dtype == kF64, a.attn, pairs, a.L * a.P, &h->amax, stream);
+    // a pixel of one (frame, head) receives, per query, at most |a| |g| from each sample (the bilinear weights of a
+    // sample are at most 1 at any one pixel):  |grad_value| <= Lq * max|g| * max_pair sum |a|
+    if (err == cudaSuccess) err = det_finalize(h, (double)a.Lq, 0, a.dtype == kF64, stream);
+    if (err == cudaSuccess && pairs > 0 && a.D > 0) {
+        switch (a.dtype) {
+            case kF32:  err = run_bwd_det<float>(a, acc, h, stream); break;
+            case kBF16: err = run_bwd_det<__nv_bfloat16>(a, acc, h, stream); break;
+            case kF16:  err = run_bwd_det<__half>(a, acc, h, stream); break;
+            case kF64:  err = launch_bwd_generic<double, true>(a, reinterpret_cast<double*>(acc), stream, h); break;
+        }
+    }
+    if (err == cudaSuccess) err = det_finish(a.dtype, acc, a.grad_value, count, h, stream);
+    return err;
+}
+
+template <typename VT, typename RT>
+static cudaError_t run_bwd_fused_det(const FusedArgs& a, long long* acc, const DetHeader* det, float* ref_part,
+                                     cudaStream_t stream)
+{
+    float* acc_f = reinterpret_cast<float*>(acc);
+    switch (a.D) {
+        case 16: return launch_bwd_fused<VT, 16, RT, true>(a, acc_f, stream, det, ref_part);
+        case 32: return launch_bwd_fused<VT, 32, RT, true>(a, acc_f, stream, det, ref_part);
+        case 64: return launch_bwd_fused<VT, 64, RT, true>(a, acc_f, stream, det, ref_part);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+cudaError_t fused_backward_deterministic(const FusedArgs& a, void* scratch, long long scratch_bytes,
+                                         cudaStream_t stream)
+{
+    if (!fused_supported(a) || !fused_raw_layout_ok(a)) return cudaErrorInvalidValue;
+    const long long count = (long long)a.N * a.S * a.M * a.D;
+    const long long rows = (long long)a.N * a.Lq * a.L;     // grad_ref rows (query, level)
+    const long long part = a.grad_ref != nullptr ? rows * a.M * a.ref_dim : 0;
+    if (scratch == nullptr || scratch_bytes < det_scratch_bytes(count, part)) return cudaErrorInvalidValue;
+    DetHeader* h = static_cast<DetHeader*>(scratch);
+    long long* acc = reinterpret_cast<long long*>(static_cast<char*>(scratch) + kDetHeaderBytes);
+    float* ref_part = det_ref_partials(scratch, count);
+    const long long pairs = (long long)a.N * a.Lq * a.M;
+    const long long nq = (long long)a.N * a.Lq;
+    const int mlp = a.M * a.L * a.P;
+    cudaError_t err = det_begin(scratch, count, stream);
+    if (err == cudaSuccess) err = det_absmax(a.dtype, a.grad_out, pairs, a.D, a.D, &h->gmax, stream);
+    // the attention weights are a softmax (sum |a| = 1 per pair): the logits are scanned only for Inf / NaN
+    if (err == cudaSuccess) err = det_absmax(a.raw_dtype, a.logits, nq, mlp, a.logit_stride, &h->amax, stream);
+    if (err == cudaSuccess) err = det_finalize(h, (double)a.Lq, 1, false, stream);
+    if (err == cudaSuccess && pairs > 0) {
+        if (a.dtype == kF32) err = run_bwd_fused_det<float, float>(a, acc, h, ref_part, stream);
+        else if (a.raw_dtype == kF32) err = run_bwd_fused_det<__nv_bfloat16, float>(a, acc, h, ref_part, stream);
+        else err = run_bwd_fused_det<__nv_bfloat16, __nv_bfloat16>(a, acc, h, ref_part, stream);
+    }
+    if (err == cudaSuccess) err = det_finish(a.dtype, acc, a.grad_value, count, h, stream);
+    if (err == cudaSuccess && a.grad_ref != nullptr) err = det_fold_ref(ref_part, a.grad_ref, rows, a.M, a.ref_dim, stream);
+    return err;
 }
 
 }  // namespace msda

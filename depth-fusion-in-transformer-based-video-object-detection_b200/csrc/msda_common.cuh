@@ -326,4 +326,30 @@ __device__ __forceinline__ void red_scaled_f32x4_if(float* p, float coef, F2 g01
                  :: "l"(p), "f"(coef), "l"(f2_bits(g01)), "l"(f2_bits(g23)) : "memory");
 }
 
+// ----------------------------------------------------------------------------------------
+// Deterministic backward (C ABI *_deterministic, csrc/deterministic.cu, DESIGN.md section 3.15): every contribution
+// to a gradient element is rounded to an integer multiple of 2^-shift and the integers are summed with 64-bit
+// reductions.  Integer addition is associative, so the sum does not depend on the order the hardware runs them in.
+// The pre-pass writes this header at the start of the caller's scratch; the accumulation kernels read the scale there.
+// ----------------------------------------------------------------------------------------
+struct DetHeader {
+    unsigned long long gmax;   // max |grad_output| as the bits of a double (NaN above +Inf: see det_abs_bits)
+    unsigned long long amax;   // max over pairs of sum |attention|, same encoding
+    double scale, inv_scale;   // 2^shift, 2^-shift
+    float scale_f;             // 2^shift for fp32 contributions
+    int shift;
+    int poison;                // non-finite bound: the finishing kernel writes NaN everywhere
+};
+constexpr long long kDetHeaderBytes = 256;   // the int64 accumulators start here
+
+__device__ __forceinline__ void red_fixed(long long* p, float v, float scale)
+{
+    // v * scale is exact (a power of two); |v * scale| < 2^62 by the choice of shift, so the conversion cannot saturate
+    atomicAdd(reinterpret_cast<unsigned long long*>(p), (unsigned long long)__float2ll_rn(v * scale));
+}
+__device__ __forceinline__ void red_fixed(long long* p, double v, double scale)
+{
+    atomicAdd(reinterpret_cast<unsigned long long*>(p), (unsigned long long)__double2ll_rn(v * scale));
+}
+
 }  // namespace msda

@@ -92,6 +92,26 @@ cudaError_t tc_backward_dv(const BwdArgs& a, unsigned char* red_levels, cudaStre
 
 cudaError_t backward(const BwdArgs& a, cudaStream_t stream);
 
+// Deterministic backward (deterministic.cu, DESIGN.md section 3.15).  scratch: [256-byte DetHeader | int64
+// accumulators, one per gradient element, padded to 256 bytes | fp32 partials of grad_reference_points (fused op)].
+struct DetHeader;
+long long det_scratch_bytes(long long grad_elements, long long ref_partial_floats);   // -1 = negative sizes
+float* det_ref_partials(void* scratch, long long grad_elements);
+cudaError_t det_begin(void* scratch, long long grad_elements, cudaStream_t stream);   // zero header + accumulators
+cudaError_t det_absmax(int dtype, const void* x, long long rows, int cols, long long ld, unsigned long long* slot,
+                       cudaStream_t stream);
+cudaError_t det_attn_sum_max(bool f64, const void* attn, long long pairs, int LP, unsigned long long* slot,
+                             cudaStream_t stream);
+// bound B = count * max|g| * (amax_mode 0: max pair sum |a|; 1: 1, or non-finite when the scanned logits are)
+cudaError_t det_finalize(DetHeader* h, double count, int amax_mode, bool f64, cudaStream_t stream);
+cudaError_t det_finish(int dtype, const long long* acc, void* out, long long count, const DetHeader* h,
+                       cudaStream_t stream);
+cudaError_t det_fold_ref(const float* part, float* grad_ref, long long rows, int M, int R, cudaStream_t stream);
+// scratch of at least det_scratch_bytes(N*S*M*D, 0) (plain) / (N*S*M*D, grad_ref ? N*Lq*L*M*ref_dim : 0) (fused)
+cudaError_t backward_deterministic(const BwdArgs& a, void* scratch, long long scratch_bytes, cudaStream_t stream);
+cudaError_t fused_backward_deterministic(const FusedArgs& a, void* scratch, long long scratch_bytes,
+                                         cudaStream_t stream);
+
 // Layer epilogues (layer_epilogue.cu):  y = LayerNorm(residual + act(branch)) * gamma + beta,
 // optional y_pos = y + pos; backward of the same.
 struct AddLayerNormArgs {
@@ -211,6 +231,9 @@ struct RoiAlignArgs {
 };
 cudaError_t roi_align_forward(const RoiAlignArgs& a, cudaStream_t stream);
 cudaError_t roi_align_backward(const RoiAlignArgs& a, cudaStream_t stream);
+// grad_accum is then the dtype gradient, fully written; scratch >= det_scratch_bytes(N*H*W*C, 0)
+cudaError_t roi_align_backward_deterministic(const RoiAlignArgs& a, void* scratch, long long scratch_bytes,
+                                             cudaStream_t stream);
 
 int colsum_blocks(int dtype, long long rows, int C);   // 0 = unsupported shape
 cudaError_t colsum(int dtype, const void* x, long long rows, int C, void* out, float* partial, int blocks,

@@ -179,11 +179,13 @@ __device__ __forceinline__ void atomic_add_ct(float* p, float v) { atomicAdd(p, 
 __device__ __forceinline__ void atomic_add_ct(double* p, double v) { atomicAdd(p, v); }
 
 // backward: every corner of every sample receives weight * grad / count (mmcv roi_align_backward_cuda_kernel);
-// accumulation in CT (fp32 for the 16-bit dtypes, the caller casts once).
-template <typename T, typename CT>
+// accumulation in CT (fp32 for the 16-bit dtypes, the caller casts once).  DET: grad_feat is the int64 accumulator of
+// the deterministic backward and every contribution is added in fixed point at det's scale (DESIGN.md section 3.15).
+template <typename T, typename CT, bool DET = false>
 __global__ void __launch_bounds__(256)
 roi_align_bwd_kernel(const T* __restrict__ grad_out, const CT* __restrict__ rois, CT* __restrict__ grad_feat, int N,
-                     int H, int W, int C, long long bins, int PH, int PW, CT scale, int sampling_ratio, int aligned)
+                     int H, int W, int C, long long bins, int PH, int PW, CT scale, int sampling_ratio, int aligned,
+                     const DetHeader* __restrict__ det)
 {
     const long long bin = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
@@ -193,7 +195,10 @@ roi_align_bwd_kernel(const T* __restrict__ grad_out, const CT* __restrict__ rois
     const RoiGeom<CT> g = roi_geom<CT>(rois + 5 * k, scale, sampling_ratio, aligned, PH, PW);
     if (g.batch < 0 || g.batch >= N) return;
     CT* map = grad_feat + (long long)g.batch * H * W * C;
-    const bool vec = (C % 4 == 0) && sizeof(CT) == 4;
+    long long* map64 = reinterpret_cast<long long*>(grad_feat) + (long long)g.batch * H * W * C;
+    CT det_scale = (CT)0;
+    if constexpr (DET) det_scale = sizeof(CT) == 8 ? (CT)det->scale : (CT)det->scale_f;
+    const bool vec = !DET && (C % 4 == 0) && sizeof(CT) == 4;
     for (int iy = 0; iy < g.grid_h; ++iy) {
         const CT y = g.y0 + (CT)ph * g.bin_h + ((CT)iy + (CT)0.5) * g.bin_h / (CT)g.grid_h;
         for (int ix = 0; ix < g.grid_w; ++ix) {
@@ -217,7 +222,10 @@ roi_align_bwd_kernel(const T* __restrict__ grad_out, const CT* __restrict__ rois
                 for (int c = lane; c < C; c += 32) {
                     const CT gv = load_as<T, CT>(grad_out + bin * C + c);
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) atomic_add_ct(map + (long long)pk[q] * C + c, wk[q] * gv);
+                    for (int q = 0; q < 4; ++q) {
+                        if constexpr (DET) red_fixed(map64 + (long long)pk[q] * C + c, wk[q] * gv, det_scale);
+                        else atomic_add_ct(map + (long long)pk[q] * C + c, wk[q] * gv);
+                    }
                 }
             }
         }
@@ -263,7 +271,7 @@ cudaError_t roi_align_backward(const RoiAlignArgs& a, cudaStream_t st)
 #define ROI_BWD(T, CT)                                                                                             \
     roi_align_bwd_kernel<T, CT><<<blocks, 256, 0, st>>>((const T*)a.grad_out, (const CT*)a.rois, (CT*)a.grad_accum, \
                                                         a.N, a.H, a.W, a.C, bins, a.PH, a.PW, (CT)a.scale,          \
-                                                        a.sampling_ratio, a.aligned)
+                                                        a.sampling_ratio, a.aligned, nullptr)
     switch (a.dtype) {
         case kF32:  ROI_BWD(float, float); break;
         case kBF16: ROI_BWD(__nv_bfloat16, float); break;
@@ -273,6 +281,39 @@ cudaError_t roi_align_backward(const RoiAlignArgs& a, cudaStream_t st)
     }
 #undef ROI_BWD
     return cudaGetLastError();
+}
+
+cudaError_t roi_align_backward_deterministic(const RoiAlignArgs& a, void* scratch, long long scratch_bytes,
+                                             cudaStream_t st)
+{
+    if (a.dtype < kF32 || a.dtype > kF16) return cudaErrorInvalidValue;
+    const long long count = (long long)a.N * a.H * a.W * a.C;
+    if (scratch == nullptr || scratch_bytes < det_scratch_bytes(count, 0)) return cudaErrorInvalidValue;
+    DetHeader* h = static_cast<DetHeader*>(scratch);
+    long long* acc = reinterpret_cast<long long*>(static_cast<char*>(scratch) + kDetHeaderBytes);
+    const long long bins = (long long)a.K * a.PH * a.PW;
+    cudaError_t err = det_begin(scratch, count, st);
+    if (err == cudaSuccess && bins > 0) err = det_absmax(a.dtype, a.grad_out, bins, a.C, a.C, &h->gmax, st);
+    // a sample adds weight * g / count to each corner and its four weights sum to 1 (clamped corners coincide, their
+    // weights add), and a bin has `count` samples: a bin adds at most |g| to any pixel, |grad| <= K*PH*PW * max|g|
+    if (err == cudaSuccess) err = det_finalize(h, (double)bins, 1, a.dtype == kF64, st);
+    if (err == cudaSuccess && bins > 0 && a.C > 0) {
+        const unsigned blocks = (unsigned)((bins + 7) / 8);
+#define ROI_BWD_DET(T, CT)                                                                                         \
+    roi_align_bwd_kernel<T, CT, true><<<blocks, 256, 0, st>>>((const T*)a.grad_out, (const CT*)a.rois, (CT*)acc,     \
+                                                              a.N, a.H, a.W, a.C, bins, a.PH, a.PW, (CT)a.scale,    \
+                                                              a.sampling_ratio, a.aligned, h)
+        switch (a.dtype) {
+            case kF32:  ROI_BWD_DET(float, float); break;
+            case kBF16: ROI_BWD_DET(__nv_bfloat16, float); break;
+            case kF16:  ROI_BWD_DET(__half, float); break;
+            case kF64:  ROI_BWD_DET(double, double); break;
+        }
+#undef ROI_BWD_DET
+        err = cudaGetLastError();
+    }
+    if (err == cudaSuccess) err = det_finish(a.dtype, acc, a.grad_accum, count, h, st);
+    return err;
 }
 
 }  // namespace msda

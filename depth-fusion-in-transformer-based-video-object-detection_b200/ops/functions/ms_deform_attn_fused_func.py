@@ -7,6 +7,8 @@ One kernel per direction replaces, inside ``MSDeformAttn.forward``, the referenc
 so the sampling locations [N,Lq,M,L,P,2] and attention weights [N,Lq,M,L,P] (and their
 gradients) are never written to HBM.  ``raw`` is the output of ONE projection GEMM whose rows are
 ``[ sampling offsets (M*L*P*2) | attention logits (M*L*P) ]``.
+Under ``torch.use_deterministic_algorithms(True)`` the backward runs ``msda_fused_backward_deterministic``
+(bitwise reproducible gradients; DESIGN.md section 3.15).
 """
 import torch
 from torch.autograd import Function
@@ -109,22 +111,30 @@ class MSDeformAttnFusedFunction(Function):
         if grad_output.dtype != value.dtype:
             grad_output = grad_output.to(value.dtype)
         lib = _lib.load()
+        deterministic = torch.are_deterministic_algorithms_enabled()
         with torch.cuda.device(value.device):
             grad_value = torch.empty_like(value)
             grad_raw = torch.empty_like(raw)
-            grad_ref = torch.zeros_like(ref) if ctx.ref_needs_grad else None
-            accum = torch.empty(value.shape, dtype=torch.float32, device=value.device) \
-                if value.dtype != torch.float32 else None
+            grad_ref = None
+            if ctx.ref_needs_grad:
+                grad_ref = torch.empty_like(ref) if deterministic else torch.zeros_like(ref)
             esz = raw.element_size()
-            code = lib.msda_fused_backward(
-                _DTYPES[value.dtype], _DTYPES[raw.dtype], grad_output.data_ptr(), value.data_ptr(),
-                spatial_shapes.data_ptr(), level_start_index.data_ptr(), ref.data_ptr(), ref.size(-1),
-                raw.data_ptr(), 3 * mlp, raw.data_ptr() + 2 * mlp * esz, 3 * mlp,
-                n, s, m, d, nl, lq, p, grad_value.data_ptr(), grad_raw.data_ptr(),
-                grad_raw.data_ptr() + 2 * mlp * esz,
-                grad_ref.data_ptr() if grad_ref is not None else None,
-                accum.data_ptr() if accum is not None else None, torch.cuda.current_stream().cuda_stream)
-        _lib.check(code, "msda_fused_backward")
+            args = (_DTYPES[value.dtype], _DTYPES[raw.dtype], grad_output.data_ptr(), value.data_ptr(),
+                    spatial_shapes.data_ptr(), level_start_index.data_ptr(), ref.data_ptr(), ref.size(-1),
+                    raw.data_ptr(), 3 * mlp, raw.data_ptr() + 2 * mlp * esz, 3 * mlp,
+                    n, s, m, d, nl, lq, p, grad_value.data_ptr(), grad_raw.data_ptr(),
+                    grad_raw.data_ptr() + 2 * mlp * esz,
+                    grad_ref.data_ptr() if grad_ref is not None else None)
+            stream = torch.cuda.current_stream().cuda_stream
+            if deterministic:
+                scratch = _lib.deterministic_scratch(value.device, value.numel(),
+                                                     grad_ref.numel() if grad_ref is not None else 0, m)
+                code = lib.msda_fused_backward_deterministic(*args, None, scratch.data_ptr(), scratch.numel(), stream)
+            else:
+                accum = torch.empty(value.shape, dtype=torch.float32, device=value.device) \
+                    if value.dtype != torch.float32 else None
+                code = lib.msda_fused_backward(*args, accum.data_ptr() if accum is not None else None, stream)
+        _lib.check(code, "msda_fused_backward_deterministic" if deterministic else "msda_fused_backward")
         if grad_ref is not None and grad_ref.dtype != ctx.ref_dtype:
             grad_ref = grad_ref.to(ctx.ref_dtype)
         return grad_value, None, None, grad_ref, grad_raw, None

@@ -95,12 +95,21 @@ class _RoIAlignTokens(torch.autograd.Function):
         (rois,) = ctx.saved_tensors
         n, height, width, c, ph, pw, scale, sampling_ratio, aligned, dtype = ctx.geom
         grad_out = grad_out.contiguous()
-        acc_dtype = torch.float64 if dtype == torch.float64 else torch.float32
-        accum = torch.zeros((n, height * width, c), dtype=acc_dtype, device=grad_out.device)
+        args = (_DTYPES[dtype], grad_out.data_ptr(), rois.data_ptr(), n, height, width, c, rois.size(0), ph, pw,
+                scale, sampling_ratio, aligned)
         with torch.cuda.device(grad_out.device):
-            code = _lib.load().msda_roi_align_backward(
-                _DTYPES[dtype], grad_out.data_ptr(), rois.data_ptr(), n, height, width, c, rois.size(0), ph, pw,
-                scale, sampling_ratio, aligned, accum.data_ptr(), torch.cuda.current_stream().cuda_stream)
+            stream = torch.cuda.current_stream().cuda_stream
+            if torch.are_deterministic_algorithms_enabled():
+                # fixed-point accumulation, bitwise reproducible (DESIGN.md section 3.15), written in the dtype
+                grad = torch.empty((n, height * width, c), dtype=dtype, device=grad_out.device)
+                scratch = _lib.deterministic_scratch(grad_out.device, grad.numel())
+                code = _lib.load().msda_roi_align_backward_deterministic(*args, grad.data_ptr(), scratch.data_ptr(),
+                                                                         scratch.numel(), stream)
+                _lib.check(code, "msda_roi_align_backward_deterministic")
+                return grad, None, None, None, None, None, None, None
+            acc_dtype = torch.float64 if dtype == torch.float64 else torch.float32
+            accum = torch.zeros((n, height * width, c), dtype=acc_dtype, device=grad_out.device)
+            code = _lib.load().msda_roi_align_backward(*args, accum.data_ptr(), stream)
         _lib.check(code, "msda_roi_align_backward")
         return accum.to(dtype), None, None, None, None, None, None, None
 

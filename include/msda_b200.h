@@ -90,6 +90,37 @@ int msda_backward(int dtype,
                   void* grad_value_accum_f32, int flags, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Deterministic backward: the same gradients as msda_backward / msda_fused_backward / msda_roi_align_backward, but
+ * two calls on the same inputs give the same bits in any launch order (what a framework's deterministic mode asks
+ * of an op).  Every contribution to a grad_value / grad_feature element is rounded to a multiple of 2^-shift and the
+ * integers are summed with 64-bit integer reductions, which are associative.  A pre-pass on the device computes a
+ * bound B >= |every element| from the inputs and picks shift = 61 - ceil(log2 B), so no partial sum can overflow; the
+ * quantum is about B * 2^-61 (finer than fp32 atomics for fp32 and 16-bit gradients, coarser than fp64 atomics for
+ * fp64 ones).  B == 0 gives zeros.  When B is not finite (Inf or NaN in grad_output, in the attention weights or in
+ * the attention logits) EVERY element of grad_value / grad_feature is NaN, where the non-deterministic calls only
+ * poison the elements the bad values reach.  The fused op's grad_reference_points is summed over the heads in a
+ * fixed order from per-(query, level, head) partials instead of atomics.
+ *   scratch: device memory of at least msda_deterministic_scratch_bytes(grad_elements, grad_reference_elements,
+ *            num_heads) bytes, 16-byte aligned, contents ignored and overwritten.  grad_elements = elements of
+ *            grad_value (batch*spatial_size*num_heads*channels) or of grad_feature (batch*height*width*channels);
+ *            grad_reference_elements = elements of grad_reference_points (batch*num_query*num_levels*ref_dim) when
+ *            the fused call is given one, else 0.  Returns -1 for negative arguments.
+ * Each call fully writes every gradient it is given (nothing needs zeroing), allocates nothing, never reads back to
+ * the host and is stream-ordered on `stream` without synchronising, so it can be captured in a CUDA graph.
+ * cudaErrorInvalidValue for a too small or NULL scratch, and from msda_backward_deterministic for MSDA_FLAG_TC (the
+ * tensor-core formulation has no deterministic variant).  grad_value_accum_f32 is ignored (may be NULL). */
+int64_t msda_deterministic_scratch_bytes(int64_t grad_elements, int64_t grad_reference_elements, int num_heads);
+int msda_backward_deterministic(int dtype,
+                                const void* grad_output,
+                                const void* value, const int64_t* spatial_shapes, const int64_t* level_start_index,
+                                const void* sampling_loc, const void* attn_weight,
+                                int batch, int spatial_size, int num_heads, int channels,
+                                int num_levels, int num_query, int num_point,
+                                void* grad_value, void* grad_sampling_loc, void* grad_attn_weight,
+                                void* grad_value_accum_f32, int flags, void* scratch, int64_t scratch_bytes,
+                                void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Fused layer op (no counterpart symbol in the reference: it replaces the chain
  * softmax -> offset/normaliser arithmetic -> MSDeformAttnFunction of MSDeformAttn.forward,
  * /root/reference/models/ops/modules/ms_deform_attn.py:98-115, with ONE kernel per direction;
@@ -161,6 +192,19 @@ int msda_fused_backward(int dtype, int raw_dtype,
                         int num_levels, int num_query, int num_point,
                         void* grad_value, void* grad_offsets_raw, void* grad_logits_raw,
                         float* grad_reference_points, void* grad_value_accum_f32, void* stream);
+/* msda_fused_backward with the guarantee of msda_backward_deterministic (see there); grad_reference_points (may be
+ * NULL) is fully written, not accumulated into. */
+int msda_fused_backward_deterministic(int dtype, int raw_dtype,
+                                      const void* grad_output,
+                                      const void* value, const int64_t* spatial_shapes, const int64_t* level_start_index,
+                                      const float* reference_points, int ref_dim,
+                                      const void* sampling_offsets_raw, int64_t offsets_query_stride,
+                                      const void* attention_logits_raw, int64_t logits_query_stride,
+                                      int batch, int spatial_size, int num_heads, int channels,
+                                      int num_levels, int num_query, int num_point,
+                                      void* grad_value, void* grad_offsets_raw, void* grad_logits_raw,
+                                      float* grad_reference_points, void* grad_value_accum_f32,
+                                      void* scratch, int64_t scratch_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Layer epilogues around the deformable attention (no counterpart symbol in the reference, which
@@ -376,6 +420,13 @@ int msda_roi_align_backward(int dtype, const void* grad_pooled, const void* rois
                             int width, int channels, int num_rois, int pooled_height, int pooled_width,
                             double spatial_scale, int sampling_ratio, int aligned, void* grad_feature_accum,
                             void* stream);
+/* msda_roi_align_backward with the guarantee of msda_backward_deterministic (see there).  grad_feature
+ * [batch, height*width, channels] is in `dtype` (not an FP32 accumulator) and fully written; the bound is
+ * num_rois * pooled_height * pooled_width * max |grad_pooled| (a bin adds at most |grad_pooled| to any pixel). */
+int msda_roi_align_backward_deterministic(int dtype, const void* grad_pooled, const void* rois, int batch, int height,
+                                          int width, int channels, int num_rois, int pooled_height, int pooled_width,
+                                          double spatial_scale, int sampling_ratio, int aligned, void* grad_feature,
+                                          void* scratch, int64_t scratch_bytes, void* stream);
 
 #ifdef __cplusplus
 }
