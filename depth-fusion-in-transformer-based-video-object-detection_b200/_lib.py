@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # MSDA_B200_LIB selects another build of the same ABI (A/B kernel experiments); default: in-tree
 LIB_PATH = os.environ.get("MSDA_B200_LIB") or os.path.join(_HERE, "libmsda_b200.so")
 
-ABI_VERSION = 23
+ABI_VERSION = 24
 DTYPE_F32, DTYPE_F64, DTYPE_BF16, DTYPE_F16 = 0, 1, 2, 3
 FLAG_FORCE_GENERIC = 1
 FLAG_TC = 4
@@ -127,6 +127,25 @@ def load():
     lib.msda_layer_norm_act_supported.argtypes = [c_int, c_int]
     lib.msda_layer_norm_act_forward.restype = c_int
     lib.msda_layer_norm_act_forward.argtypes = [c_int, c_vp, c_vp, c_vp, c_i64, c_int, c_f, c_int, c_vp, c_vp]
+    lib.msda_layer_dropout_rule.restype = c_int
+    lib.msda_layer_dropout_rule.argtypes = [c_f, ctypes.POINTER(ctypes.c_uint32), ctypes.POINTER(c_f)]
+    lib.msda_layer_add_layernorm_dropout_supported.restype = c_int
+    lib.msda_layer_add_layernorm_dropout_supported.argtypes = [c_int, c_int]
+    lib.msda_layer_add_layernorm_dropout_forward.restype = c_int
+    lib.msda_layer_add_layernorm_dropout_forward.argtypes = lib.msda_layer_add_layernorm_forward.argtypes[:-1] + \
+        [c_f, c_vp, c_vp]
+    lib.msda_layer_add_layernorm_dropout_backward.restype = c_int
+    lib.msda_layer_add_layernorm_dropout_backward.argtypes = lib.msda_layer_add_layernorm_backward.argtypes[:-1] + \
+        [c_f, c_vp, c_vp]
+    lib.msda_layer_dropout.restype = c_int
+    lib.msda_layer_dropout.argtypes = [c_int, c_vp, c_vp, c_i64, c_f, c_vp, c_vp]
+    lib.msda_layer_relu_dropout_grad.restype = c_int
+    lib.msda_layer_relu_dropout_grad.argtypes = [c_int, c_vp, c_vp, c_vp, c_i64, c_f, c_vp]
+    lib.msda_layer_linear_bf16_relu_dropout.restype = c_int
+    lib.msda_layer_linear_bf16_relu_dropout.argtypes = [c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_f, c_vp, c_vp, c_vp]
+    lib.msda_layer_linear_tf32x3_relu_dropout.restype = c_int
+    lib.msda_layer_linear_tf32x3_relu_dropout.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_int, c_f, c_vp, c_vp,
+                                                          c_vp]
     lib.msda_layer_colsum_blocks.restype = c_int
     lib.msda_layer_colsum_blocks.argtypes = [c_int, c_i64, c_int]
     lib.msda_layer_colsum.restype = c_int

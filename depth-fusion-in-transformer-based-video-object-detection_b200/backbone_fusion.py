@@ -14,7 +14,7 @@ off by one stage, SURVEY.md section 9.2) and the convolutional stems are outside
 import torch
 from torch import nn
 
-from .ops.functions import add_layer_norm, linear
+from .ops.functions import add_layer_norm, dropout, linear
 from .ops.modules import MSDeformAttn
 from .transformer_layers import _add_pos, _get_activation_fn, encoder_reference_points
 
@@ -42,16 +42,16 @@ class DepthDeformableTransformerEncoderLayer(nn.Module):
         return _add_pos(tensor, pos)
 
     def forward_ffn(self, tgt):
-        if (self.dropout4.training and self.dropout4.p > 0) or self._activation_name not in ("relu", "gelu"):
-            return add_layer_norm(self.norm3, self.dropout4(self.activation(linear(self.linear1, tgt))), tgt)
-        return add_layer_norm(self.norm3, linear(self.linear1, tgt), tgt, self._activation_name)
+        if self._activation_name not in ("relu", "gelu"):
+            return add_layer_norm(self.norm3, dropout(self.dropout4, self.activation(linear(self.linear1, tgt))), tgt)
+        return add_layer_norm(self.norm3, linear(self.linear1, tgt), tgt, self._activation_name, dropout=self.dropout4)
 
     def forward(self, tgt, query_pos, src_pos, tgt_spatial_shapes, reference_points, depth_reference_points,
                 src, src_spatial_shapes, frame_start_index, tgt_padding_mask=None, src_padding_mask=None):
         src = add_layer_norm(self.norm_depth_scale, linear(self.depth_scale_adapt, src))
         sampled = self.cross_attn(_add_pos(tgt, query_pos), reference_points, src, src_spatial_shapes,
                                   frame_start_index, src_padding_mask)
-        tgt = add_layer_norm(self.norm1, self.dropout1(linear(self.cross_scale_adapt, sampled)), tgt)
+        tgt = add_layer_norm(self.norm1, linear(self.cross_scale_adapt, sampled), tgt, dropout=self.dropout1)
         return self.forward_ffn(tgt)
 
 

@@ -66,15 +66,25 @@ template <typename T> __device__ __forceinline__ void store16(T* p, const float*
 // round-trip through the storage type (y_pos is defined on the ROUNDED y, like the unfused chain)
 template <typename T> __device__ __forceinline__ float round_to(float v) { return to_f32<T>(from_f32<T>(v)); }
 
+// keep bits of the V elements from flat index e0 on (e0 % 8 + V <= 8): bit i = element e0 + i kept
+__device__ __forceinline__ unsigned keep_bits(long long e0, unsigned long long key, unsigned thresh)
+{
+    return dropout_keep8((unsigned long long)e0 >> 3, key, thresh) >> (e0 & 7);
+}
+// a * mask * scale: a dropped element is a * 0, so NaN and Inf propagate as in torch's dropout
+__device__ __forceinline__ float drop_mul(unsigned bits, int e, float scale) { return (bits >> e) & 1u ? scale : 0.f; }
+
 constexpr int kLnWarps = 8;
 
 // K = 16-byte chunks per lane: C = K * 32 * (16 / sizeof(T)).
-template <typename T, int K, int ACT>
+// DROP: v = residual + act(branch) * mask * scale (dropout on the branch, mask of element row * C + c).
+template <typename T, int K, int ACT, bool DROP>
 __global__ void __launch_bounds__(kLnWarps * 32)
 add_layernorm_fwd_kernel(const T* __restrict__ branch, const T* __restrict__ residual,
                          const T* __restrict__ gamma, const T* __restrict__ beta, const T* __restrict__ pos,
                          T* __restrict__ y, T* __restrict__ y_pos, float* __restrict__ mean_out,
-                         float* __restrict__ rstd_out, long long rows, float eps)
+                         float* __restrict__ rstd_out, long long rows, float eps,
+                         const unsigned long long* __restrict__ drop_key, unsigned drop_thresh, float drop_scale)
 {
     constexpr int V = Vec16<T>::n;
     constexpr int C = K * 32 * V;
@@ -88,11 +98,21 @@ add_layernorm_fwd_kernel(const T* __restrict__ branch, const T* __restrict__ res
         load16<T>(gamma + (k * 32 + lane) * V, g[k]);
         load16<T>(beta + (k * 32 + lane) * V, b[k]);
     }
+    unsigned long long key = 0;
+    if constexpr (DROP) key = *drop_key;
     for (long long row = warp0; row < rows; row += nwarps) {
         const long long base = row * C;
         float v[K][V];
 #pragma unroll
         for (int k = 0; k < K; ++k) load16_stream<T>(branch + base + (k * 32 + lane) * V, v[k]);
+        if constexpr (DROP) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+                const unsigned bits = keep_bits(base + (k * 32 + lane) * V, key, drop_thresh);
+#pragma unroll
+                for (int e = 0; e < V; ++e) v[k][e] = act_fwd<ACT>(v[k][e]) * drop_mul(bits, e, drop_scale);
+            }
+        }
         if (residual != nullptr) {
             float r[K][V];
 #pragma unroll
@@ -100,8 +120,8 @@ add_layernorm_fwd_kernel(const T* __restrict__ branch, const T* __restrict__ res
 #pragma unroll
             for (int k = 0; k < K; ++k)
 #pragma unroll
-                for (int e = 0; e < V; ++e) v[k][e] = r[k][e] + act_fwd<ACT>(v[k][e]);
-        } else {
+                for (int e = 0; e < V; ++e) v[k][e] = r[k][e] + (DROP ? v[k][e] : act_fwd<ACT>(v[k][e]));
+        } else if constexpr (!DROP) {
 #pragma unroll
             for (int k = 0; k < K; ++k)
 #pragma unroll
@@ -143,13 +163,15 @@ add_layernorm_fwd_kernel(const T* __restrict__ branch, const T* __restrict__ res
 // d_branch = d v * act'(branch), d_residual = d v, with
 //   d v = rstd * (gy*gamma - mean_c(gy*gamma) - xhat * mean_c(gy*gamma*xhat)),  gy = dy (+ dy_pos)
 // partial[blockIdx][0][c] = sum over this CTA's rows of gy*xhat, partial[blockIdx][1][c] = sum of gy.
-template <typename T, int K, int ACT>
-__global__ void __launch_bounds__(kLnWarps * 32)
+// DROP: the forward's mask is regenerated from the key, both for v and for d_branch = d v * mask * scale * act'(branch).
+template <typename T, int K, int ACT, bool DROP>
+__global__ void __launch_bounds__(kLnWarps * 32, DROP ? 1 : 0)
 add_layernorm_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ dy_pos, const T* __restrict__ branch,
                          const T* __restrict__ residual, const T* __restrict__ gamma,
                          const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
                          T* __restrict__ d_branch, T* __restrict__ d_residual, float* __restrict__ partial,
-                         long long rows)
+                         long long rows, const unsigned long long* __restrict__ drop_key, unsigned drop_thresh,
+                         float drop_scale)
 {
     constexpr int V = Vec16<T>::n;
     constexpr int C = K * 32 * V;
@@ -165,9 +187,16 @@ add_layernorm_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ dy_pos,
 #pragma unroll
         for (int e = 0; e < V; ++e) { dg[k][e] = 0.f; db[k][e] = 0.f; }
     }
+    unsigned long long key = 0;
+    if constexpr (DROP) key = *drop_key;
     for (long long row = warp0; row < rows; row += nwarps) {
         const long long base = row * C;
         float gy[K][V], x[K][V], v[K][V];
+        unsigned bits[K];
+        if constexpr (DROP) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) bits[k] = keep_bits(base + (k * 32 + lane) * V, key, drop_thresh);
+        }
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             load16_stream<T>(dy + base + (k * 32 + lane) * V, gy[k]);
@@ -188,12 +217,14 @@ add_layernorm_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ dy_pos,
 #pragma unroll
             for (int k = 0; k < K; ++k)
 #pragma unroll
-                for (int e = 0; e < V; ++e) v[k][e] += act_fwd<ACT>(x[k][e]);
+                for (int e = 0; e < V; ++e)
+                    v[k][e] += DROP ? act_fwd<ACT>(x[k][e]) * drop_mul(bits[k], e, drop_scale) : act_fwd<ACT>(x[k][e]);
         } else {
 #pragma unroll
             for (int k = 0; k < K; ++k)
 #pragma unroll
-                for (int e = 0; e < V; ++e) v[k][e] = act_fwd<ACT>(x[k][e]);
+                for (int e = 0; e < V; ++e)
+                    v[k][e] = DROP ? act_fwd<ACT>(x[k][e]) * drop_mul(bits[k], e, drop_scale) : act_fwd<ACT>(x[k][e]);
         }
         const float mean = mean_in[row], rstd = rstd_in[row];
         float c1 = 0.f, c2 = 0.f;
@@ -218,7 +249,11 @@ add_layernorm_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ dy_pos,
 #pragma unroll
             for (int e = 0; e < V; ++e) dv[e] = rstd * (gy[k][e] - c1 - v[k][e] * c2);
             if (d_residual != nullptr) store16<T>(d_residual + base + (k * 32 + lane) * V, dv);
-            if (ACT != kActNone || d_residual == nullptr) {
+            if (DROP) {
+#pragma unroll
+                for (int e = 0; e < V; ++e) dv[e] *= drop_mul(bits[k], e, drop_scale) * act_bwd<ACT>(x[k][e]);
+                store16<T>(d_branch + base + (k * 32 + lane) * V, dv);
+            } else if (ACT != kActNone || d_residual == nullptr) {
 #pragma unroll
                 for (int e = 0; e < V; ++e) dv[e] *= act_bwd<ACT>(x[k][e]);
                 store16<T>(d_branch + base + (k * 32 + lane) * V, dv);
@@ -520,14 +555,14 @@ int add_layernorm_chunks(int dtype, int C)
     return (k == 1 || k == 2 || k == 4) ? k : 0;
 }
 
-template <typename T, int K>
+template <typename T, int K, bool DROP>
 static cudaError_t launch_ln_fwd(const AddLayerNormArgs& a, cudaStream_t st)
 {
     const int grid = ln_grid(a.rows);
 #define MSDA_LN_FWD(ACT) \
-    add_layernorm_fwd_kernel<T, K, ACT><<<grid, kLnWarps * 32, 0, st>>>( \
+    add_layernorm_fwd_kernel<T, K, ACT, DROP><<<grid, kLnWarps * 32, 0, st>>>( \
         (const T*)a.branch, (const T*)a.residual, (const T*)a.gamma, (const T*)a.beta, (const T*)a.pos, \
-        (T*)a.y, (T*)a.y_pos, a.mean, a.rstd, a.rows, a.eps)
+        (T*)a.y, (T*)a.y_pos, a.mean, a.rstd, a.rows, a.eps, a.drop_key, a.drop.thresh, a.drop.scale)
     switch (a.act) {
         case kActNone: MSDA_LN_FWD(kActNone); break;
         case kActRelu: MSDA_LN_FWD(kActRelu); break;
@@ -538,14 +573,14 @@ static cudaError_t launch_ln_fwd(const AddLayerNormArgs& a, cudaStream_t st)
     return cudaGetLastError();
 }
 
-template <typename T, int K>
+template <typename T, int K, bool DROP>
 static cudaError_t launch_ln_bwd(const AddLayerNormArgs& a, cudaStream_t st)
 {
     const int grid = a.partial_blocks;
 #define MSDA_LN_BWD(ACT) \
-    add_layernorm_bwd_kernel<T, K, ACT><<<grid, kLnWarps * 32, 0, st>>>( \
+    add_layernorm_bwd_kernel<T, K, ACT, DROP><<<grid, kLnWarps * 32, 0, st>>>( \
         (const T*)a.dy, (const T*)a.dy_pos, (const T*)a.branch, (const T*)a.residual, (const T*)a.gamma, \
-        a.mean, a.rstd, (T*)a.d_branch, (T*)a.d_residual, a.partial, a.rows)
+        a.mean, a.rstd, (T*)a.d_branch, (T*)a.d_residual, a.partial, a.rows, a.drop_key, a.drop.thresh, a.drop.scale)
     switch (a.act) {
         case kActNone: MSDA_LN_BWD(kActNone); break;
         case kActRelu: MSDA_LN_BWD(kActRelu); break;
@@ -559,18 +594,33 @@ static cudaError_t launch_ln_bwd(const AddLayerNormArgs& a, cudaStream_t st)
     return cudaGetLastError();
 }
 
-template <typename T>
+template <typename T, bool DROP>
 static cudaError_t dispatch_ln(const AddLayerNormArgs& a, bool backward, cudaStream_t st)
 {
     switch (add_layernorm_chunks(a.dtype, a.C)) {
-        case 1: return backward ? launch_ln_bwd<T, 1>(a, st) : launch_ln_fwd<T, 1>(a, st);
-        case 2: return backward ? launch_ln_bwd<T, 2>(a, st) : launch_ln_fwd<T, 2>(a, st);
-        case 4: return backward ? launch_ln_bwd<T, 4>(a, st) : launch_ln_fwd<T, 4>(a, st);
+        case 1: return backward ? launch_ln_bwd<T, 1, DROP>(a, st) : launch_ln_fwd<T, 1, DROP>(a, st);
+        case 2: return backward ? launch_ln_bwd<T, 2, DROP>(a, st) : launch_ln_fwd<T, 2, DROP>(a, st);
+        case 4:
+            if constexpr (DROP) return cudaErrorInvalidValue;       // see add_layernorm_dropout_supported
+            else return backward ? launch_ln_bwd<T, 4, false>(a, st) : launch_ln_fwd<T, 4, false>(a, st);
         default: return cudaErrorInvalidValue;
     }
 }
+template <typename T>
+static cudaError_t dispatch_ln(const AddLayerNormArgs& a, bool backward, cudaStream_t st)
+{
+    return a.drop_key != nullptr ? dispatch_ln<T, true>(a, backward, st) : dispatch_ln<T, false>(a, backward, st);
+}
 
 int add_layernorm_partial_blocks(long long rows) { return ln_grid(rows); }
+
+// With dropout: one or two 16-byte chunks per lane (up to 512 channels of a 16-bit type, 256 of fp32).  The four-chunk
+// GELU backward already spills without dropout; the dropout instantiations stop at two chunks and spill nothing.
+bool add_layernorm_dropout_supported(int dtype, int C)
+{
+    const int k = add_layernorm_chunks(dtype, C);
+    return k == 1 || k == 2;
+}
 
 cudaError_t add_layernorm(const AddLayerNormArgs& a, bool backward, cudaStream_t st)
 {
@@ -1042,6 +1092,115 @@ cudaError_t zero_masked_rows(int dtype, void* data, const unsigned char* mask, l
     const int grid = (int)(want < 148 * 8 ? want : 148 * 8);
     if (esz == 4) zero_masked_rows_kernel<float><<<grid, 256, 0, st>>>((float*)data, mask, rows, C);
     else zero_masked_rows_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((__nv_bfloat16*)data, mask, rows, C);
+    return cudaGetLastError();
+}
+
+// Standalone dropout, y = x * mask * scale (x == y allowed): thread = one group of 8 elements = one Philox call, 16-byte
+// accesses when both pointers are 16-byte aligned (`vec`), element by element for the tail group.
+template <typename T>
+__global__ void __launch_bounds__(256)
+dropout_kernel(const T* x, T* y, long long n, const unsigned long long* __restrict__ key_ptr, unsigned thresh,
+               float scale, int vec)
+{
+    constexpr int V = Vec16<T>::n;
+    const unsigned long long key = *key_ptr;
+    const long long groups = (n + 7) >> 3;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < groups; g += stride) {
+        const unsigned bits = dropout_keep8((unsigned long long)g, key, thresh);
+        const long long e0 = g << 3;
+        if (vec && e0 + 8 <= n) {
+#pragma unroll
+            for (int h = 0; h < 8 / V; ++h) {
+                float f[V];
+                load16<T>(x + e0 + h * V, f);
+#pragma unroll
+                for (int e = 0; e < V; ++e) f[e] *= drop_mul(bits, h * V + e, scale);
+                store16<T>(y + e0 + h * V, f);
+            }
+        } else {
+            for (int i = 0; i < 8 && e0 + i < n; ++i)
+                y[e0 + i] = from_f32<T>(to_f32<T>(x[e0 + i]) * drop_mul(bits, i, scale));
+        }
+    }
+}
+
+// Backward of dropout(relu(.)) from its saved output: dx = out > 0 ? g * scale : 0.  A dropped element and a non-positive
+// pre-activation both have out == 0, so neither the mask nor the key is needed.
+template <typename T>
+__global__ void __launch_bounds__(256)
+relu_dropout_grad_kernel(const T* __restrict__ g, const T* __restrict__ out, T* dx, long long n, float scale, int vec)
+{
+    constexpr int V = Vec16<T>::n;
+    const long long chunks = (n + V - 1) / V;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < chunks; c += stride) {
+        const long long e0 = c * V;
+        if (vec && e0 + V <= n) {
+            float fg[V], fo[V];
+            load16_stream<T>(g + e0, fg);
+            load16_stream<T>(out + e0, fo);
+#pragma unroll
+            for (int e = 0; e < V; ++e) fg[e] = fo[e] > 0.f ? fg[e] * scale : 0.f;
+            store16<T>(dx + e0, fg);
+        } else {
+            for (long long e = e0; e < n && e < e0 + V; ++e)
+                dx[e] = from_f32<T>(to_f32<T>(out[e]) > 0.f ? to_f32<T>(g[e]) * scale : 0.f);
+        }
+    }
+}
+
+static int elementwise_grid(long long items)
+{
+    const long long want = (items + 255) / 256;
+    return (int)(want < 148 * 16 ? (want > 0 ? want : 1) : 148 * 16);
+}
+
+cudaError_t dropout(int dtype, const void* x, void* y, long long n, const unsigned long long* key, DropoutRule rule,
+                    cudaStream_t st)
+{
+    if (n < 0 || key == nullptr) return cudaErrorInvalidValue;
+    if (n == 0) return cudaSuccess;
+    const int vec = (reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) % 16 == 0;
+    const int grid = elementwise_grid((n + 7) / 8);
+    switch (dtype) {
+        case kF32:
+            dropout_kernel<float><<<grid, 256, 0, st>>>((const float*)x, (float*)y, n, key, rule.thresh, rule.scale, vec);
+            break;
+        case kBF16:
+            dropout_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((const __nv_bfloat16*)x, (__nv_bfloat16*)y, n, key,
+                                                                 rule.thresh, rule.scale, vec);
+            break;
+        case kF16:
+            dropout_kernel<__half><<<grid, 256, 0, st>>>((const __half*)x, (__half*)y, n, key, rule.thresh, rule.scale, vec);
+            break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t relu_dropout_grad(int dtype, const void* g, const void* out, void* dx, long long n, float scale,
+                              cudaStream_t st)
+{
+    if (n < 0) return cudaErrorInvalidValue;
+    if (n == 0) return cudaSuccess;
+    const int vec = (reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(dx)) %
+                    16 == 0;
+    switch (dtype) {
+        case kF32:
+            relu_dropout_grad_kernel<float><<<elementwise_grid((n + 3) / 4), 256, 0, st>>>(
+                (const float*)g, (const float*)out, (float*)dx, n, scale, vec);
+            break;
+        case kBF16:
+            relu_dropout_grad_kernel<__nv_bfloat16><<<elementwise_grid((n + 7) / 8), 256, 0, st>>>(
+                (const __nv_bfloat16*)g, (const __nv_bfloat16*)out, (__nv_bfloat16*)dx, n, scale, vec);
+            break;
+        case kF16:
+            relu_dropout_grad_kernel<__half><<<elementwise_grid((n + 7) / 8), 256, 0, st>>>(
+                (const __half*)g, (const __half*)out, (__half*)dx, n, scale, vec);
+            break;
+        default: return cudaErrorInvalidValue;
+    }
     return cudaGetLastError();
 }
 

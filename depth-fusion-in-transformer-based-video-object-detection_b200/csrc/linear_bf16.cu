@@ -69,10 +69,13 @@ __device__ __forceinline__ unsigned long long lb_desc(const void* smem_ptr)
     return d;
 }
 
+// DROP: dropout after the ReLU, mask of element row * N + col (dropout_keep8: one Philox call per 8 columns a lane packs)
+template <bool DROP>
 __global__ void __cluster_dims__(kLbCluster, 1, 1) __launch_bounds__(kLbThreads, 1)
 linear_bf16_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w,
                    const __grid_constant__ CUtensorMap tm_y, const __nv_bfloat16* __restrict__ bias,
-                   const unsigned char* __restrict__ row_mask, long long rows, int N, int K, int relu, int bn)
+                   const unsigned char* __restrict__ row_mask, long long rows, int N, int K, int relu, int bn,
+                   const unsigned long long* __restrict__ drop_key, unsigned drop_thresh, float drop_scale)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     unsigned char* s_out = smem + kLbStages * kLbStageBytes;            // [8 epilogue warps][kLbOutBytes], 1024-byte aligned
@@ -160,6 +163,8 @@ linear_bf16_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
         // two warps per TMEM lane quadrant: warps 0-3 take the even 64-column chunks, warps 4-7 the odd ones
         const int quad = warp & 3, half = warp >> 2;
         const unsigned lane_base = (unsigned)(quad * 32) << 16;
+        unsigned long long key = 0;
+        if constexpr (DROP) key = *drop_key;
         unsigned it = 0;
         for (long long t = first; t < tiles; t += stride, ++it) {
             const long long m0 = ((t / tiles_n) * kLbCluster + rank) * kLbBM;
@@ -187,10 +192,14 @@ linear_bf16_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_consta
 #pragma unroll
                 for (int q = 0; q < 8; ++q) {
                     float o[8];
+                    unsigned bits = 0;
+                    if constexpr (DROP)
+                        bits = dropout_keep8((unsigned long long)(row * N + n0 + c + 8 * q) >> 3, key, drop_thresh);
 #pragma unroll
                     for (int e = 0; e < 8; ++e) {
                         o[e] = v[8 * q + e] + s_bias[c + 8 * q + e];
                         if (relu) o[e] = fmaxf(o[e], 0.f);
+                        if constexpr (DROP) o[e] *= (bits >> e) & 1u ? drop_scale : 0.f;
                         if (dead) o[e] = 0.f;
                     }
                     *reinterpret_cast<uint4*>(stage + lane * 128 + ((q ^ (lane & 7)) << 4)) = pack<__nv_bfloat16>(o);
@@ -256,8 +265,10 @@ bool linear_bf16_supported(int n, int k)
     return n >= 64 && n % 64 == 0 && k >= 64 && k % 64 == 0;
 }
 
-cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const unsigned char* row_mask, long long rows, int n,
-                        int k, int relu, void* y, cudaStream_t stream)
+template <bool DROP>
+static cudaError_t launch_linear_bf16(const void* x, const void* w, const void* bias, const unsigned char* row_mask,
+                                      long long rows, int n, int k, int relu, const unsigned long long* key,
+                                      DropoutRule rule, void* y, cudaStream_t stream)
 {
     if (!linear_bf16_supported(n, k) || rows < 0 || rows >= (1ll << 31) - 1024) return cudaErrorInvalidValue;
     if (rows == 0) return cudaSuccess;
@@ -267,7 +278,7 @@ cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const un
     cudaGetDevice(&dev);
     static bool configured[64] = {};          // the attribute is per device: one process may drive several GPUs
     if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(linear_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLbSmem);
+        cudaError_t e = cudaFuncSetAttribute(linear_bf16_kernel<DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLbSmem);
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) configured[dev] = true;
     }
@@ -285,9 +296,22 @@ cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const un
     const long long units = ((tiles_m + kLbCluster - 1) / kLbCluster) * ((n + bn - 1) / bn);
     const long long clusters = sms / kLbCluster;
     const int grid = (int)(units < clusters ? units : clusters) * kLbCluster;
-    linear_bf16_kernel<<<grid, kLbThreads, kLbSmem, stream>>>(tm_x, tm_w, tm_y, (const __nv_bfloat16*)bias, row_mask, rows, n, k,
-                                                               relu, bn);
+    linear_bf16_kernel<DROP><<<grid, kLbThreads, kLbSmem, stream>>>(tm_x, tm_w, tm_y, (const __nv_bfloat16*)bias, row_mask, rows,
+                                                                     n, k, relu, bn, key, rule.thresh, rule.scale);
     return cudaGetLastError();
+}
+
+cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const unsigned char* row_mask, long long rows, int n,
+                        int k, int relu, void* y, cudaStream_t stream)
+{
+    return launch_linear_bf16<false>(x, w, bias, row_mask, rows, n, k, relu, nullptr, DropoutRule{0u, 1.f}, y, stream);
+}
+
+cudaError_t linear_bf16_relu_dropout(const void* x, const void* w, const void* bias, long long rows, int n, int k,
+                                     const unsigned long long* key, DropoutRule rule, void* y, cudaStream_t stream)
+{
+    if (key == nullptr) return cudaErrorInvalidValue;
+    return launch_linear_bf16<true>(x, w, bias, nullptr, rows, n, k, 1, key, rule, y, stream);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -98,10 +98,14 @@ __device__ __forceinline__ void mma_tf32(unsigned tmem_d, unsigned long long des
 // two ROW tiles of the same column tile in lockstep, each loads HALF of every W tile and multicasts it into both CTAs'
 // shared memory: 48 KB per K block and CTA.  A stage is released by the MMAs of BOTH CTAs (multicast tcgen05.commit on
 // the `empty` barrier of each).
+//
+// DROP: dropout after the ReLU, mask of element row * N + col (dropout_keep8: one Philox call per two float4 of a lane).
+template <bool DROP>
 __global__ void __cluster_dims__(kLtCluster, 1, 1) __launch_bounds__(kLtThreads, 1)
 linear_tf32x3_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_wh,
                      const __grid_constant__ CUtensorMap tm_wl, const __grid_constant__ CUtensorMap tm_y,
-                     const float* __restrict__ bias, long long rows, int N, int K, int relu, int bn)
+                     const float* __restrict__ bias, long long rows, int N, int K, int relu, int bn,
+                     const unsigned long long* __restrict__ drop_key, unsigned drop_thresh, float drop_scale)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     unsigned char* s_out = smem + kLtStages * kLtStageBytes;            // [8 epilogue warps][kLtOutBytes], 1024-byte aligned
@@ -235,6 +239,8 @@ linear_tf32x3_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
         // two warps per TMEM lane quadrant (warp % 4): warps 0-3 take the even 32-column chunks, warps 10-13 the odd ones
         const int quad = warp & 3, half = warp < 4 ? 0 : 1, et = half * 128 + quad * 32 + lane;
         const unsigned lane_base = (unsigned)(quad * 32) << 16;
+        unsigned long long key = 0;
+        if constexpr (DROP) key = *drop_key;
         unsigned it = 0;
         for (long long t = first; t < tiles; t += stride, ++it) {
             const long long m0 = ((t / tiles_n) * kLtCluster + rank) * kLtBM;
@@ -258,12 +264,23 @@ linear_tf32x3_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
                 tmem_ld32(tmem + kLtBN + c + lane_base, w);
                 if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
                 __syncwarp();
+                unsigned bits = 0;
 #pragma unroll
                 for (int q = 0; q < 8; ++q) {
                     const float4 b4 = *reinterpret_cast<const float4*>(s_bias + c + 4 * q);
                     float4 o = make_float4(v[4 * q] + w[4 * q] + b4.x, v[4 * q + 1] + w[4 * q + 1] + b4.y,
                                            v[4 * q + 2] + w[4 * q + 2] + b4.z, v[4 * q + 3] + w[4 * q + 3] + b4.w);
                     if (relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
+                    if constexpr (DROP) {
+                        if ((q & 1) == 0)
+                            bits = dropout_keep8((unsigned long long)((long long)(row0 + lane) * N + n0 + c + 4 * q) >> 3, key,
+                                                 drop_thresh);
+                        const unsigned b = bits >> (4 * (q & 1));
+                        o.x *= b & 1u ? drop_scale : 0.f;
+                        o.y *= b & 2u ? drop_scale : 0.f;
+                        o.z *= b & 4u ? drop_scale : 0.f;
+                        o.w *= b & 8u ? drop_scale : 0.f;
+                    }
                     *reinterpret_cast<float4*>(stage + lane * 128 + ((q ^ (lane & 7)) << 4)) = o;
                 }
                 fence_proxy_async();                 // generic-proxy writes -> TMA (async proxy) read
@@ -329,8 +346,10 @@ bool linear_tf32x3_supported(int n, int k)
     return n >= 32 && n % 32 == 0 && k >= 32 && k % 32 == 0;
 }
 
-cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, const float* bias, long long rows, int n,
-                          int k, int relu, float* y, cudaStream_t stream)
+template <bool DROP>
+static cudaError_t launch_linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, const float* bias,
+                                        long long rows, int n, int k, int relu, const unsigned long long* key,
+                                        DropoutRule rule, float* y, cudaStream_t stream)
 {
     if (!linear_tf32x3_supported(n, k) || rows < 0 || rows >= (1ll << 31) - 1024) return cudaErrorInvalidValue;   // row coordinates are int
     if (rows == 0) return cudaSuccess;
@@ -341,7 +360,7 @@ cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, 
     cudaGetDevice(&dev);
     static bool configured[64] = {};          // the attribute is per device: one process may drive several GPUs
     if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(linear_tf32x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLtSmem);
+        cudaError_t e = cudaFuncSetAttribute(linear_tf32x3_kernel<DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLtSmem);
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) configured[dev] = true;
     }
@@ -360,8 +379,23 @@ cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, 
     const long long units = ((tiles_m + kLtCluster - 1) / kLtCluster) * ((n + bn - 1) / bn);
     const long long clusters = sms / kLtCluster;
     const int grid = (int)(units < clusters ? units : clusters) * kLtCluster;
-    linear_tf32x3_kernel<<<grid, kLtThreads, kLtSmem, stream>>>(tm_x, tm_wh, tm_wl, tm_y, bias, rows, n, k, relu, bn);
+    linear_tf32x3_kernel<DROP><<<grid, kLtThreads, kLtSmem, stream>>>(tm_x, tm_wh, tm_wl, tm_y, bias, rows, n, k, relu, bn,
+                                                                       key, rule.thresh, rule.scale);
     return cudaGetLastError();
+}
+
+cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, const float* bias, long long rows, int n,
+                          int k, int relu, float* y, cudaStream_t stream)
+{
+    return launch_linear_tf32x3<false>(x, w_hi, w_lo, bias, rows, n, k, relu, nullptr, DropoutRule{0u, 1.f}, y, stream);
+}
+
+cudaError_t linear_tf32x3_relu_dropout(const float* x, const float* w_hi, const float* w_lo, const float* bias,
+                                       long long rows, int n, int k, const unsigned long long* key, DropoutRule rule,
+                                       float* y, cudaStream_t stream)
+{
+    if (key == nullptr) return cudaErrorInvalidValue;
+    return launch_linear_tf32x3<true>(x, w_hi, w_lo, bias, rows, n, k, 1, key, rule, y, stream);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -7,7 +7,7 @@ static bool bad_dims(int N, int S, int M, int D, int L, int Lq, int P)
     return N < 0 || S < 0 || M < 0 || D < 0 || L < 0 || Lq < 0 || P < 0;
 }
 
-extern "C" int msda_abi_version(void) { return 23; }
+extern "C" int msda_abi_version(void) { return 24; }
 
 extern "C" const char* msda_error_string(int code)
 {
@@ -207,10 +207,10 @@ extern "C" int msda_layer_add_layernorm_partial_blocks(int64_t rows)
     return msda::add_layernorm_partial_blocks((long long)rows);
 }
 
-extern "C" int msda_layer_add_layernorm_forward(int dtype, int act, const void* branch, const void* residual,
-                                                const void* gamma, const void* beta, const void* pos,
-                                                int64_t rows, int channels, float eps, void* y, void* y_pos,
-                                                float* mean, float* rstd, void* stream)
+static int add_layernorm_forward(int dtype, int act, const void* branch, const void* residual, const void* gamma,
+                                 const void* beta, const void* pos, int64_t rows, int channels, float eps, void* y,
+                                 void* y_pos, float* mean, float* rstd, const uint64_t* drop_key, msda::DropoutRule drop,
+                                 void* stream)
 {
     if (rows < 0 || msda::add_layernorm_chunks(dtype, channels) == 0 || (y_pos != nullptr) != (pos != nullptr) ||
         (mean != nullptr) != (rstd != nullptr))
@@ -219,21 +219,31 @@ extern "C" int msda_layer_add_layernorm_forward(int dtype, int act, const void* 
     a.dtype = dtype; a.act = act; a.rows = rows; a.C = channels; a.eps = eps;
     a.branch = branch; a.residual = residual; a.gamma = gamma; a.beta = beta; a.pos = pos;
     a.y = y; a.y_pos = y_pos; a.mean = mean; a.rstd = rstd;
+    a.drop_key = reinterpret_cast<const unsigned long long*>(drop_key); a.drop = drop;
     return (int)msda::add_layernorm(a, false, (cudaStream_t)stream);
 }
 
-extern "C" int msda_layer_add_layernorm_backward(int dtype, int act, const void* grad_y, const void* grad_y_pos,
-                                                 const void* branch, const void* residual, const void* gamma,
-                                                 const float* mean, const float* rstd, int64_t rows, int channels,
-                                                 void* grad_branch, void* grad_residual, void* grad_gamma,
-                                                 void* grad_beta, float* partial_scratch, int partial_blocks,
-                                                 void* stream)
+extern "C" int msda_layer_add_layernorm_forward(int dtype, int act, const void* branch, const void* residual,
+                                                const void* gamma, const void* beta, const void* pos,
+                                                int64_t rows, int channels, float eps, void* y, void* y_pos,
+                                                float* mean, float* rstd, void* stream)
+{
+    return add_layernorm_forward(dtype, act, branch, residual, gamma, beta, pos, rows, channels, eps, y, y_pos, mean, rstd,
+                                 nullptr, msda::DropoutRule{0u, 1.f}, stream);
+}
+
+static int add_layernorm_backward(int dtype, int act, const void* grad_y, const void* grad_y_pos, const void* branch,
+                                  const void* residual, const void* gamma, const float* mean, const float* rstd,
+                                  int64_t rows, int channels, void* grad_branch, void* grad_residual, void* grad_gamma,
+                                  void* grad_beta, float* partial_scratch, int partial_blocks, const uint64_t* drop_key,
+                                  msda::DropoutRule drop, void* stream)
 {
     if (rows < 0 || msda::add_layernorm_chunks(dtype, channels) == 0 || partial_blocks < 1 ||
         partial_blocks > msda::add_layernorm_partial_blocks((long long)rows) ||
         (grad_residual == nullptr) != (residual == nullptr))
         return (int)cudaErrorInvalidValue;
     msda::AddLayerNormArgs a = {};
+    a.drop_key = reinterpret_cast<const unsigned long long*>(drop_key); a.drop = drop;
     a.dtype = dtype; a.act = act; a.rows = rows; a.C = channels;
     a.branch = branch; a.residual = residual; a.gamma = gamma;
     a.mean = const_cast<float*>(mean); a.rstd = const_cast<float*>(rstd);
@@ -246,6 +256,78 @@ extern "C" int msda_layer_add_layernorm_backward(int dtype, int act, const void*
         return (int)cudaMemsetAsync(grad_beta, 0, channels * esz, (cudaStream_t)stream);
     }
     return (int)msda::add_layernorm(a, true, (cudaStream_t)stream);
+}
+
+extern "C" int msda_layer_add_layernorm_backward(int dtype, int act, const void* grad_y, const void* grad_y_pos,
+                                                 const void* branch, const void* residual, const void* gamma,
+                                                 const float* mean, const float* rstd, int64_t rows, int channels,
+                                                 void* grad_branch, void* grad_residual, void* grad_gamma,
+                                                 void* grad_beta, float* partial_scratch, int partial_blocks,
+                                                 void* stream)
+{
+    return add_layernorm_backward(dtype, act, grad_y, grad_y_pos, branch, residual, gamma, mean, rstd, rows, channels,
+                                  grad_branch, grad_residual, grad_gamma, grad_beta, partial_scratch, partial_blocks,
+                                  nullptr, msda::DropoutRule{0u, 1.f}, stream);
+}
+
+// ---- dropout (DESIGN.md section 3.16) ------------------------------------------------------------
+extern "C" int msda_layer_dropout_rule(float p, uint32_t* threshold, float* scale)
+{
+    msda::DropoutRule r;
+    if (!msda::dropout_rule(p, &r) || threshold == nullptr || scale == nullptr) return (int)cudaErrorInvalidValue;
+    *threshold = r.thresh;
+    *scale = r.scale;
+    return 0;
+}
+
+extern "C" int msda_layer_add_layernorm_dropout_supported(int dtype, int channels)
+{
+    return msda::add_layernorm_dropout_supported(dtype, channels) ? 1 : 0;
+}
+
+extern "C" int msda_layer_add_layernorm_dropout_forward(int dtype, int act, const void* branch, const void* residual,
+                                                        const void* gamma, const void* beta, const void* pos,
+                                                        int64_t rows, int channels, float eps, void* y, void* y_pos,
+                                                        float* mean, float* rstd, float p, const uint64_t* key,
+                                                        void* stream)
+{
+    msda::DropoutRule r;
+    if (!msda::dropout_rule(p, &r) || key == nullptr || !msda::add_layernorm_dropout_supported(dtype, channels))
+        return (int)cudaErrorInvalidValue;
+    return add_layernorm_forward(dtype, act, branch, residual, gamma, beta, pos, rows, channels, eps, y, y_pos, mean, rstd,
+                                 key, r, stream);
+}
+
+extern "C" int msda_layer_add_layernorm_dropout_backward(int dtype, int act, const void* grad_y, const void* grad_y_pos,
+                                                         const void* branch, const void* residual, const void* gamma,
+                                                         const float* mean, const float* rstd, int64_t rows,
+                                                         int channels, void* grad_branch, void* grad_residual,
+                                                         void* grad_gamma, void* grad_beta, float* partial_scratch,
+                                                         int partial_blocks, float p, const uint64_t* key, void* stream)
+{
+    msda::DropoutRule r;
+    if (!msda::dropout_rule(p, &r) || key == nullptr || !msda::add_layernorm_dropout_supported(dtype, channels) ||
+        grad_branch == nullptr || grad_branch == grad_residual)
+        return (int)cudaErrorInvalidValue;
+    return add_layernorm_backward(dtype, act, grad_y, grad_y_pos, branch, residual, gamma, mean, rstd, rows, channels,
+                                  grad_branch, grad_residual, grad_gamma, grad_beta, partial_scratch, partial_blocks, key,
+                                  r, stream);
+}
+
+extern "C" int msda_layer_dropout(int dtype, const void* x, void* y, int64_t n, float p, const uint64_t* key, void* stream)
+{
+    msda::DropoutRule r;
+    if (!msda::dropout_rule(p, &r) || key == nullptr) return (int)cudaErrorInvalidValue;
+    return (int)msda::dropout(dtype, x, y, (long long)n, reinterpret_cast<const unsigned long long*>(key), r,
+                              (cudaStream_t)stream);
+}
+
+extern "C" int msda_layer_relu_dropout_grad(int dtype, const void* grad_y, const void* y, void* grad_x, int64_t n, float p,
+                                            void* stream)
+{
+    msda::DropoutRule r;
+    if (!msda::dropout_rule(p, &r)) return (int)cudaErrorInvalidValue;
+    return (int)msda::relu_dropout_grad(dtype, grad_y, y, grad_x, (long long)n, r.scale, (cudaStream_t)stream);
 }
 
 extern "C" int msda_layer_zero_masked_rows(int dtype, void* data, const uint8_t* mask, int64_t rows, int channels,
@@ -464,6 +546,16 @@ extern "C" int msda_layer_linear_bf16(const void* x, const void* weight, const v
                                   (cudaStream_t)stream);
 }
 
+extern "C" int msda_layer_linear_bf16_relu_dropout(const void* x, const void* weight, const void* bias, int64_t rows,
+                                                   int out_features, int in_features, float p, const uint64_t* key, void* y,
+                                                   void* stream)
+{
+    msda::DropoutRule r;
+    if (rows < 0 || !msda::dropout_rule(p, &r) || key == nullptr) return (int)cudaErrorInvalidValue;
+    return (int)msda::linear_bf16_relu_dropout(x, weight, bias, (long long)rows, out_features, in_features,
+                                               reinterpret_cast<const unsigned long long*>(key), r, y, (cudaStream_t)stream);
+}
+
 extern "C" int msda_layer_linear_bf16_wgrad_supported(int out_features, int in_features)
 {
     return msda::linear_bf16_wgrad_supported(out_features, in_features) ? 1 : 0;
@@ -493,6 +585,17 @@ extern "C" int msda_layer_linear_tf32x3(const float* x, const float* weight_hi, 
     if (rows < 0) return (int)cudaErrorInvalidValue;
     return (int)msda::linear_tf32x3(x, weight_hi, weight_lo, bias, (long long)rows, out_features, in_features, relu, y,
                                     (cudaStream_t)stream);
+}
+
+extern "C" int msda_layer_linear_tf32x3_relu_dropout(const float* x, const float* weight_hi, const float* weight_lo,
+                                                     const float* bias, int64_t rows, int out_features, int in_features,
+                                                     float p, const uint64_t* key, float* y, void* stream)
+{
+    msda::DropoutRule r;
+    if (rows < 0 || !msda::dropout_rule(p, &r) || key == nullptr) return (int)cudaErrorInvalidValue;
+    return (int)msda::linear_tf32x3_relu_dropout(x, weight_hi, weight_lo, bias, (long long)rows, out_features, in_features,
+                                                 reinterpret_cast<const unsigned long long*>(key), r, y,
+                                                 (cudaStream_t)stream);
 }
 
 extern "C" int msda_layer_linear_tf32x3_wgrad_supported(int out_features, int in_features)

@@ -352,4 +352,35 @@ __device__ __forceinline__ void red_fixed(long long* p, double v, double scale)
     atomicAdd(reinterpret_cast<unsigned long long*>(p), (unsigned long long)__double2ll_rn(v * scale));
 }
 
+// ----------------------------------------------------------------------------------------
+// Dropout mask (DESIGN.md section 3.16).  Element e of a call's contiguous [rows, C] output draws the 16-bit number
+//     u(e) = (r[(e & 7) >> 1] >> (16 * (e & 1))) & 0xFFFF,   r = Philox4x32-10(counter (lo32(e >> 3), hi32(e >> 3), 0, 0),
+//                                                                               key (lo32(key), hi32(key)))
+// and is kept iff u(e) >= thresh (dropout_rule in msda_launch.h).  One Philox call covers the 8 elements of a group.
+// ----------------------------------------------------------------------------------------
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, unsigned k0, unsigned k1)
+{
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r > 0) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+        const unsigned hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const unsigned hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
+    }
+    return c;
+}
+
+// keep bits of the elements 8 * group + i, i = 0..7: bit i set = element kept
+__device__ __forceinline__ unsigned dropout_keep8(unsigned long long group, unsigned long long key, unsigned thresh)
+{
+    const uint4 r = philox4x32_10(make_uint4((unsigned)group, (unsigned)(group >> 32), 0u, 0u), (unsigned)key,
+                                  (unsigned)(key >> 32));
+    const unsigned w[4] = {r.x, r.y, r.z, r.w};
+    unsigned m = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        m |= ((w[i] & 0xFFFFu) >= thresh ? 1u : 0u) << (2 * i) | ((w[i] >> 16) >= thresh ? 1u : 0u) << (2 * i + 1);
+    return m;
+}
+
 }  // namespace msda

@@ -112,6 +112,21 @@ cudaError_t backward_deterministic(const BwdArgs& a, void* scratch, long long sc
 cudaError_t fused_backward_deterministic(const FusedArgs& a, void* scratch, long long scratch_bytes,
                                          cudaStream_t stream);
 
+// Dropout keep rule (DESIGN.md section 3.16): an element is kept iff its 16-bit Philox draw (dropout_keep8 in
+// msda_common.cuh) is >= thresh = floor(p * 65536 + 0.5); kept values are multiplied by scale = float(1 / (1 - p)).
+// false for p outside (0, 1).
+struct DropoutRule {
+    unsigned thresh;
+    float scale;
+};
+inline bool dropout_rule(float p, DropoutRule* r)
+{
+    if (!(p > 0.f && p < 1.f)) return false;
+    r->thresh = (unsigned)((double)p * 65536.0 + 0.5);
+    r->scale = (float)(1.0 / (1.0 - (double)p));
+    return true;
+}
+
 // Layer epilogues (layer_epilogue.cu):  y = LayerNorm(residual + act(branch)) * gamma + beta,
 // optional y_pos = y + pos; backward of the same.
 struct AddLayerNormArgs {
@@ -138,10 +153,21 @@ struct AddLayerNormArgs {
     void* d_beta;             // [C]
     float* partial;           // [partial_blocks, 2, C] fp32 scratch
     int partial_blocks;       // from add_layernorm_partial_blocks(rows)
+    // dropout on act(branch): v = residual + act(branch) * mask * scale; null key = no dropout.  With dropout, d_branch
+    // is always written (never aliases d_residual)
+    const unsigned long long* drop_key;
+    DropoutRule drop;
 };
 int add_layernorm_chunks(int dtype, int C);            // 0 = unsupported shape
 int add_layernorm_partial_blocks(long long rows);
+bool add_layernorm_dropout_supported(int dtype, int C);   // the widths the dropout path takes
 cudaError_t add_layernorm(const AddLayerNormArgs& a, bool backward, cudaStream_t stream);
+// y = x * mask * scale over n contiguous elements (in place allowed); dx = out > 0 ? g * scale : 0 (the backward of
+// dropout(relu(.)) from its saved output)
+cudaError_t dropout(int dtype, const void* x, void* y, long long n, const unsigned long long* key, DropoutRule rule,
+                    cudaStream_t stream);
+cudaError_t relu_dropout_grad(int dtype, const void* g, const void* out, void* dx, long long n, float scale,
+                              cudaStream_t stream);
 // Fused feed-forward block on tcgen05 (ffn_fused.cu): y = LayerNorm(x + W2 relu(W1 x + b1) + b2), y_pos = y + pos
 struct FfnArgs {
     int dtype;                // kBF16
@@ -194,6 +220,9 @@ cudaError_t tf32_split(const float* x, float* out, long long rows, int cols, cud
 bool linear_bf16_supported(int n, int k);
 cudaError_t linear_bf16(const void* x, const void* w, const void* bias, const unsigned char* row_mask, long long rows, int n,
                         int k, int relu, void* y, cudaStream_t stream);
+// y = dropout(relu(x W^T + b)) in the epilogue: mask of element row * n + col from `key` (dropout_keep8)
+cudaError_t linear_bf16_relu_dropout(const void* x, const void* w, const void* bias, long long rows, int n, int k,
+                                     const unsigned long long* key, DropoutRule rule, void* y, cudaStream_t stream);
 // weight / bias gradient of that layer: dW [n, k] = g^T x, db [n] = sum over rows of g (bf16, fp32 split-K partials in
 // `scratch`, summed in a fixed order by a second kernel: deterministic)
 bool linear_bf16_wgrad_supported(int n, int k);
@@ -203,6 +232,10 @@ cudaError_t linear_bf16_wgrad(const void* g, const void* x, long long rows, int 
 bool linear_tf32x3_supported(int n, int k);
 cudaError_t linear_tf32x3(const float* x, const float* w_hi, const float* w_lo, const float* bias, long long rows, int n,
                           int k, int relu, float* y, cudaStream_t stream);
+// y = dropout(relu(x W^T + b)) in the epilogue: mask of element row * n + col from `key` (dropout_keep8)
+cudaError_t linear_tf32x3_relu_dropout(const float* x, const float* w_hi, const float* w_lo, const float* bias,
+                                       long long rows, int n, int k, const unsigned long long* key, DropoutRule rule,
+                                       float* y, cudaStream_t stream);
 // weight / bias gradient of that layer: dW [n, k] = g^T x, db [n] = sum over rows of g (fp32, the three-term split with
 // both operands split in shared memory; fp32 split-K partials in `scratch`, summed in a fixed order: deterministic)
 bool linear_tf32x3_wgrad_supported(int n, int k);

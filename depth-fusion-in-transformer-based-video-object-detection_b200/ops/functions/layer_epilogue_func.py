@@ -6,10 +6,14 @@
 as ONE kernel per direction.  ``zero_masked_rows_`` is MSDeformAttn's
 ``value.masked_fill(mask[..., None], 0)`` (models/ops/modules/ms_deform_attn.py:95-96) in place.
 ``linear_relu`` is ``relu(linear1(x))`` with the activation in the GEMM epilogue (library GEMM).
+Both take the layer's ``nn.Dropout`` and then apply it inside the same kernels (``dropout`` for the other sites).
 CUDA tensors only; callers keep the PyTorch composition for shapes the kernels do not cover.
 """
+import ctypes
+
 import torch
 import torch.nn.functional as F
+from torch import nn
 from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 
@@ -33,11 +37,99 @@ def _dense(t):
     return t if t.data_ptr() % 16 == 0 else t.clone()
 
 
-class AddLayerNormFunction(Function):
-    """apply(branch, residual|None, gamma, beta, eps, act_code, pos|None) -> y  or  (y, y + pos)"""
+# Dropout on the package's kernels (DESIGN.md section 3.16): each call draws one int64 key on the device, and the mask of
+# element e of the call's [rows, C] output is a function of (key, e) (Philox4x32-10, msda_common.cuh: dropout_keep8).  The
+# backward regenerates it from the saved key, so no mask is stored and no separate dropout pass runs: the mask is applied
+# inside the add-LayerNorm and ReLU-GEMM kernels.  Taken when the module is exactly nn.Dropout, in training, 0 < p < 1,
+# on a CUDA fp32 / bf16 / fp16 tensor; False keeps torch's nn.Dropout between the kernels (the A/B of
+# tools/bench_dropout.py).
+PACKAGE_DROPOUT = True
+
+
+def _dropout_key(device):
+    """The key of one dropout call: one int64 from torch's CUDA generator, never read back (graph-capturable)."""
+    return torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=device)
+
+
+def _dropout_mode(module, x):
+    """"none": no dropout (no module, eval mode or p == 0: no key is drawn); "package": the package's kernels;
+    "module": torch's ``module(x)``."""
+    if module is None:
+        return "none"
+    if type(module) is not nn.Dropout:
+        return "module"
+    if not module.training or module.p == 0:
+        return "none"
+    if PACKAGE_DROPOUT and 0 < module.p < 1 and x.is_cuda and x.dtype in _DTYPES:
+        return "package"
+    return "module"
+
+
+def dropout_rule(p):
+    """(threshold, scale) of the keep rule at rate p: an element is kept iff its 16-bit draw is >= threshold."""
+    t, scale = ctypes.c_uint32(), ctypes.c_float()
+    _lib.check(_lib.load().msda_layer_dropout_rule(float(p), ctypes.byref(t), ctypes.byref(scale)),
+               "msda_layer_dropout_rule")
+    return t.value, scale.value
+
+
+def _dropout_into(x, y, p, key):
+    """y = x * mask(key) * scale over the contiguous x (y may be x)."""
+    with torch.cuda.device(x.device):
+        code = _lib.load().msda_layer_dropout(_DTYPES[x.dtype], x.data_ptr(), y.data_ptr(), x.numel(), float(p),
+                                              key.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(code, "msda_layer_dropout")
+    return y
+
+
+def relu_dropout_grad(grad, out, p):
+    """grad * scale where out > 0, else 0: the backward of dropout(relu(.)) at rate p from its output alone."""
+    grad = grad.reshape(out.shape).contiguous()
+    if grad.dtype != out.dtype:
+        grad = grad.to(out.dtype)
+    dx = torch.empty_like(out)
+    with torch.cuda.device(out.device):
+        code = _lib.load().msda_layer_relu_dropout_grad(_DTYPES[out.dtype], grad.data_ptr(), out.data_ptr(), dx.data_ptr(),
+                                                        out.numel(), float(p), torch.cuda.current_stream().cuda_stream)
+    _lib.check(code, "msda_layer_relu_dropout_grad")
+    return dx
+
+
+class DropoutFunction(Function):
+    """apply(x, p, key) -> x * mask * scale; the backward is the same kernel on the gradient with the same key."""
 
     @staticmethod
-    def forward(ctx, branch, residual, gamma, beta, eps, act, pos):
+    def forward(ctx, x, p, key):
+        xc = x.contiguous()
+        y = _dropout_into(xc, torch.empty_like(xc), p, key)
+        ctx.save_for_backward(key)
+        ctx.p = p
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad):
+        (key,) = ctx.saved_tensors
+        g = grad.contiguous()
+        return _dropout_into(g, torch.empty_like(g), ctx.p, key), None, None
+
+
+def dropout(module, x):
+    """``module(x)`` for the layer's dropout module: the package's kernel when it applies (see PACKAGE_DROPOUT)."""
+    mode = _dropout_mode(module, x)
+    if mode == "none":
+        return x
+    if mode == "module":
+        return module(x)
+    return DropoutFunction.apply(x, float(module.p), _dropout_key(x.device))
+
+
+class AddLayerNormFunction(Function):
+    """apply(branch, residual|None, gamma, beta, eps, act_code, pos|None[, p, key]) -> y  or  (y, y + pos);
+    with a key, dropout at rate p on act(branch)."""
+
+    @staticmethod
+    def forward(ctx, branch, residual, gamma, beta, eps, act, pos, p=0.0, key=None):
         shape = branch.shape
         c = shape[-1]
         dt = branch.dtype
@@ -53,13 +145,17 @@ class AddLayerNormFunction(Function):
             y_pos = torch.empty_like(branch) if pos is not None else None
             mean = torch.empty(rows, dtype=torch.float32, device=branch.device) if needs_grad else None
             rstd = torch.empty_like(mean) if needs_grad else None
-            code = lib.msda_layer_add_layernorm_forward(
-                _DTYPES[dt], act, branch.data_ptr(), _ptr(residual), gamma_c.data_ptr(), beta_c.data_ptr(),
-                _ptr(pos), rows, c, float(eps), y.data_ptr(), _ptr(y_pos), _ptr(mean), _ptr(rstd),
-                torch.cuda.current_stream().cuda_stream)
+            args = (_DTYPES[dt], act, branch.data_ptr(), _ptr(residual), gamma_c.data_ptr(), beta_c.data_ptr(),
+                    _ptr(pos), rows, c, float(eps), y.data_ptr(), _ptr(y_pos), _ptr(mean), _ptr(rstd))
+            stream = torch.cuda.current_stream().cuda_stream
+            if key is None:
+                code = lib.msda_layer_add_layernorm_forward(*args, stream)
+            else:
+                code = lib.msda_layer_add_layernorm_dropout_forward(*args, float(p), key.data_ptr(), stream)
         _lib.check(code, "msda_layer_add_layernorm_forward")
         if needs_grad:
-            ctx.save_for_backward(branch, residual, gamma_c, mean, rstd)
+            ctx.save_for_backward(branch, residual, gamma_c, mean, rstd, key)
+            ctx.p = p
             ctx.act = act
             ctx.param_dtypes = (gamma.dtype, beta.dtype)
             ctx.has_pos = pos is not None
@@ -70,12 +166,12 @@ class AddLayerNormFunction(Function):
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_y, grad_y_pos=None):
-        branch, residual, gamma, mean, rstd = ctx.saved_tensors
+        branch, residual, gamma, mean, rstd, key = ctx.saved_tensors
         c = branch.shape[-1]
         rows = branch.numel() // c
         dt = branch.dtype
         if grad_y is None and grad_y_pos is None:
-            return (None,) * 7
+            return (None,) * 9
         if grad_y is None:            # only the y + pos output was used downstream
             grad_y, grad_y_pos_k = grad_y_pos, None
         else:
@@ -85,32 +181,43 @@ class AddLayerNormFunction(Function):
         lib = _lib.load()
         with torch.cuda.device(branch.device):
             d_res = torch.empty_like(branch) if residual is not None else None
-            d_branch = torch.empty_like(branch) if (ctx.act != 0 or residual is None) else d_res
+            own = ctx.act != 0 or residual is None or key is not None
+            d_branch = torch.empty_like(branch) if own else d_res
             d_gamma = torch.empty_like(gamma)
             d_beta = torch.empty_like(gamma)
             blocks = lib.msda_layer_add_layernorm_partial_blocks(rows)
             partial = torch.empty((blocks, 2, c), dtype=torch.float32, device=branch.device)
-            code = lib.msda_layer_add_layernorm_backward(
-                _DTYPES[dt], ctx.act, grad_y.data_ptr(), _ptr(grad_y_pos_k), branch.data_ptr(), _ptr(residual),
-                gamma.data_ptr(), mean.data_ptr(), rstd.data_ptr(), rows, c, d_branch.data_ptr(), _ptr(d_res),
-                d_gamma.data_ptr(), d_beta.data_ptr(), partial.data_ptr(), blocks,
-                torch.cuda.current_stream().cuda_stream)
+            args = (_DTYPES[dt], ctx.act, grad_y.data_ptr(), _ptr(grad_y_pos_k), branch.data_ptr(), _ptr(residual),
+                    gamma.data_ptr(), mean.data_ptr(), rstd.data_ptr(), rows, c, d_branch.data_ptr(), _ptr(d_res),
+                    d_gamma.data_ptr(), d_beta.data_ptr(), partial.data_ptr(), blocks)
+            stream = torch.cuda.current_stream().cuda_stream
+            if key is None:
+                code = lib.msda_layer_add_layernorm_backward(*args, stream)
+            else:
+                code = lib.msda_layer_add_layernorm_dropout_backward(*args, float(ctx.p), key.data_ptr(), stream)
         _lib.check(code, "msda_layer_add_layernorm_backward")
         d_pos = grad_y_pos if ctx.has_pos else None
         return (d_branch, d_res, d_gamma.to(ctx.param_dtypes[0]), d_beta.to(ctx.param_dtypes[1]), None, None,
-                d_pos)
+                d_pos, None, None)
 
 
-def add_layer_norm(norm, branch, residual=None, act=None, pos=None):
-    """``norm(residual + act(branch))`` and, when ``pos`` is given, also ``that + pos``.
+def add_layer_norm(norm, branch, residual=None, act=None, pos=None, dropout=None):
+    """``norm(residual + dropout(act(branch)))`` and, when ``pos`` is given, also ``that + pos``.
 
     ``norm`` is the layer's ``nn.LayerNorm`` (parameters / eps are read from it, so state_dict keys
-    stay the reference's).  Returns ``y`` or ``(y, y_pos)``."""
+    stay the reference's), ``dropout`` the layer's ``nn.Dropout`` or None.  Returns ``y`` or ``(y, y_pos)``."""
     c = branch.shape[-1]
     fusable = (add_layer_norm_supported(branch, c) and norm.elementwise_affine and norm.bias is not None
                and tuple(norm.normalized_shape) == (c,) and act in ACT_CODES
                and (residual is None or residual.shape == branch.shape)
                and (pos is None or pos.shape == branch.shape))
+    mode = _dropout_mode(dropout, branch)
+    if mode == "package" and fusable and _lib.load().msda_layer_add_layernorm_dropout_supported(_DTYPES[branch.dtype], c):
+        return AddLayerNormFunction.apply(branch, residual, norm.weight, norm.bias, norm.eps, ACT_CODES[act], pos,
+                                          float(dropout.p), _dropout_key(branch.device))
+    if mode != "none":
+        h = branch if act in (None, "none") else getattr(F, act)(branch)
+        return add_layer_norm(norm, globals()["dropout"](dropout, h), residual, None, pos)
     if fusable:
         return AddLayerNormFunction.apply(branch, residual, norm.weight, norm.bias, norm.eps, ACT_CODES[act], pos)
     # PyTorch composition (shapes the kernel does not cover)
@@ -335,18 +442,25 @@ def _tf32x3_kernel_wins(n, k):
     return True
 
 
-def _linear_tf32x3_kernel(x2, w_hi, w_lo, bias, relu=False):
+def _linear_tf32x3_kernel(x2, w_hi, w_lo, bias, relu=False, dropout=None):
     """x2 [rows, k] @ (w_hi + w_lo)^T + bias -> a fresh [rows, n] (ReLU) on csrc/linear_tf32x3.cu; (w_hi, w_lo) [n, k]
-    contiguous, the TF32 split of a weight (_tf32_weight_split) or of its transpose."""
+    contiguous, the TF32 split of a weight (_tf32_weight_split) or of its transpose.  dropout = (p, key): ReLU, then
+    dropout in the epilogue."""
     n, k = w_hi.shape
     if not x2.is_contiguous() or x2.data_ptr() % 16 != 0:
         x2 = x2.contiguous()
     b = None if bias is None else bias.detach().contiguous()
     y = torch.empty((x2.shape[0], n), dtype=torch.float32, device=x2.device)
     with torch.cuda.device(x2.device):
-        code = _lib.load().msda_layer_linear_tf32x3(x2.data_ptr(), w_hi.data_ptr(), w_lo.data_ptr(),
-                                                    None if b is None else b.data_ptr(), x2.shape[0], n, k,
-                                                    1 if relu else 0, y.data_ptr(), torch.cuda.current_stream().cuda_stream)
+        stream = torch.cuda.current_stream().cuda_stream
+        if dropout is None:
+            code = _lib.load().msda_layer_linear_tf32x3(x2.data_ptr(), w_hi.data_ptr(), w_lo.data_ptr(),
+                                                        None if b is None else b.data_ptr(), x2.shape[0], n, k,
+                                                        1 if relu else 0, y.data_ptr(), stream)
+        else:
+            code = _lib.load().msda_layer_linear_tf32x3_relu_dropout(
+                x2.data_ptr(), w_hi.data_ptr(), w_lo.data_ptr(), None if b is None else b.data_ptr(), x2.shape[0], n, k,
+                float(dropout[0]), dropout[1].data_ptr(), y.data_ptr(), stream)
     _lib.check(code, "msda_layer_linear_tf32x3")
     return y
 
@@ -614,25 +728,35 @@ class LinearReLUFunction(Function):
     "tf32x3": the three-term TF32 kernels in both directions (_fp32_train_kernels_apply)."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias):
+    def forward(ctx, x, weight, bias, p=0.0, key=None):
+        # with a key: dropout(relu(.)) at rate p; the saved output is the dropped one, and it alone gives the backward
         x2 = x.reshape(-1, x.shape[-1])
         ctx.kernels = any(ctx.needs_input_grad) and _bf16_train_kernels_apply(x2, weight, bias)
         ctx.tf32x3 = not ctx.kernels and any(ctx.needs_input_grad) and _fp32_train_kernels_apply(x2, weight, bias)
+        fused = key is not None and _relu_dropout_epilogue_wins(weight.shape[0], weight.shape[1])
         if ctx.kernels:
-            out = linear_bf16(x2, weight, bias, relu=True)
+            out = _linear_bf16_relu_dropout(x2, weight, bias, p, key) if fused else linear_bf16(x2, weight, bias, relu=True)
         elif ctx.tf32x3:
-            out = _linear_tf32x3_kernel(x2, *_tf32_weight_split(weight, live=True), bias, relu=True)
+            w_split = _tf32_weight_split(weight, live=True)
+            out = _linear_tf32x3_kernel(x2, *w_split, bias, relu=True, dropout=(p, key) if fused else None)
         else:
             out = torch._addmm_activation(bias, x2, weight.t(), use_gelu=False)
+            fused = False
+        if key is not None and not fused:
+            _dropout_into(out, out, p, key)
         ctx.save_for_backward(x2, weight, out)
         ctx.x_shape = x.shape
+        ctx.p = p if key is not None else None
         return out.view(*x.shape[:-1], weight.shape[0])
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad):
         x2, weight, out = ctx.saved_tensors
-        g = torch.ops.aten.threshold_backward(grad.reshape(out.shape), out, 0)
+        if ctx.p is None:
+            g = torch.ops.aten.threshold_backward(grad.reshape(out.shape), out, 0)
+        else:
+            g = relu_dropout_grad(grad, out, ctx.p)
         if ctx.kernels:
             dx, dw, db = _bf16_linear_backward(ctx.needs_input_grad, g.contiguous(), x2, weight,
                                                (weight.dtype, weight.dtype))
@@ -642,11 +766,44 @@ class LinearReLUFunction(Function):
             dx = g @ weight if ctx.needs_input_grad[0] else None
             dw = g.t() @ x2 if ctx.needs_input_grad[1] else None
             db = column_sum(g) if ctx.needs_input_grad[2] else None
-        return (None if dx is None else dx.view(ctx.x_shape)), dw, db
+        return (None if dx is None else dx.view(ctx.x_shape)), dw, db, None, None
 
 
-def linear_relu(linear, x):
-    """``relu(linear(x))``; epilogue-fused on CUDA for 16-bit / fp32 dense inputs."""
+def _relu_dropout_epilogue_wins(n, k):
+    """Dropout in the GEMM epilogue (bf16 and tf32x3 kernel routes) against the plain ReLU GEMM + the in-place dropout
+    kernel.  Measured on one B200 (1000 W) at 88 892 rows, 1024 <- 256, bf16 forward + backward (tools/bench_dropout.py,
+    DESIGN.md section 3.16): 0.354 ms in the epilogue, 0.389 ms as GEMM + dropout kernel, so the epilogue is taken."""
+    return True
+
+
+def _linear_bf16_relu_dropout(x2, weight, bias, p, key):
+    """dropout(relu(x2 W^T + b)) -> a fresh bf16 [rows, n] on csrc/linear_bf16.cu, the mask applied in the epilogue."""
+    n, k = weight.shape
+    if not x2.is_contiguous() or x2.data_ptr() % 16 != 0:
+        x2 = x2.contiguous()
+    w = weight.detach()
+    if not w.is_contiguous() or w.data_ptr() % 16 != 0:
+        w = w.contiguous()
+    b = None if bias is None else bias.detach().contiguous()
+    y = torch.empty((x2.shape[0], n), dtype=torch.bfloat16, device=x2.device)
+    with torch.cuda.device(x2.device):
+        code = _lib.load().msda_layer_linear_bf16_relu_dropout(
+            x2.data_ptr(), w.data_ptr(), None if b is None else b.data_ptr(), x2.shape[0], n, k, float(p), key.data_ptr(),
+            y.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(code, "msda_layer_linear_bf16_relu_dropout")
+    return y
+
+
+def linear_relu(linear, x, dropout=None):
+    """``dropout(relu(linear(x)))``; epilogue-fused on CUDA for 16-bit / fp32 dense inputs.  ``dropout`` is the layer's
+    ``nn.Dropout`` or None."""
+    mode = _dropout_mode(dropout, x)
+    if mode == "module":
+        return dropout(linear_relu(linear, x))
+    if mode == "package":
+        if x.dtype == linear.weight.dtype and linear.bias is not None:
+            return LinearReLUFunction.apply(x, linear.weight, linear.bias, float(dropout.p), _dropout_key(x.device))
+        return globals()["dropout"](dropout, linear_relu(linear, x))
     if _tf32x3_wanted(x, linear.weight):
         return linear_tf32x3(x, linear.weight, linear.bias, relu=True)
     if _bf16_kernel_wanted(x, linear.weight, linear.bias):

@@ -25,7 +25,7 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
-from .ops.functions import (add_layer_norm, ffn_layer_norm, ffn_layer_norm_supported, linear, linear_relu,
+from .ops.functions import (add_layer_norm, dropout, ffn_layer_norm, ffn_layer_norm_supported, linear, linear_relu,
                             proj_layer_norm)
 from .ops.modules import MSDeformAttn, project_values
 from .ops.modules.ms_deform_attn import host_shape_list
@@ -120,9 +120,9 @@ class DeformableTransformerEncoderLayer(nn.Module):
         if self._activation_name == "relu" and not (self.training and (self.dropout2.p > 0 or self.dropout3.p > 0)) \
                 and self.use_fused_ffn and ffn_layer_norm_supported(src, self.linear1, self.linear2, self.norm2):
             return ffn_layer_norm(self.linear1, self.linear2, self.norm2, src, pos)     # one tcgen05 kernel
-        hidden = linear_relu(self.linear1, src) if self._activation_name == "relu" \
-            else self.activation(linear(self.linear1, src))
-        return add_layer_norm(self.norm2, self.dropout3(linear(self.linear2, self.dropout2(hidden))), src, None, pos)
+        hidden = linear_relu(self.linear1, src, self.dropout2) if self._activation_name == "relu" \
+            else dropout(self.dropout2, self.activation(linear(self.linear1, src)))
+        return add_layer_norm(self.norm2, linear(self.linear2, hidden), src, None, pos, dropout=self.dropout3)
 
     def forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask=None,
                 rgbd_src=None, query=None, emit_query=False):
@@ -133,7 +133,7 @@ class DeformableTransformerEncoderLayer(nn.Module):
             query = rgbd_src if rgbd_src is not None else _add_pos(src, pos)
         if self.training and self.dropout1.p > 0:
             attended = self.self_attn(query, reference_points, src, spatial_shapes, level_start_index, padding_mask)
-            src = add_layer_norm(self.norm1, self.dropout1(attended), src)
+            src = add_layer_norm(self.norm1, attended, src, dropout=self.dropout1)
         else:       # output projection + residual + LayerNorm as one kernel (bf16 inference), else GEMM + fused norm
             heads = self.self_attn(query, reference_points, src, spatial_shapes, level_start_index, padding_mask,
                                    project_output=False)
@@ -201,9 +201,8 @@ class _CrossModalFusion(nn.Module):
 
     def forward_ffn(self, tgt):
         drop, norm = getattr(self, self._ffn_dropout), getattr(self, self._ffn_norm)
-        if drop.training and drop.p > 0:
-            return add_layer_norm(norm, drop(self.activation(linear(self.linear1, tgt))), tgt)
-        return add_layer_norm(norm, linear(self.linear1, tgt), tgt, "gelu")       # GELU inside the norm kernel
+        # GELU (and the dropout, when training) inside the norm kernel
+        return add_layer_norm(norm, linear(self.linear1, tgt), tgt, "gelu", dropout=drop)
 
     def _fuse(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index, src_padding_mask,
               query=None):
@@ -214,7 +213,7 @@ class _CrossModalFusion(nn.Module):
         sampled = self.cross_attn(query, reference_points, src, src_spatial_shapes, level_start_index,
                                   src_padding_mask)
         if self.training and self.dropout1.p > 0:
-            tgt = add_layer_norm(self.norm1, self.dropout1(linear(self.cross_scale_adapt, sampled)), tgt)
+            tgt = add_layer_norm(self.norm1, linear(self.cross_scale_adapt, sampled), tgt, dropout=self.dropout1)
         else:
             tgt = proj_layer_norm(self.cross_scale_adapt, self.norm1, sampled, tgt)
         return self.forward_ffn(tgt)
@@ -324,9 +323,9 @@ class DeformableTransformerDecoderLayer(nn.Module):
     with_pos_embed = staticmethod(_add_pos)
 
     def forward_ffn(self, tgt, pos=None):
-        hidden = linear_relu(self.linear1, tgt) if self._activation_name == "relu" \
-            else self.activation(linear(self.linear1, tgt))
-        return add_layer_norm(self.norm3, self.dropout4(linear(self.linear2, self.dropout3(hidden))), tgt, None, pos)
+        hidden = linear_relu(self.linear1, tgt, self.dropout3) if self._activation_name == "relu" \
+            else dropout(self.dropout3, self.activation(linear(self.linear1, tgt)))
+        return add_layer_norm(self.norm3, linear(self.linear2, hidden), tgt, None, pos, dropout=self.dropout4)
 
     def forward(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
                 src_padding_mask=None, qk=None, emit_qk=False, value=None):
@@ -337,12 +336,12 @@ class DeformableTransformerDecoderLayer(nn.Module):
             qk = _add_pos(tgt, query_pos)
         mixed = mha_batch_first(self.self_attn, qk, qk, tgt)
         if query_pos is not None:
-            tgt, query = add_layer_norm(self.norm2, self.dropout2(mixed), tgt, None, query_pos)
+            tgt, query = add_layer_norm(self.norm2, mixed, tgt, None, query_pos, dropout=self.dropout2)
         else:
-            tgt = query = add_layer_norm(self.norm2, self.dropout2(mixed), tgt)
+            tgt = query = add_layer_norm(self.norm2, mixed, tgt, dropout=self.dropout2)
         sampled = self.cross_attn(query, reference_points, src, src_spatial_shapes, level_start_index,
                                   src_padding_mask, precomputed_value=value)
-        tgt = add_layer_norm(self.norm1, self.dropout1(sampled), tgt)
+        tgt = add_layer_norm(self.norm1, sampled, tgt, dropout=self.dropout1)
         if not emit_qk:
             return self.forward_ffn(tgt)
         if query_pos is None:

@@ -428,6 +428,53 @@ int msda_roi_align_backward_deterministic(int dtype, const void* grad_pooled, co
                                           double spatial_scale, int sampling_ratio, int aligned, void* grad_feature,
                                           void* scratch, int64_t scratch_bytes, void* stream);
 
+/* Dropout on the package's kernels (DESIGN.md section 3.16).  `key` points to ONE uint64 in device memory
+ * (drawn per call by the caller on the device; it is never read on the host, so the calls
+ * can be captured in a CUDA graph).  Element e of a call's contiguous [rows, channels] output draws
+ *     u(e) = (r[(e & 7) >> 1] >> (16 * (e & 1))) & 0xFFFF,
+ *     r = Philox4x32-10(counter (lo32(e >> 3), hi32(e >> 3), 0, 0), key (lo32(key), hi32(key)))
+ * and is kept iff u(e) >= threshold = floor(p * 65536 + 0.5); kept values are multiplied by
+ * scale = float(1 / (1 - p)).  msda_layer_dropout_rule reports threshold and scale.  Every call returns
+ * cudaErrorInvalidValue for p outside (0, 1) or a NULL key.
+ *
+ * add-LayerNorm with dropout on the branch: v = residual + act(branch) * mask * scale, otherwise as
+ * msda_layer_add_layernorm_forward / _backward.  The backward regenerates the mask from the same key and p; it
+ * always writes grad_branch (never aliased with grad_residual).  Channel counts:
+ * msda_layer_add_layernorm_dropout_supported (1 or 2 sixteen-byte chunks per lane: 128/256 F32, 256/512 16-bit).
+ *
+ * msda_layer_dropout: y = x * mask * scale over n contiguous elements of dtype; y == x is allowed.  Called on a
+ * gradient with the same key and p it is the backward.
+ * msda_layer_relu_dropout_grad: grad_x = y > 0 ? grad_y * scale : 0, the backward of dropout(relu(.)) from its
+ * output y alone (no key).
+ * msda_layer_linear_bf16_relu_dropout / msda_layer_linear_tf32x3_relu_dropout: msda_layer_linear_bf16 /
+ * msda_layer_linear_tf32x3 with relu = 1 and dropout applied in the epilogue (element index row * out_features + col). */
+int msda_layer_dropout_rule(float p, uint32_t* threshold, float* scale);
+int msda_layer_add_layernorm_dropout_supported(int dtype, int channels);
+int msda_layer_add_layernorm_dropout_forward(int dtype, int act,
+                                             const void* branch, const void* residual,
+                                             const void* gamma, const void* beta, const void* pos,
+                                             int64_t rows, int channels, float eps,
+                                             void* y, void* y_pos, float* mean, float* rstd,
+                                             float p, const uint64_t* key, void* stream);
+int msda_layer_add_layernorm_dropout_backward(int dtype, int act,
+                                              const void* grad_y, const void* grad_y_pos,
+                                              const void* branch, const void* residual, const void* gamma,
+                                              const float* mean, const float* rstd,
+                                              int64_t rows, int channels,
+                                              void* grad_branch, void* grad_residual,
+                                              void* grad_gamma, void* grad_beta,
+                                              float* partial_scratch, int partial_blocks,
+                                              float p, const uint64_t* key, void* stream);
+int msda_layer_dropout(int dtype, const void* x, void* y, int64_t n, float p, const uint64_t* key, void* stream);
+int msda_layer_relu_dropout_grad(int dtype, const void* grad_y, const void* y, void* grad_x, int64_t n, float p,
+                                 void* stream);
+int msda_layer_linear_bf16_relu_dropout(const void* x, const void* weight, const void* bias, int64_t rows,
+                                        int out_features, int in_features, float p, const uint64_t* key, void* y,
+                                        void* stream);
+int msda_layer_linear_tf32x3_relu_dropout(const float* x, const float* weight_hi, const float* weight_lo,
+                                          const float* bias, int64_t rows, int out_features, int in_features,
+                                          float p, const uint64_t* key, float* y, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
