@@ -12,12 +12,15 @@ Layout (only what the hot path needs):
   deformable_transformer.py              single-frame DeformableTransformer (baseline / Late Fusion / Encoder Cross Fusion)
   position_encoding.py                   PositionEmbeddingSine written token-major (lvl_pos_embed_flatten in one pass)
   temporal_stage.py                      TransVOD++ multi-frame transformer: RoIAlign, QRF head, TQE, TDTD
+  criterion.py                           Deformable DETR's HungarianMatcher / SetCriterion, assignment solved on the GPU
 
 The directory name carries hyphens; import it through the alias module ``dfvod_b200`` at the
 repository root (``import dfvod_b200``), or put ``ops`` in place of the reference's ``models/ops``.
 """
 from . import MultiScaleDeformableAttention
+from .criterion import HungarianMatcher, SetCriterion, pad_targets
 from .ops.functions import MSDeformAttnFunction
 from .ops.modules import MSDeformAttn
 
-__all__ = ["MultiScaleDeformableAttention", "MSDeformAttnFunction", "MSDeformAttn"]
+__all__ = ["MultiScaleDeformableAttention", "MSDeformAttnFunction", "MSDeformAttn", "HungarianMatcher", "SetCriterion",
+           "pad_targets"]

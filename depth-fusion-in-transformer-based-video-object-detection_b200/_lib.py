@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # MSDA_B200_LIB selects another build of the same ABI (A/B kernel experiments); default: in-tree
 LIB_PATH = os.environ.get("MSDA_B200_LIB") or os.path.join(_HERE, "libmsda_b200.so")
 
-ABI_VERSION = 24
+ABI_VERSION = 25
 DTYPE_F32, DTYPE_F64, DTYPE_BF16, DTYPE_F16 = 0, 1, 2, 3
 FLAG_FORCE_GENERIC = 1
 FLAG_TC = 4
@@ -152,6 +152,11 @@ def load():
     lib.msda_layer_colsum.argtypes = [c_int, c_vp, c_i64, c_int, c_vp, c_vp, c_int, c_vp]
     lib.msda_layer_zero_masked_rows.restype = c_int
     lib.msda_layer_zero_masked_rows.argtypes = [c_int, c_vp, c_vp, c_i64, c_int, c_vp]
+    lib.msda_linear_assignment_scratch_bytes.restype = c_i64
+    lib.msda_linear_assignment_scratch_bytes.argtypes = [c_int, c_int, c_int]
+    lib.msda_linear_assignment.restype = c_int
+    lib.msda_linear_assignment.argtypes = [c_vp, c_i64, c_i64, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_i64,
+                                           c_vp]
     if lib.msda_abi_version() != ABI_VERSION:
         raise MSDAError(f"libmsda_b200.so ABI {lib.msda_abi_version()} != binding ABI {ABI_VERSION}; rebuild")
     _lib = lib

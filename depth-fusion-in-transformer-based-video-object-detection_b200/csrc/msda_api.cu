@@ -7,7 +7,7 @@ static bool bad_dims(int N, int S, int M, int D, int L, int Lq, int P)
     return N < 0 || S < 0 || M < 0 || D < 0 || L < 0 || Lq < 0 || P < 0;
 }
 
-extern "C" int msda_abi_version(void) { return 24; }
+extern "C" int msda_abi_version(void) { return 25; }
 
 extern "C" const char* msda_error_string(int code)
 {
@@ -614,4 +614,21 @@ extern "C" int msda_layer_linear_tf32x3_wgrad(const float* grad_y, const float* 
 {
     return (int)msda::linear_tf32x3_wgrad(grad_y, x, (long long)rows, out_features, in_features, grad_weight, grad_bias,
                                           scratch, (long long)scratch_floats, (cudaStream_t)stream);
+}
+
+// ---- batched linear assignment (hungarian.cu) ------------------------------------------------------
+
+extern "C" int64_t msda_linear_assignment_scratch_bytes(int num_problems, int num_queries, int max_targets)
+{
+    return (int64_t)msda::linear_assignment_scratch_bytes(num_problems, num_queries, max_targets);
+}
+
+extern "C" int msda_linear_assignment(const float* cost, int64_t problem_stride, int64_t query_stride,
+                                      const int64_t* counts, int num_problems, int num_queries, int max_targets,
+                                      int32_t* query_of_target, int32_t* target_of_query, int32_t* status,
+                                      void* scratch, int64_t scratch_bytes, void* stream)
+{
+    return (int)msda::linear_assignment(cost, (long long)problem_stride, (long long)query_stride, counts,
+                                        num_problems, num_queries, max_targets, query_of_target, target_of_query,
+                                        status, scratch, (long long)scratch_bytes, (cudaStream_t)stream);
 }

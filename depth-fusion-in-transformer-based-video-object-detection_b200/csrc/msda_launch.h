@@ -274,4 +274,11 @@ cudaError_t colsum(int dtype, const void* x, long long rows, int C, void* out, f
 cudaError_t zero_masked_rows(int dtype, void* data, const unsigned char* mask, long long rows, int C,
                              cudaStream_t stream);
 
+// Batched rectangular linear assignment (hungarian.cu, DESIGN.md section 3.17)
+long long linear_assignment_scratch_bytes(int P, int Q, int Tmax);
+cudaError_t linear_assignment(const float* cost, long long problem_stride, long long query_stride,
+                              const int64_t* counts, int P, int Q, int Tmax, int* query_of_target,
+                              int* target_of_query, int* status, void* scratch, long long scratch_bytes,
+                              cudaStream_t stream);
+
 }  // namespace msda

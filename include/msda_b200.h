@@ -475,6 +475,28 @@ int msda_layer_linear_tf32x3_relu_dropout(const float* x, const float* weight_hi
                                           const float* bias, int64_t rows, int out_features, int in_features,
                                           float p, const uint64_t* key, float* y, void* stream);
 
+/* Batched rectangular linear assignment (csrc/hungarian.cu, DESIGN.md section 3.17): the Hungarian matching of
+ * Deformable DETR's set criterion, solved on the device for many (image, output head) problems in one launch.
+ *   cost             fp32; problem p's cost of matching query q to target t is
+ *                    cost[p * problem_stride + q * query_stride + t]  (t < max_targets, q < num_queries)
+ *   counts           [num_problems] int64 target counts T_p, read on the device; 0 <= T_p <= min(max_targets,
+ *                    num_queries) is required
+ *   query_of_target  [num_problems, max_targets] int32: the query matched to target t, -1 for t >= T_p
+ *   target_of_query  [num_problems, num_queries] int32: the target matched to query q, -1 if unmatched
+ *   status           [num_problems] int32: 0 solved; 1 a cost of the first T_p targets is NaN or +-Inf;
+ *                    2 T_p out of range; 3 no feasible matching.  A non-zero status writes -1 to all of the
+ *                    problem's outputs.  The call never traps on bad data.
+ * Every target is matched, at the least total cost: the shortest-augmenting-path algorithm of
+ * scipy.optimize.linear_sum_assignment on the same fp64-widened costs with fp64 potentials, so costs without
+ * ties give scipy's assignment.  Among equal-cost solutions the choice may differ from scipy's.
+ * `scratch` of msda_linear_assignment_scratch_bytes bytes (0 for num_queries <= 1024, when the state lives in
+ * shared memory); the scratch bytes call returns -1 for negative sizes. */
+int64_t msda_linear_assignment_scratch_bytes(int num_problems, int num_queries, int max_targets);
+int msda_linear_assignment(const float* cost, int64_t problem_stride, int64_t query_stride, const int64_t* counts,
+                           int num_problems, int num_queries, int max_targets, int32_t* query_of_target,
+                           int32_t* target_of_query, int32_t* status, void* scratch, int64_t scratch_bytes,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif
